@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this engine (one rank per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs (see dump_outputs)
 
 A "step" is one pass of the hot path -- keyswitch + programmable bootstrap with per-ciphertext lookup table -- over one batch of
 `--batch` independent LWE ciphertexts per GPU at PARAM_MESSAGE_2_CARRY_2_KS_PBS.  `value` is device-timed whole-job KS-PBS/s with
@@ -149,6 +150,24 @@ class CpuReference:
         return self.wl.check(self.out[:n_cts], self.vals[:n_cts], self.idx[:n_cts])["ok"]
 
 
+DUMP_ROWS = 2048        # 2048 x 2049 words x 8 B = 34 MB of float64 for the 2_2 and multi-bit sets
+
+
+def dump_rows(n: int) -> np.ndarray:
+    """the rows dump_outputs keeps of an n-ciphertext batch: all of them, or a fixed, seeded sample of DUMP_ROWS in batch order"""
+    return np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0xD0).choice(n, DUMP_ROWS, replace=False))
+
+
+def dump_outputs(out_dir: str, cts: np.ndarray):
+    """Writes out_dir/ks_pbs_out.npy: the output LWE ciphertexts of the last timed step, rows dump_rows(batch), as float64 torus values
+    (signed word / 2^64, in [-0.5, 0.5]).  The inputs are seeded, so two builds run with the same arguments can be compared row for row;
+    the low bits of each word carry the FFT's rounding, so the comparison wants a tolerance rather than equality."""
+    torus = np.ascontiguousarray(cts[dump_rows(cts.shape[0])]).view(np.int64).astype(np.float64) / 2.0**64
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "ks_pbs_out.npy", torus)
+
+
 def cpu_reference_rate(wl: Workload, n_cts: int):
     ref = CpuReference(wl, n_cts)
     ref.run(min(n_cts, ref.cores))          # warm-up: page in the Fourier key, spin up the OpenMP team
@@ -171,6 +190,8 @@ def run_reference(args):
         if s >= args.warmup:
             total_t += dt
     ok = ref.validate(min(per_step, 256))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ref.out[:per_step])
     value = per_step * args.steps / total_t
     line = {
         "impl": "reference", "metric": "batched KS-PBS throughput", "value": value, "unit": "PBS/s", "n_gpus": args.gpus,
@@ -504,7 +525,10 @@ def run_b200(args):
     ms = ev0.elapsed_time(ev1)
     launches = eng.kernel_launches - launches0
     # the timed configuration's outputs, decrypted: every ciphertext of the batch against its lookup-table value
-    validation = wl.check(d_out.cpu().numpy().view(np.uint64), vals, idx)
+    h_last = d_out.cpu().numpy().view(np.uint64)
+    validation = wl.check(h_last, vals, idx)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, h_last)
     # per-kernel durations of the dominant kernel, measured live (CUDA events on the launching stream)
     for _ in range(min(args.steps, 5)):
         step()
@@ -653,7 +677,13 @@ def main():
     ap.add_argument("--param-sweep", default="", help="comma-separated classic sets (e.g. 1_1,3_3,4_4): per-set KS-PBS/s on one GPU + CPU oracle, then exit")
     ap.add_argument("--other-sets", default="1_1,3_3", help="classic sets measured briefly after the headline and reported as other_parameter_sets ('' = skip)")
     ap.add_argument("--cpu-sample", type=int, default=-1, help="KS-PBS evaluated by the CPU baseline leg (-1 = host cores x 320, about 10 s; 0 = skip)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the output ciphertexts of the last timed step to DIR/ks_pbs_out.npy (rank 0 only; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.param_sweep:
+        ap.error("--dump-outputs writes the KS-PBS benchmark's outputs; --param-sweep has none to write")
     # stdout carries the one JSON line and nothing else: libraries that write to file descriptor 1 behind Python's back (NCCL's version
     # banner and warnings, OpenMP runtime notices) are sent to stderr; emit() writes the line to the saved descriptor
     global _JSON_FD

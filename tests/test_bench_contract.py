@@ -41,3 +41,30 @@ def test_reference_arm_under_torchrun_rank0_only_all_cores():
                        capture_output=True, text=True, timeout=900, cwd=ROOT, env=env)
     assert r.returncode == 0, r.stderr[-2000:]
     _check(_one_line(r.stdout), 2)
+
+
+def test_dump_outputs_decrypt_and_repeat(tmp_path):
+    """--dump-outputs writes the last timed step's output ciphertexts as float64 torus values: a second run with the same arguments
+    writes the same array, and the words recovered from it decrypt to the lookup-table values of their rows"""
+    import numpy as np
+    import bench
+    dumps = []
+    for run in ("a", "b"):
+        r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                            "--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        dumps.append(np.load(tmp_path / run / "ks_pbs_out.npy"))
+    a, b = dumps
+    assert a.dtype == np.float64 and a.ndim == 2 and a.nbytes <= 64 << 20
+    assert np.array_equal(a, b)
+    assert np.all(np.abs(a) <= 0.5)
+    n = _one_line(r.stdout)["config"]["batch_per_step"]
+    rows = bench.dump_rows(n)
+    assert a.shape[0] == len(rows)
+    wl = bench.Workload("2_2")
+    _, vals, idx = wl.batch(n)
+    w = np.round(a * 2.0**64)
+    w[w >= 2.0**63] -= 2.0**64
+    words = w.astype(np.int64).view(np.uint64)
+    assert words.shape[1] == wl.p.big_dim + 1
+    assert wl.check(words, vals[rows], idx[rows])["ok"]
