@@ -102,6 +102,9 @@ def lib():
         "orc_pbs_f64_pow2_modulus": (None, [_PP, C.c_void_p, _u64p, _u64p, _u64p, C.c_uint32]),
         "orc_pbs_f64_partial": (None, [_PP, C.c_void_p, _u64p, _u64p, _u64p, C.c_size_t]),
         "orc_pbs_exact": (None, [_PP, _u64p, _u64p, _u64p, _u64p]),
+        "orc_pbs_exact_steps": (None, [_PP, _u64p, _u64p, _u64p, _u64p, C.c_size_t]),
+        "orc_pbs_exact_batch": (C.c_int, [_PP, _u64p, _u64p, C.c_void_p, _u64p, _u64p, C.c_size_t, C.c_size_t, C.c_int]),
+        "orc_pbs_f64_batch": (C.c_int, [_PP, C.c_void_p, _u64p, C.c_void_p, _u64p, _u64p, C.c_size_t, C.c_size_t, C.c_int]),
         "orc_ks_pbs_batch": (C.c_int, [_PP, _u64p, C.c_void_p, _u64p, C.c_void_p, _u64p, _u64p, C.c_void_p, C.c_size_t, C.c_int]),
         "orc_max_threads": (C.c_int, []),
         "orc_aes_sbox": (C.POINTER(C.c_uint8), []),
@@ -309,6 +312,46 @@ class ServerKey:
         used = lib().orc_ks_pbs_batch(C.byref(p), self.ksk, self.fourier, luts, idx_ptr, cts, out, ks_ptr, batch, threads)
         self.last_threads = used
         return (out, ks) if want_ks else out
+
+
+class FourierKey:
+    """The oracle's Fourier copy of an explicit standard-domain (multi-bit) BSK, e.g. a test key that is not an encryption."""
+
+    def __init__(self, p: Params, bsk: np.ndarray):
+        self.p = p
+        self.ptr = lib().orc_fourier_bsk_new(C.byref(p), np.ascontiguousarray(bsk, dtype=np.uint64))
+
+    def __del__(self):
+        if getattr(self, "ptr", None):
+            lib().orc_fourier_bsk_free(self.ptr)
+            self.ptr = None
+
+
+def _pbs_batch(fn, p: Params, key, small, luts, lut_idx, max_steps, threads):
+    small = np.ascontiguousarray(small, dtype=np.uint64).reshape(-1, p.lwe_dim + 1)
+    luts = np.ascontiguousarray(luts, dtype=np.uint64).reshape(-1, p.lut_len)
+    out = np.zeros((small.shape[0], p.big_dim + 1), dtype=np.uint64)
+    idx_ptr = None
+    if lut_idx is not None:
+        lut_idx = np.ascontiguousarray(lut_idx, dtype=np.uint32)
+        assert lut_idx.shape == (small.shape[0],) and (small.shape[0] == 0 or int(lut_idx.max()) < luts.shape[0])
+        idx_ptr = lut_idx.ctypes.data_as(C.c_void_p)
+    steps = C.c_size_t(-1).value if max_steps is None else int(max_steps)
+    fn(C.byref(p), key, luts, idx_ptr, small, out, small.shape[0], steps, threads)
+    return out
+
+
+def pbs_exact_batch(p: Params, bsk: np.ndarray, small, luts, lut_idx=None, max_steps=None, threads: int = 0) -> np.ndarray:
+    """Exact integer PBS (classic or multi-bit) of a batch under an explicit standard-domain BSK, stopped after max_steps mask elements /
+    groups (None: the whole rotation).  Cost O(n * (k+1)^2 * l * N * nnz) per ciphertext, nnz = nonzeros per key polynomial."""
+    bsk = np.ascontiguousarray(bsk, dtype=np.uint64)
+    assert bsk.size == lib().orc_bsk_len(C.byref(p))
+    return _pbs_batch(lib().orc_pbs_exact_batch, p, bsk, small, luts, lut_idx, max_steps, threads)
+
+
+def pbs_f64_batch(p: Params, fourier: FourierKey, small, luts, lut_idx=None, max_steps=None, threads: int = 0) -> np.ndarray:
+    """The oracle's f64 PBS (what orc_pbs_f64_partial computes) over a batch, same arguments as pbs_exact_batch."""
+    return _pbs_batch(lib().orc_pbs_f64_batch, p, fourier.ptr, small, luts, lut_idx, max_steps, threads)
 
 
 def decompose(x: int, base_log: int, level: int) -> list[int]:

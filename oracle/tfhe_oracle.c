@@ -855,6 +855,129 @@ void orc_pbs_exact(const orc_params *p, const uint64_t *bsk_std, const uint64_t 
     free(ct0); free(ct1);
 }
 
+/* o += d * g in Z_2^64[X]/(X^N+1), iterating over the nonzero coefficients of g: O(N * nnz(g)), so sparse test keys are cheap */
+ORC_CLONES
+static void negacyclic_mul_add_by_key(uint64_t *restrict o, const uint64_t *restrict d, const uint64_t *restrict g, size_t N) {
+    for (size_t b = 0; b < N; b++) {
+        const uint64_t c = g[b];
+        if (!c) continue;
+        for (size_t a = 0; a < N - b; a++) o[a + b] += d[a] * c;
+        for (size_t a = N - b; a < N; a++) o[a + b - N] -= d[a] * c;
+    }
+}
+
+/* orc_add_external_product_exact with the product above and caller-owned scratch (states: k1*N, digits: N) */
+static void add_external_product_exact_by_key(const orc_params *p, const uint64_t *ggsw_std, uint64_t *out, const uint64_t *glwe,
+                                              uint64_t *states, uint64_t *digits) {
+    size_t N = p->poly_size, k1 = p->glwe_dim + 1, L = p->pbs_level;
+    uint32_t bl = p->pbs_base_log;
+    uint64_t mask = ((uint64_t)1 << bl) - 1;
+    for (size_t j = 0; j < k1 * N; j++)
+        states[j] = orc_closest_representable(glwe[j], bl, p->pbs_level) >> (64 - bl * L);
+    for (size_t lv = L; lv >= 1; lv--) {
+        for (size_t row = 0; row < k1; row++) {
+            for (size_t j = 0; j < N; j++) digits[j] = decompose_one_level(bl, &states[row * N + j], mask);
+            for (size_t col = 0; col < k1; col++)
+                negacyclic_mul_add_by_key(out + col * N, digits, ggsw_std + ((((lv - 1) * k1 + row) * k1) + col) * N, N);
+        }
+    }
+}
+
+/* Exact PBS, classic and multi-bit, stopping after max_steps mask elements (classic) / groups (multi-bit) like orc_pbs_f64_partial.
+ * Classic: the control flow of orc_pbs_exact.  Multi-bit: the order of blind_rotate_f64_steps, with the combined GGSW
+ * G = G_0 + sum_idx X^{sw_idx} * G_idx (prepare_multi_bit_ggsw) built by exact negacyclic monomial products. */
+static void pbs_exact_steps_scratch(const orc_params *p, const uint64_t *bsk_std, const uint64_t *lwe_in, const uint64_t *acc,
+                                    uint64_t *lwe_out, size_t max_steps, uint64_t *ct0, uint64_t *ct1, uint64_t *states,
+                                    uint64_t *digits, uint64_t *G, uint64_t *mono) {
+    size_t N = p->poly_size, k1 = p->glwe_dim + 1, n = p->lwe_dim, gl = ggsw_len(p);
+    uint32_t lgN = ilog2(N);
+    size_t b_hat = (size_t)orc_modulus_switch(lwe_in[n], lgN);
+    for (size_t q = 0; q < k1; q++) orc_monomial_div(ct0 + q * N, acc + q * N, N, b_hat);
+    if (p->grouping_factor == 0) {
+        for (size_t i = 0; i < n && i < max_steps; i++) {
+            if (lwe_in[i] == 0) continue;
+            size_t a_hat = (size_t)orc_modulus_switch(lwe_in[i], lgN);
+            for (size_t q = 0; q < k1; q++) orc_monomial_mul_and_subtract(ct1 + q * N, ct0 + q * N, N, a_hat);
+            add_external_product_exact_by_key(p, bsk_std + i * gl, ct0, ct1, states, digits);
+        }
+    } else {
+        size_t g = p->grouping_factor, per = (size_t)1 << g, groups = n / g;
+        uint64_t *src = ct0, *dst = ct1;
+        for (size_t grp = 0; grp < groups && grp < max_steps; grp++) {
+            const uint64_t *base = bsk_std + grp * per * gl, *mask_elems = lwe_in + grp * g;
+            memcpy(G, base, gl * 8);
+            for (size_t idx = 1; idx < per; idx++) {
+                uint64_t deg = 0;
+                for (size_t mi = 0; mi < g; mi++) deg += (uint64_t)((idx >> (g - (mi + 1))) & 1) * mask_elems[mi];
+                size_t sw = (size_t)orc_modulus_switch(deg, lgN);
+                for (size_t q = 0; q < gl / N; q++) {
+                    orc_monomial_mul(mono, base + idx * gl + q * N, N, sw);
+                    for (size_t j = 0; j < N; j++) G[q * N + j] += mono[j];
+                }
+            }
+            memset(dst, 0, k1 * N * 8);
+            add_external_product_exact_by_key(p, G, dst, src, states, digits);
+            uint64_t *t = src; src = dst; dst = t;
+        }
+        if (src != ct0) memcpy(ct0, src, k1 * N * 8);
+    }
+    orc_sample_extract0(p, ct0, lwe_out);
+}
+
+void orc_pbs_exact_steps(const orc_params *p, const uint64_t *bsk_std, const uint64_t *lwe_in, const uint64_t *acc, uint64_t *lwe_out,
+                         size_t max_steps) {
+    size_t N = p->poly_size, k1 = p->glwe_dim + 1, gl = ggsw_len(p);
+    uint64_t *ct0 = (uint64_t *)malloc(k1 * N * 8), *ct1 = (uint64_t *)malloc(k1 * N * 8), *states = (uint64_t *)malloc(k1 * N * 8);
+    uint64_t *digits = (uint64_t *)malloc(N * 8), *G = (uint64_t *)malloc(gl * 8), *mono = (uint64_t *)malloc(N * 8);
+    pbs_exact_steps_scratch(p, bsk_std, lwe_in, acc, lwe_out, max_steps, ct0, ct1, states, digits, G, mono);
+    free(ct0); free(ct1); free(states); free(digits); free(G); free(mono);
+}
+
+/* batch PBS without keyswitch, one ciphertext per OpenMP thread: exact (f == NULL, integer products on bsk_std) or f64 (f) */
+static int pbs_batch_steps(const orc_params *p, const orc_fourier_bsk *f, const uint64_t *bsk_std, const uint64_t *luts,
+                           const uint32_t *lut_idx, const uint64_t *in, uint64_t *out, size_t batch, size_t max_steps, int threads) {
+    size_t big = (size_t)p->glwe_dim * p->poly_size + 1, small = p->lwe_dim + 1;
+    size_t N = p->poly_size, k1 = p->glwe_dim + 1, gl = ggsw_len(p);
+    (void)get_plan(N);
+    int used = 1;
+#ifdef _OPENMP
+    if (threads <= 0) threads = omp_get_max_threads();
+    used = threads;
+#else
+    (void)threads;
+#endif
+    #pragma omp parallel num_threads(threads)
+    {
+        pbs_scratch s; scratch_init(&s, p);
+        uint64_t *states = (uint64_t *)malloc(k1 * N * 8), *digits = (uint64_t *)malloc(N * 8), *G = (uint64_t *)malloc(gl * 8);
+        #pragma omp for schedule(dynamic, 1)
+        for (long b = 0; b < (long)batch; b++) {
+            const uint64_t *acc = luts + (size_t)(lut_idx ? lut_idx[b] : 0) * k1 * N;
+            const uint64_t *x = in + (size_t)b * small;
+            uint64_t *y = out + (size_t)b * big;
+            if (f) {
+                memcpy(s.ct0, acc, k1 * N * 8);
+                blind_rotate_f64_steps(p, f, x, &s, max_steps);
+                orc_sample_extract0(p, s.ct0, y);
+            } else {
+                pbs_exact_steps_scratch(p, bsk_std, x, acc, y, max_steps, s.ct0, s.ct1, states, digits, G, s.mono);
+            }
+        }
+        free(states); free(digits); free(G); scratch_free(&s);
+    }
+    return used;
+}
+
+int orc_pbs_exact_batch(const orc_params *p, const uint64_t *bsk_std, const uint64_t *luts, const uint32_t *lut_idx,
+                        const uint64_t *in, uint64_t *out, size_t batch, size_t max_steps, int threads) {
+    return pbs_batch_steps(p, NULL, bsk_std, luts, lut_idx, in, out, batch, max_steps, threads);
+}
+
+int orc_pbs_f64_batch(const orc_params *p, const orc_fourier_bsk *f, const uint64_t *luts, const uint32_t *lut_idx,
+                      const uint64_t *in, uint64_t *out, size_t batch, size_t max_steps, int threads) {
+    return pbs_batch_steps(p, f, NULL, luts, lut_idx, in, out, batch, max_steps, threads);
+}
+
 int orc_max_threads(void) {
 #ifdef _OPENMP
     return omp_get_max_threads();

@@ -112,6 +112,16 @@ void orc_pbs_f64(const orc_params *p, const orc_fourier_bsk *f, const uint64_t *
 void orc_pbs_f64_partial(const orc_params *p, const orc_fourier_bsk *f, const uint64_t *lwe_in, const uint64_t *acc, uint64_t *lwe_out,
                          size_t n_steps);
 void orc_pbs_exact(const orc_params *p, const uint64_t *bsk_std, const uint64_t *lwe_in, const uint64_t *acc, uint64_t *lwe_out);
+/* Exact PBS for classic AND multi-bit keys, stopped after max_steps like orc_pbs_f64_partial (SIZE_MAX = whole rotation).  The
+ * polynomial products iterate over the key's nonzero coefficients, O(N * nnz) each: sparse test keys make whole batches affordable. */
+void orc_pbs_exact_steps(const orc_params *p, const uint64_t *bsk_std, const uint64_t *lwe_in, const uint64_t *acc, uint64_t *lwe_out,
+                         size_t max_steps);
+/* batches of the above (no keyswitch), one ciphertext per OpenMP thread; luts: n_luts * (k+1)*N, lut_idx per ct or NULL (LUT 0).
+ * orc_pbs_f64_batch is the same over a Fourier key.  Both return the threads used. */
+int orc_pbs_exact_batch(const orc_params *p, const uint64_t *bsk_std, const uint64_t *luts, const uint32_t *lut_idx,
+                        const uint64_t *in, uint64_t *out, size_t batch, size_t max_steps, int threads);
+int orc_pbs_f64_batch(const orc_params *p, const orc_fourier_bsk *f, const uint64_t *luts, const uint32_t *lut_idx,
+                      const uint64_t *in, uint64_t *out, size_t batch, size_t max_steps, int threads);
 
 /* shortint/server_key/mod.rs:783-857: batched KS -> PBS, one independent ciphertext per OpenMP thread
  * (same structure as benches/core_crypto/pbs_bench.rs:512-536).  luts: n_luts * (k+1)*N, lut_idx per ct.
