@@ -15,7 +15,7 @@ import numpy as np
 _PKG = Path(__file__).resolve().parent
 _SO = _PKG / "libtfhe_b200.so"
 _SOURCES = ["csrc/pbs_v4.cu", "csrc/pbs_v8.cu", "csrc/pbs_multibit_v4.cu", "csrc/pbs_multibit_v8.cu", "csrc/pbs_generic.cu", "csrc/pbs_n512.cu", "csrc/pbs_n8192.cu", "csrc/keyswitch.cu", "csrc/keyswitch_mma.cu", "csrc/keyswitch_tc.cu", "csrc/leveled.cu", "csrc/seeded.cu", "csrc/probe.cu", "csrc/exchange.cu", "csrc/c_api.cu", "csrc/host_api.cu"]
-_HEADERS = ["csrc/fft_core.cuh", "csrc/fft16_core.cuh", "csrc/fft8_core.cuh", "csrc/fft16x_slots.cuh", "csrc/pbs16_common.cuh", "csrc/pbs8_common.cuh", "csrc/ring_helpers.cuh", "csrc/kernels.h", "csrc/ctx.h", "csrc/host/program.h", "csrc/host/radix.h", "csrc/host/strings.h", "../include/tfhe_b200.h"]
+_HEADERS = ["csrc/fft_core.cuh", "csrc/fft16_core.cuh", "csrc/fft8_core.cuh", "csrc/fft16x_slots.cuh", "csrc/pbs16_common.cuh", "csrc/pbs8_common.cuh", "csrc/ring_helpers.cuh", "csrc/kernels.h", "csrc/ctx.h", "csrc/host/program.h", "csrc/host/radix.h", "csrc/host/strings.h", "csrc/host/padded.h", "../include/tfhe_b200.h"]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

@@ -14,6 +14,8 @@
 // (radix_parallel/cmux.rs:211-250), the amount itself being the radix index of a one-hot boundary flag, never a sum that could overflow
 // a block.
 #pragma once
+#include <tuple>
+
 #include "strings.h"
 
 namespace tbh {
@@ -360,6 +362,326 @@ class PaddedStringServerKey {
         FheString acc = s;
         for (size_t k = 1; k < count; ++k) acc = concat(acc, s);
         return acc;
+    }
+
+    // ---- replace / replacen / split / splitn / split_once / rsplit_once: str's methods with a &str pattern ------------------------------
+    // Matches are found left to right and never overlap; the empty pattern matches at every char boundary 0 ..= len.  The pattern is a
+    // padded string (secret length, maybe empty) or a clear one (trivial chars, no padding, so its least length m_min is its length).
+    // The sizes are public bounds: at most M = max_matches(capacity, m_min) matches, so
+    //   replacen returns capacity + min(count, M) * max(0, capacity_to - m_min) chars, and split returns M + 1 parts (splitn: at most n).
+    // Every step is a wide level of independent PBS plus leveled sums; no PBS input exceeds 15 nominal noise units, and every result block
+    // is a PBS output or trivial.
+    struct Pattern {
+        FheString chars;
+        std::string text;      // the clear pattern
+        bool clear = false;
+        size_t min_len() const { return clear ? chars.len() : 0; }
+    };
+    Pattern padded_pattern(const FheString &pat) { Pattern pt; pt.chars = pat; return pt; }
+    Pattern clear_pattern(const std::string &text) { Pattern pt; pt.chars = ssk.trivial_string(text); pt.text = text; pt.clear = true; return pt; }
+    static size_t max_matches(size_t capacity, size_t m_min) { return m_min == 0 ? capacity + 1 : capacity / m_min; }
+
+    bool is_const(const Ct &c, uint64_t v) const { return c.is_trivial() && c.body == v * p.delta(); }
+    Ct and_flags(const Ct &a, const Ct &b) {
+        if (is_const(a, 0) || is_const(b, 0)) return pg.create_trivial(0);
+        if (a.is_trivial()) return b;
+        if (b.is_trivial()) return a;
+        return isk.boolean_bitand(a, b);
+    }
+    // a + b where at most one is non-zero (the sum's degree is `degree`)
+    Ct add_disjoint(const Ct &a, const Ct &b, uint64_t degree) {
+        if (is_const(a, 0)) return b;
+        if (is_const(b, 0)) return a;
+        Ct s = pg.unchecked_add(a, b);
+        s.degree = degree;
+        return s;
+    }
+    Ct keep_block(const Ct &blk, const Ct &flag) {
+        if (is_const(blk, 0) || is_const(flag, 0)) return pg.create_trivial(0);
+        if (flag.is_trivial()) return blk;
+        return pg.pbs_bivariate(blk, flag, [](uint64_t v, uint64_t k) { return (k & 1) ? v : uint64_t(0); });
+    }
+    Radix keep(const Radix &c, const Ct &flag) {
+        Radix r;
+        for (auto &blk : c) r.push_back(keep_block(blk, flag));
+        return r;
+    }
+    // the sum of flags of which at most one is set, its noise kept <= budget: the earliest-ready flags are summed (15 units at a time)
+    // and cleaned first, which keeps the cleaning off the critical path of a chain
+    Ct onehot_sum(std::vector<Ct> t, uint64_t budget) {
+        t.erase(std::remove_if(t.begin(), t.end(), [this](const Ct &c) { return is_const(c, 0); }), t.end());
+        if (t.empty()) return pg.create_trivial(0);
+        const uint64_t cap = p.total_mod() - 1;
+        for (;;) {
+            uint64_t total = 0;
+            for (auto &c : t) total += c.noise;
+            if (total <= budget) break;
+            std::stable_sort(t.begin(), t.end(), [](const Ct &a, const Ct &b) { return a.ready < b.ready; });
+            size_t k = 0;
+            uint64_t noise = 0;
+            while (k < t.size() && noise + t[k].noise <= cap) noise += t[k++].noise;
+            if (k == 0 || (k == 1 && t[0].noise <= 1)) throw std::logic_error("onehot_sum: a flag is too noisy");
+            Ct sum = t[0];
+            for (size_t j = 1; j < k; ++j) sum = pg.unchecked_add(sum, t[j]);
+            t.erase(t.begin(), t.begin() + k);
+            t.push_back(pg.pbs(sum, [](uint64_t x) { return uint64_t(x != 0); }));
+        }
+        Ct sum = t[0];
+        for (size_t j = 1; j < t.size(); ++j) sum = pg.unchecked_add(sum, t[j]);
+        sum.degree = 1;
+        return sum;
+    }
+    // inclusive prefix counts of boolean flags, each a radix of nd digits: Hillis-Steele over the positions, one radix addition
+    // (add_parallelized) per position and step, on only as many digits as the counts of that step can fill
+    std::vector<Radix> prefix_count(const std::vector<Ct> &f, size_t nd) {
+        const size_t n = f.size();
+        std::vector<Radix> c(n);
+        for (size_t i = 0; i < n; ++i) {
+            c[i].push_back(f[i]);
+            while (c[i].size() < nd) c[i].push_back(pg.create_trivial(0));
+        }
+        for (size_t d = 1; d < n; d *= 2) {
+            const size_t used = std::min(nd, digits_for(std::min(2 * d, n)));
+            std::vector<Radix> nxt = c;
+            for (size_t i = d; i < n; ++i) {
+                Radix s = isk.add(Radix(c[i].begin(), c[i].begin() + used), Radix(c[i - d].begin(), c[i - d].begin() + used));
+                while (s.size() < nd) s.push_back(pg.create_trivial(0));
+                nxt[i] = s;
+            }
+            c.swap(nxt);
+        }
+        return c;
+    }
+    // sign of (digits - c): 0 less, 1 equal, 2 greater.  Pairs of digits are compared with c by table lookup and the signs reduced with
+    // the comparator's tree; nothing is subtracted, so no value reaches the padding bit
+    Ct scalar_sign(const Radix &digits, uint64_t c) {
+        std::vector<Ct> packed = isk.pack_pairs(digits), signs;
+        for (size_t i = 0; i < packed.size(); ++i) {
+            const uint64_t mod = 2 * i + 1 < digits.size() ? uint64_t(p.msg_mod) * p.msg_mod : p.msg_mod, cv = c % mod;
+            c /= mod;
+            signs.push_back(pg.pbs(packed[i], [cv](uint64_t x) { return x < cv ? uint64_t(0) : (x == cv ? uint64_t(1) : uint64_t(2)); }));
+        }
+        if (c != 0) return pg.create_trivial(IntegerServerKey::IS_INFERIOR);
+        return isk.reduce_signs(signs);
+    }
+    Radix trivial_radix(uint64_t v, size_t nd) {
+        Radix r;
+        for (size_t b = 0; b < nd; ++b) r.push_back(pg.create_trivial((v >> (2 * b)) & 3));
+        return r;
+    }
+
+    struct Matches {
+        std::vector<Ct> raw;         // windows 0 ..= capacity: the pattern occurs at w (and w is inside the string or at its end)
+        std::vector<Ct> over, cov;   // d = 0 .. cap_pat - 1: matches d apart can overlap (d >= 1) / a match covers the char d after its start
+    };
+    Matches find_all(const FheString &hay, const Pattern &pt) {
+        const size_t n = hay.len(), m = pt.chars.len();
+        Matches r;
+        r.raw.assign(n + 1, pg.create_trivial(0));
+        if (m == 0) {
+            std::vector<Ct> nz = nonzero_flags(hay);
+            r.raw[0] = pg.create_trivial(1);
+            for (size_t w = 1; w <= n; ++w) r.raw[w] = nz[w - 1];
+            return r;
+        }
+        if (pt.clear) {
+            // a non-empty clear pattern starts with a non-zero char, so it never matches in the padding.  Two matches d apart can both be
+            // candidates only if d is a period of the pattern (it has a border of length m - d); every other shift needs no check
+            std::vector<Ct> mw = ssk.window_matches(hay, pt.chars);   // windows 0 ..= n - m
+            for (size_t w = 0; w < mw.size(); ++w) r.raw[w] = mw[w];
+            for (size_t d = 0; d < m; ++d) {
+                r.cov.push_back(pg.create_trivial(1));
+                r.over.push_back(pg.create_trivial(d > 0 && pt.text.compare(d, m - d, pt.text, 0, m - d) == 0));
+            }
+            return r;
+        }
+        // padded: as find -- a window must start inside the string or right at its end, which only matters for the empty pattern
+        std::vector<Ct> pz = zero_flags(pt.chars), nz = nonzero_flags(hay);
+        for (size_t w = 0; w <= n; ++w) {
+            Ct mw = w < n ? window_match(hay, pt.chars, w, pz) : isk.are_all_comparisons_block_true(pz);
+            r.raw[w] = w > 0 ? isk.boolean_bitand(mw, nz[w - 1]) : mw;
+        }
+        for (size_t d = 0; d < m; ++d) r.cov.push_back(isk.boolean_bitnot(pz[d]));   // [the pattern is longer than d]
+        r.over = r.cov;
+        return r;
+    }
+    // leftmost non-overlapping matches: acc[w] = raw[w] AND NOT OR_{1 <= d < cap_pat} (acc[w - d] AND over[d]).  A chain over w where some
+    // over[d] can be set; with a clear pattern that has no proper border every over[d] is trivially 0 and acc = raw.
+    std::vector<Ct> non_overlapping(const std::vector<Ct> &raw, const std::vector<Ct> &over) {
+        std::vector<Ct> acc(raw.size());
+        for (size_t w = 0; w < raw.size(); ++w) {
+            acc[w] = raw[w];
+            if (is_const(raw[w], 0)) continue;
+            std::vector<Ct> t;
+            for (size_t d = 1; d < over.size() && d <= w; ++d) t.push_back(and_flags(acc[w - d], over[d]));
+            Ct blocked = onehot_sum(t, p.total_mod() - 1 - raw[w].noise);   // at most one accepted match covers w
+            if (is_const(blocked, 0)) continue;
+            acc[w] = pg.pbs(pg.unchecked_add(isk.boolean_bitnot(raw[w]), blocked), [](uint64_t x) { return uint64_t(x == 0); });
+        }
+        return acc;
+    }
+    // covered[i] = OR_d (starts[i - d] AND cov[d]) for the chars i < n; the starts never overlap, so this is a sum (noise <= 2)
+    std::vector<Ct> covered(const std::vector<Ct> &starts, const std::vector<Ct> &cov, size_t n) {
+        std::vector<Ct> out(n);
+        for (size_t i = 0; i < n; ++i) {
+            std::vector<Ct> t;
+            for (size_t d = 0; d < cov.size() && d <= i; ++d) t.push_back(and_flags(starts[i - d], cov[d]));
+            out[i] = onehot_sum(t, 2);
+        }
+        return out;
+    }
+    // the first `limit` of the accepted matches: acc[w] AND [count of accepted matches up to w <= limit]
+    std::vector<Ct> first_matches(const std::vector<Ct> &acc, const std::vector<Radix> &cnt, size_t limit) {
+        std::vector<Ct> lim(acc.size());
+        for (size_t w = 0; w < acc.size(); ++w)
+            lim[w] = is_const(acc[w], 0) ? acc[w]
+                                         : pg.pbs_bivariate(scalar_sign(cnt[w], limit), acc[w], [](uint64_t s, uint64_t a) { return uint64_t(s != 2 && (a & 1)); });
+        return lim;
+    }
+
+    // removes the zero chars of s in order and returns the first out_len positions.  Char j moves left by the number D_j of zero chars
+    // before it, one bit of D_j per stage, least significant first.  For non-zero chars j < j', D_j' - D_j <= j' - j - 1, so their
+    // positions stay strictly increasing after every stage: no two chars ever meet, a stage is a sum of two keep_if per block, and the
+    // remaining bits of D_j travel with their char.
+    FheString compact(const FheString &s, size_t out_len) {
+        const size_t E = s.len();
+        FheString out;
+        if (E == 0) return extend(out, out_len);
+        std::vector<Ct> z(E);
+        for (size_t j = 0; j < E; ++j) z[j] = is_zero(s.chars[j]);
+        size_t T = 0;
+        while ((size_t(1) << T) <= E - 1) ++T;
+        std::vector<Radix> D = prefix_count(z, digits_for(E));
+        std::vector<std::vector<Ct>> B(T, std::vector<Ct>(E));
+        for (size_t t = 0; t < T; ++t)
+            for (size_t j = 0; j < E; ++j)
+                B[t][j] = pg.pbs_bivariate(D[j][t / 2], z[j], [t](uint64_t d, uint64_t zz) { return (zz & 1) ? uint64_t(0) : (d >> (t % 2)) & 1; });
+        FheString cur = s;
+        for (size_t t = 0; t < T; ++t) {
+            const size_t k = size_t(1) << t, reach = (size_t(1) << T) - (size_t(2) << t);   // what the later stages can still move a char
+            const size_t live = std::min(E, out_len + reach);
+            FheString nxt;
+            nxt.chars.assign(E, trivial_char(0));
+            std::vector<std::vector<Ct>> nB(T, std::vector<Ct>(E, pg.create_trivial(0)));
+            for (size_t i = 0; i < live; ++i) {
+                const Ct stay = isk.boolean_bitnot(B[t][i]);
+                const bool src = i + k < E;
+                const Ct zero = pg.create_trivial(0), move = src ? B[t][i + k] : zero;
+                for (size_t b = 0; b < 4; ++b)
+                    nxt.chars[i][b] = add_disjoint(keep_block(cur.chars[i][b], stay), src ? keep_block(cur.chars[i + k][b], move) : zero, p.msg_mod - 1);
+                for (size_t u = t + 1; u < T; ++u)
+                    nB[u][i] = add_disjoint(and_flags(B[u][i], stay), src ? and_flags(B[u][i + k], move) : zero, 1);
+            }
+            cur = nxt;
+            B = nB;
+        }
+        for (size_t i = 0; i < std::min(out_len, E); ++i) {
+            Radix c;
+            for (auto &blk : cur.chars[i])
+                c.push_back(blk.noise <= 1 && blk.degree < p.msg_mod ? blk : pg.pbs(blk, [this](uint64_t x) { return x % p.msg_mod; }));
+            out.chars.push_back(c);
+        }
+        return extend(out, out_len);
+    }
+
+    // replacen (count = SIZE_MAX: replace).  Slot i of the expanded string holds `to` if an accepted match starts at i, then s[i] unless a
+    // match covers it; compacting the zero chars away gives the result
+    FheString replace(const FheString &s, const Pattern &pt, const FheString &to, size_t count) {
+        const size_t n = s.len(), m_min = pt.min_len(), M = max_matches(n, m_min);
+        count = std::min(count, M);
+        const size_t out_len = n + count * (to.len() > m_min ? to.len() - m_min : 0);
+        if (count == 0) return s;
+        Matches mt = find_all(s, pt);
+        std::vector<Ct> acc = non_overlapping(mt.raw, mt.over);
+        if (count < M) acc = first_matches(acc, prefix_count(acc, digits_for(M)), count);
+        std::vector<Ct> cov = covered(acc, mt.cov, n);
+        FheString ex;   // chars known to be zero are left out: compaction removes them anyway
+        for (size_t i = 0; i <= n; ++i) {
+            if (!is_const(acc[i], 0))
+                for (auto &c : to.chars) ex.chars.push_back(keep(c, acc[i]));
+            if (i < n && !is_const(cov[i], 1)) ex.chars.push_back(keep(s.chars[i], isk.boolean_bitnot(cov[i])));
+        }
+        return compact(ex, out_len);
+    }
+
+    // the chars of s selected by `in` -- one contiguous run, which may reach into the padding -- moved to the start
+    FheString part(const FheString &s, const std::vector<Ct> &in) {
+        const size_t n = s.len();
+        FheString masked;
+        for (size_t i = 0; i < n; ++i) masked.chars.push_back(keep(s.chars[i], in[i]));
+        if (n <= 1) return masked;
+        std::vector<Ct> st(n);   // one-hot: the run starts at i
+        st[0] = in[0];
+        for (size_t i = 1; i < n; ++i)
+            st[i] = pg.pbs(pg.unchecked_add(in[i], pg.unchecked_scalar_mul(in[i - 1], 2)), [](uint64_t x) { return uint64_t(x == 1); });
+        size_t n_bits = 0;
+        while ((size_t(1) << n_bits) <= n - 1) ++n_bits;
+        Radix start = onehot_to_radix(st, digits_for(n - 1), [](size_t w) { return uint64_t(w); });
+        return shift(masked, bits_of(start, n_bits), true);
+    }
+
+    // splitn (n_parts = SIZE_MAX: split): (part count as digits_for(P) digits, P parts of capacity chars), P = min(M + 1, n_parts).  Char i
+    // belongs to part min(#accepted matches at or before i, P - 1) unless a match covers it; parts past the count are empty.
+    std::pair<Radix, std::vector<FheString>> split(const FheString &s, const Pattern &pt, size_t n_parts) {
+        const size_t n = s.len(), M = max_matches(n, pt.min_len()), P = std::min(M + 1, n_parts), nd = digits_for(P);
+        std::vector<FheString> parts;
+        if (P == 0) return {trivial_radix(0, nd), parts};
+        if (P == 1) { parts.push_back(s); return {trivial_radix(1, nd), parts}; }
+        const size_t last = P - 1;
+        Matches mt = find_all(s, pt);
+        std::vector<Ct> acc = non_overlapping(mt.raw, mt.over);
+        std::vector<Radix> cnt = prefix_count(acc, digits_for(M));   // counts of every accepted match, up to M
+        std::vector<Ct> lim = last < M ? first_matches(acc, cnt, last) : acc;
+        std::vector<Ct> cov = covered(lim, mt.cov, n);
+        // count = min(#matches, last) + 1: when there are fewer than `last` matches, their number fits nd digits
+        Radix total(cnt[n].begin(), cnt[n].begin() + std::min(nd, cnt[n].size()));
+        while (total.size() < nd) total.push_back(pg.create_trivial(0));
+        Radix count = isk.add(total, trivial_radix(1, nd));
+        if (last < M) {
+            Ct more = pg.pbs(scalar_sign(cnt[n], last), [](uint64_t x) { return uint64_t(x != 0); });
+            count = isk.if_then_else(more, trivial_radix(P, nd), count);
+        }
+        for (size_t k = 0; k < P; ++k) {
+            std::vector<Ct> in(n);
+            for (size_t i = 0; i < n; ++i) {
+                const bool tail = k == last;
+                in[i] = pg.pbs_bivariate(scalar_sign(cnt[i], k), cov[i], [tail](uint64_t sg, uint64_t c) {
+                    return uint64_t((tail ? sg != 0 : sg == 1) && !(c & 1));
+                });
+            }
+            if (k == 0) {   // part 0 starts at 0
+                FheString p0;
+                for (size_t i = 0; i < n; ++i) p0.chars.push_back(keep(s.chars[i], in[i]));
+                parts.push_back(p0);
+            } else parts.push_back(part(s, in));
+        }
+        return {count, parts};
+    }
+
+    // split_once / rsplit_once: (found, before, after) around the first (last: the last, as rfind finds it) match; both strings are empty
+    // when there is none
+    std::tuple<BooleanBlock, FheString, FheString> split_once(const FheString &s, const Pattern &pt, bool last) {
+        const size_t n = s.len();
+        Matches mt = find_all(s, pt);
+        std::vector<Ct> raw = mt.raw;
+        if (last) std::reverse(raw.begin(), raw.end());
+        std::vector<Ct> any = prefix_or(raw, true);   // [a match at or before w] (last: at or after w)
+        if (last) std::reverse(any.begin(), any.end());
+        auto flag_sub = [this](const Ct &a, const Ct &b) { Ct r = pg.lwe_sub(a, b); r.degree = 1; return r; };
+        const Ct found = last ? any[0] : any[n];
+        std::vector<Ct> start(n + 1);                  // one-hot: the splitting match
+        for (size_t w = 0; w <= n; ++w) {
+            if (last) start[w] = w < n ? flag_sub(any[w], any[w + 1]) : any[n];
+            else start[w] = w > 0 ? flag_sub(any[w], any[w - 1]) : any[0];
+        }
+        std::vector<Ct> cov = covered(start, mt.cov, n), before(n), after(n);
+        for (size_t i = 0; i < n; ++i) {
+            before[i] = last ? any[i + 1] : flag_sub(found, any[i]);
+            after[i] = last ? flag_sub(flag_sub(found, any[i + 1]), cov[i]) : flag_sub(any[i], cov[i]);
+        }
+        FheString b;
+        for (size_t i = 0; i < n; ++i) b.chars.push_back(keep(s.chars[i], before[i]));
+        return {found, b, part(s, after)};
     }
 
     Program &pg;

@@ -6,6 +6,7 @@
 #include "ctx.h"
 #include "host/padded.h"
 
+#include <cstring>
 #include <memory>
 
 using tbc::DevBuf;
@@ -42,6 +43,65 @@ tbh::Radix input_radix(tbh::Program &pg, size_t n) {
 
 void output_radix(tbh::Program &pg, const tbh::Radix &r) { for (auto &b : r) pg.output(b); }
 void output_string(tbh::Program &pg, const tbh::FheString &s) { for (auto &c : s.chars) output_radix(pg, c); }
+
+// pstring_{replace,replacen} {capacity, capacity_from, capacity_to[, count]}: inputs s, from, to -> the result string
+// pstring_{split,splitn} {capacity, capacity_pat[, n]}: inputs s, pat -> part count, then the parts
+// pstring_{split_once,rsplit_once} {capacity, capacity_pat}: inputs s, pat -> found, before, after
+// A clear pattern replaces the `from` / `pat` input; its capacity argument must be its length.
+bool record_split_replace(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh::StringServerKey &ssk, const std::string &op,
+                          const std::string &f, const uint64_t *a, size_t na, const char *clear, std::string &err) {
+    const bool rep = f == "replace" || f == "replacen";
+    const size_t n_args = f == "replacen" ? 4 : (f == "replace" || f == "splitn") ? 3 : 2;
+    if (na < n_args) {
+        static const std::map<std::string, std::string> names = {
+            {"replace", "{capacity, capacity_from, capacity_to}"}, {"replacen", "{capacity, capacity_from, capacity_to, count}"},
+            {"split", "{capacity, capacity_pat}"}, {"splitn", "{capacity, capacity_pat, n}"},
+            {"split_once", "{capacity, capacity_pat}"}, {"rsplit_once", "{capacity, capacity_pat}"}};
+        err = op + ": expected " + std::to_string(n_args) + " integer arguments " + names.at(f);
+        return false;
+    }
+    const uint64_t cap = a[0], cap_pat = a[1], cap_to = rep ? a[2] : 0;
+    if (clear && std::strlen(clear) != cap_pat) {
+        err = op + ": the pattern capacity " + std::to_string(cap_pat) + " differs from the clear pattern's length " + std::to_string(std::strlen(clear));
+        return false;
+    }
+    // sizes arrive from outside: bound the result and the intermediate strings before anything is recorded (slot indices are 32-bit)
+    constexpr uint64_t kMaxChars = uint64_t(1) << 20;
+    if (cap > kMaxChars || cap_pat > kMaxChars || cap_to > kMaxChars) {
+        err = op + ": capacities are limited to " + std::to_string(kMaxChars) + " chars";
+        return false;
+    }
+    const uint64_t m_min = clear ? cap_pat : 0, M = tbh::PaddedStringServerKey::max_matches(cap, m_min);
+    unsigned __int128 chars;   // the largest string the program holds at once
+    if (rep) {
+        const uint64_t count = f == "replacen" ? std::min<uint64_t>(a[3], M) : M;
+        chars = (unsigned __int128)(cap + 1) * (cap_to + 1);                                        // the expanded string
+        chars = std::max(chars, (unsigned __int128)cap + (unsigned __int128)count * (cap_to > m_min ? cap_to - m_min : 0));
+    } else {
+        const uint64_t P = f == "splitn" ? std::min<uint64_t>(M + 1, a[2]) : (f == "split" ? M + 1 : 2);
+        chars = (unsigned __int128)P * cap;
+    }
+    if (chars > kMaxChars) {
+        err = op + ": the result or the expanded string would exceed " + std::to_string(kMaxChars) + " chars";
+        return false;
+    }
+    tbh::FheString s = ssk.input_string(cap);
+    const tbh::PaddedStringServerKey::Pattern pt = clear ? psk.clear_pattern(clear) : psk.padded_pattern(ssk.input_string(cap_pat));
+    if (rep) {
+        tbh::FheString to = ssk.input_string(cap_to);
+        output_string(pg, psk.replace(s, pt, to, f == "replacen" ? a[3] : SIZE_MAX));
+    } else if (f == "split" || f == "splitn") {
+        auto r = psk.split(s, pt, f == "splitn" ? a[2] : SIZE_MAX);
+        output_radix(pg, r.first);
+        for (auto &part : r.second) output_string(pg, part);
+    } else {
+        auto r = psk.split_once(s, pt, f == "rsplit_once");
+        pg.output(std::get<0>(r));
+        output_string(pg, std::get<1>(r));
+        output_string(pg, std::get<2>(r));
+    }
+    return true;
+}
 
 // records `op`; returns false with a message when the op / arguments are unknown
 bool record(tfhe_b200_program &h, const std::string &op_in, const uint64_t *a, size_t na, const char *clear, std::string &err) {
@@ -194,6 +254,8 @@ bool record(tfhe_b200_program &h, const std::string &op_in, const uint64_t *a, s
         if (!need(1)) return false;
         tbh::PaddedStringServerKey psk(pg);
         const std::string f = op.substr(8);
+        if (f == "replace" || f == "replacen" || f == "split" || f == "splitn" || f == "split_once" || f == "rsplit_once")
+            return record_split_replace(pg, psk, ssk, op, f, a, na, clear, err);
         tbh::FheString s = ssk.input_string(a[0]);
         if (f == "len") { output_radix(pg, psk.len(s)); return true; }
         if (f == "is_empty") { pg.output(psk.is_empty(s)); return true; }

@@ -154,6 +154,16 @@ int tfhe_b200_pbs_batch_partial(tfhe_b200_ctx *ctx, const uint64_t *lwe_small, c
  *   string_{eq,ne,lt,le,contains}_many {len_a, len_b, count}   (count independent pairs in one program)
  *   pstring_{len,is_empty,trim_start,trim_end,trim} {capacity}     pstring_{strip_prefix,strip_suffix} {capacity} + clear pattern
  *   pstring_{eq,ne,lt,le,gt,ge,contains,starts_with,ends_with,find,rfind,concat} {capacity_a, capacity_b}     pstring_repeat {capacity, count}
+ *   pstring_replace {capacity, capacity_from, capacity_to}  pstring_replacen {capacity, capacity_from, capacity_to, count}: inputs s, from,
+ *     to -> C = capacity + min(count, M) * max(0, capacity_to - m_min) chars (replace: count unbounded)
+ *   pstring_split {capacity, capacity_pat}  pstring_splitn {capacity, capacity_pat, n}: inputs s, pat -> the part count (ceil(log4(P + 1))
+ *     blocks), then P parts of capacity chars, P = M + 1 (splitn: min(M + 1, n); the last part is the unsplit rest; n = 0: count 0)
+ *   pstring_split_once / pstring_rsplit_once {capacity, capacity_pat}: inputs s, pat -> found, before, after (capacity chars each; both
+ *     empty when nothing is found).  rsplit_once splits at the last match as rfind finds it
+ *     -- Rust's str methods with a &str pattern: leftmost non-overlapping matches, the empty pattern matching at every char boundary
+ *        0 ..= len.  With clear_operand != NULL it is the pattern (from / pat, not an input) and capacity_from / capacity_pat must equal
+ *        its length.  m_min is the least pattern length (0 for a padded pattern, the length of a clear one) and M the most matches:
+ *        capacity + 1 when m_min = 0, else capacity / m_min.  Parts past the count are all zero.
  *     -- NULL-PADDED strings: public capacity, secret length, content followed by zero bytes (host/padded.h); len returns a radix of
  *        ceil(log4(capacity + 1)) blocks, the string-valued ops return 4 blocks per char of the result capacity
  * Appending "_packed" to a string op (or radix_eq) selects packed block equalities: one PBS per PAIR of blocks built from
