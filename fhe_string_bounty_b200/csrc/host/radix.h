@@ -24,9 +24,15 @@ class IntegerServerKey {
     explicit IntegerServerKey(Program &prog) : pg(prog), p(prog.params()) {}
 
     // ---- boolean count-trees (scalar_comparison.rs:147-240) -------------------------------------------------
+    // booleans summed per PBS: total_mod - 1.  With a message space of two values a sum of one boolean never shrinks the list.
+    size_t count_tree_arity(size_t n_blocks) const {
+        const size_t max_value = p.total_mod() - 1;
+        if (n_blocks > 1 && max_value < 2) throw std::invalid_argument("boolean reduction: needs a message space of at least 3 values");
+        return max_value;
+    }
     Ct are_all_comparisons_block_true(std::vector<Ct> blocks) {
         if (blocks.empty()) return pg.create_trivial(1);
-        const size_t max_value = p.total_mod() - 1;
+        const size_t max_value = count_tree_arity(blocks.size());
         while (blocks.size() > 1) {
             std::vector<Ct> next;
             for (size_t i = 0; i < blocks.size(); i += max_value) {
@@ -41,7 +47,7 @@ class IntegerServerKey {
     }
     Ct is_at_least_one_comparisons_block_true(std::vector<Ct> blocks) {
         if (blocks.empty()) return pg.create_trivial(1);   // sic: scalar_comparison.rs:204-206
-        const size_t max_value = p.total_mod() - 1;
+        const size_t max_value = count_tree_arity(blocks.size());
         while (blocks.size() > 1) {
             std::vector<Ct> next;
             for (size_t i = 0; i < blocks.size(); i += max_value) {
@@ -81,9 +87,13 @@ class IntegerServerKey {
     std::vector<Ct> packed_block_equalities(const Radix &lhs, const Radix &rhs) {
         if (lhs.size() != rhs.size()) throw std::invalid_argument("radix size mismatch");
         std::vector<Ct> pl = pack_pairs(lhs), pr = pack_pairs(rhs), out;
+        // the difference lies in (-total_mod, total_mod) only if both packed operands fit the message space (carry_mod >= msg_mod for
+        // clean blocks); otherwise hi * msg_mod + lo wraps and distinct pairs compare equal: one PBS per block instead
+        for (size_t i = 0; i < pl.size(); ++i)
+            if (pl[i].degree >= p.total_mod() || pr[i].degree >= p.total_mod()) return block_equalities(lhs, rhs);
         for (size_t i = 0; i < pl.size(); ++i) {
             Ct d = pg.lwe_sub(pl[i], pr[i]);
-            d.degree = p.total_mod() - 1;
+            d.degree = p.total_mod() - 1;      // negative differences reach the padding bit on purpose (see above)
             out.push_back(pg.pbs(d, [](uint64_t x) { return uint64_t(x == 0); }));
         }
         return out;
@@ -216,11 +226,14 @@ class IntegerServerKey {
     }
 
     // ---- carry propagation (radix_parallel/add.rs:518-603,724-772), always the parallel form (SURVEY App. B note) ---------------
-    // blocks hold message + carry (degree < total_mod); returns clean blocks of the propagated number (mod 4^B)
+    // blocks hold message + at most one carry (degree <= 2 msg_mod - 2, so that block + incoming carry <= 2 msg_mod - 1 carries out at
+    // most one); returns clean blocks of the propagated number (mod msg_mod^B)
     Radix full_propagate(const Radix &in) {
         const uint64_t m = p.msg_mod;
         const size_t B = in.size();
         if (B == 0) return in;
+        for (auto &b : in)
+            if (b.degree > 2 * m - 2) throw std::logic_error("single-carry propagation on a block of degree " + std::to_string(b.degree));
         enum : uint64_t { NONE = 0, GENERATED = 1, PROPAGATED = 2 };   // add.rs:19-34 OutputCarry
         // generate_init_carry_array (add.rs:724-772): first block can only generate
         std::vector<Ct> state(B);
@@ -229,10 +242,16 @@ class IntegerServerKey {
             else state[i] = pg.pbs(in[i], [m](uint64_t x) { return x >= m ? uint64_t(GENERATED) : (x == m - 1 ? uint64_t(PROPAGATED) : uint64_t(NONE)); });
         }
         // Hillis-Steele inclusive prefix (add.rs:572-603) with prefix_sum_carry_propagation (add.rs:36-42)
+        // the pair (cur, prev) of states in {0, 1, 2} is packed as cur * msg_mod + prev; with msg_mod = 2 that is not injective, so the
+        // one-bit sets pack it as cur * 3 + prev (a univariate LUT on [0, 8]: a message space of at least 9 values)
+        auto combine = [](uint64_t cur, uint64_t prev) { return cur == PROPAGATED ? prev : cur; };
         for (size_t d = 1; d < B; d *= 2) {
             std::vector<Ct> next = state;
-            for (size_t i = d; i < B; ++i)
-                next[i] = pg.pbs_bivariate(state[i], state[i - d], [](uint64_t cur, uint64_t prev) { return cur == PROPAGATED ? prev : cur; });
+            for (size_t i = d; i < B; ++i) {
+                if (m >= 3) next[i] = pg.pbs_bivariate(state[i], state[i - d], combine);
+                else next[i] = pg.pbs(pg.unchecked_add(pg.unchecked_scalar_mul(state[i], 3), state[i - d]),
+                                      [combine](uint64_t x) { return x < 9 ? combine(x / 3, x % 3) : uint64_t(0); });
+            }
             state.swap(next);
         }
         // add the incoming carry and extract the message (add.rs:544-570)
@@ -247,21 +266,26 @@ class IntegerServerKey {
         return out;
     }
     // full_propagate_parallelized on blocks of ANY degree < total_mod (radix_parallel/mod.rs:88-156, parallel branch): message_extract
-    // and carry_extract of every block in one level, the carries added one block up (message + carry <= 2 (msg_mod - 1)), then the
-    // single-carry propagation above.  Blocks whose degree already allows a single carry go straight to it.
-    Radix full_propagate_any_degree(const Radix &in) {
+    // and carry_extract of every block in one level, the carries added one block up, then the single-carry propagation above.  One
+    // extraction leaves message + carry <= (msg_mod - 1) + (d / msg_mod); when carry_mod > msg_mod that can still exceed 2 msg_mod - 2,
+    // so the extraction repeats until every block allows a single carry.  Blocks that already do go straight to it.
+    Radix full_propagate_any_degree(Radix in) {
         const uint64_t m = p.msg_mod;
-        uint64_t worst = 0;
-        for (auto &b : in) worst = std::max(worst, b.degree);
-        if (worst <= 2 * m - 1) return full_propagate(in);       // x <= 2 msg_mod - 1: at most one carry out of every block
-        Radix msg(in.size()), carry(in.size());
-        for (size_t i = 0; i < in.size(); ++i) {
-            msg[i] = pg.pbs(in[i], [m](uint64_t x) { return x % m; });
-            if (i + 1 < in.size()) carry[i] = pg.pbs(in[i], [m](uint64_t x) { return x / m; });
+        auto worst_of = [](const Radix &r) { uint64_t w = 0; for (auto &b : r) w = std::max(w, b.degree); return w; };
+        while (worst_of(in) > 2 * m - 2) {
+            Radix msg(in.size()), carry(in.size());
+            for (size_t i = 0; i < in.size(); ++i) {
+                msg[i] = pg.pbs(in[i], [m](uint64_t x) { return x % m; });
+                msg[i].degree = std::min(in[i].degree, m - 1);
+                if (i + 1 < in.size()) {
+                    carry[i] = pg.pbs(in[i], [m](uint64_t x) { return x / m; });
+                    carry[i].degree = in[i].degree / m;
+                }
+            }
+            for (size_t i = 1; i < in.size(); ++i) msg[i] = pg.unchecked_add(msg[i], carry[i - 1]);
+            in.swap(msg);
         }
-        Radix sum(in.size());
-        for (size_t i = 0; i < in.size(); ++i) sum[i] = i == 0 ? msg[i] : pg.unchecked_add(msg[i], carry[i - 1]);
-        return full_propagate(sum);
+        return full_propagate(in);
     }
     bool block_carries_are_empty(const Radix &r) const {      // integer/ciphertext/base.rs: every degree < msg_mod
         for (auto &b : r) if (b.degree >= p.msg_mod) return false;

@@ -46,6 +46,8 @@ class Program:
         h = C.c_void_p()
         if isinstance(clear, str):
             clear = clear.encode("latin-1")
+        if clear is not None and b"\0" in clear:   # the C ABI takes a NUL-terminated string: the pattern would be cut short
+            raise ValueError(f"{op}: a clear operand cannot contain a NUL char")
         rc = self.lib.tfhe_b200_program_build(C.byref(self.p), op.encode(), a.ctypes.data if a.size else None, a.size, clear, C.byref(h))
         if rc != 0:
             raise NativeError(self.lib.tfhe_b200_last_error().decode())
