@@ -101,10 +101,10 @@ def pbs_steps(p):
     return p.lwe_dim // p.grouping_factor if p.grouping_factor else p.lwe_dim
 
 
-def lattice_bsk(orc, p, seed, nnz=8, cmax=127):
+def lattice_bsk(orc, p, seed, nnz=8, cmax=127, shift=None):
     """standard-domain (multi-bit) BSK of small multiples c * 2^s, 0 < |c| <= cmax, at nnz random positions per polynomial (nnz=None: every
-    coefficient drawn from [-cmax, cmax])"""
-    N, s = p.poly_size, lattice_shift(p)
+    coefficient drawn from [-cmax, cmax]); s = lattice_shift(p) unless `shift` is given (coarse_bsk_shift(p) for whole programs)"""
+    N, s = p.poly_size, lattice_shift(p) if shift is None else shift
     n_polys = lib_bsk_len(orc, p) // N
     rng = np.random.default_rng(seed)
     if nnz is None:
@@ -225,3 +225,136 @@ def assert_on_lattice(got, exact, s, label, run_rows=None, ref_rows=None, n_step
           f"(half lattice 2^{s - 1}, bound 2^{bound})")
     assert res <= 2**bound, f"{label}: residual 2^{np.log2(res):.1f} > 2^{bound}"
     return res
+
+
+# ---- coarse lattice for whole programs (DESIGN section 4): every word that can reach a keyswitch is a multiple of 2^u, u = 63 - log2 N -----
+# 2^u is the unit of the PBS modulus switch.  With the BSK, the program inputs and the KSK body column on 2^u (and the accumulators and
+# bodies on delta >= 2^u), the exact rotation stays on 2^u, the keyswitch digits of (exact + eps) are those of the exact word, the small
+# mask words are exact and the modulus switch rounds eps away from the body: a program's GPU outputs rounded to 2^u must equal the exact
+# integer executor's (run_program_exact with orc.pbs_exact_batch) on every word, as long as sum|coef| * eps stays below the headroom.
+
+def coarse_shift(p):
+    """u = 63 - log2 N, asserting the three conditions of the argument: u >= 64 - B_pbs * l_pbs (the rotation lattice of lattice_shift),
+    u >= 64 - B_ks * l_ks (every PBS output word is representable by the keyswitch decomposition) and delta >= 2^u"""
+    lg = int(p.poly_size).bit_length() - 1
+    u = 63 - lg
+    tm = p.msg_mod * p.carry_mod
+    assert u >= lattice_shift(p), (u, lattice_shift(p))
+    assert u >= 64 - p.ks_base_log * p.ks_level, (u, p.ks_base_log, p.ks_level)
+    assert tm & (tm - 1) == 0 and (1 << 63) // tm >= 1 << u, (tm, u)
+    return u
+
+
+def coarse_bsk_shift(p):
+    """64 - B_pbs: a level-j digit of a word on 2^a is a multiple of 2^(a - 64 + j * B_pbs), so GGSW rows on 2^(64 - B_pbs) keep every
+    external product on 2^a, and an accumulator on the delta lattice stays there through the whole rotation.  (Rows on 2^u would not do:
+    at 2_2 a digit of a delta-lattice word is a multiple of 2^18, and 2^18 * 2^52 vanishes modulo 2^64, so the outputs would not
+    depend on the BSK or on the mask.)"""
+    return 64 - p.pbs_base_log
+
+
+def coarse_headroom_log2(p):
+    """log2 of the largest |eps| the hand-off tolerates: half the coarser of 2^u and the keyswitch granularity 2^(64 - B_ks * l_ks)"""
+    return min(coarse_shift(p), 64 - p.ks_base_log * p.ks_level) - 1
+
+
+def coarse_ksk(p, seed):
+    """test KSK [k*N, l_ks, n+1]: uniform random mask words and a body column of random multiples of 2^u (not an encryption, like the
+    lattice BSK: the body column on the lattice keeps every small body on 2^u + eps)"""
+    u = coarse_shift(p)
+    rng = np.random.default_rng(seed)
+    ksk = rng.integers(0, 2**64, size=(p.big_dim, p.ks_level, p.lwe_dim + 1), dtype=np.uint64)
+    ksk[:, :, p.lwe_dim] = rng.integers(0, 2**(64 - u), size=(p.big_dim, p.ks_level), dtype=np.uint64) << np.uint64(u)
+    return ksk.ravel()
+
+
+def coarse_inputs(p, rows, seed):
+    """big LWEs [rows, k*N+1] of random multiples of 2^u; about a quarter of the words replaced by 0, 2^63, 2^64 - 2^u or a multiple of
+    delta (a noise-free plaintext), and row 0 (if any) all zero"""
+    u = coarse_shift(p)
+    delta_log = 63 - (int(p.msg_mod * p.carry_mod).bit_length() - 1)
+    rng = np.random.default_rng(seed)
+    x = rng.integers(0, 2**(64 - u), size=(rows, p.big_dim + 1), dtype=np.uint64) << np.uint64(u)
+    fixed = np.array([0, 2**63, 2**64 - 2**u], dtype=np.uint64)
+    plain = rng.integers(0, 2**(64 - delta_log), size=x.shape, dtype=np.uint64) << np.uint64(delta_log)
+    edge = np.where(rng.random(x.shape) < 0.5, fixed[rng.integers(0, 3, size=x.shape)], plain)
+    pick = rng.random(x.shape) < 0.25
+    x[pick] = edge[pick]
+    if rows:
+        x[0] = 0
+    return x
+
+
+def keyswitch_rows(orc, p, ksk, big):
+    """orc_keyswitch of every row (the C calls release the GIL: one row per thread)"""
+    from concurrent.futures import ThreadPoolExecutor
+    big = np.ascontiguousarray(big, dtype=np.uint64)
+    out = np.zeros((big.shape[0], p.lwe_dim + 1), dtype=np.uint64)
+    L = orc.lib()
+
+    def one(i):
+        L.orc_keyswitch(C.byref(p), ksk, big[i], out[i])
+    with ThreadPoolExecutor(max(1, min(16, int(L.orc_max_threads())))) as pool:
+        list(pool.map(one, range(big.shape[0])))
+    return out
+
+
+class ProgramTrace:
+    """what run_program_exact saw at each level with PBS: level index, the arena rows entering the keyswitch, the LUT indices, the small
+    LWEs and the PBS outputs"""
+
+    def __init__(self):
+        self.levels, self.big_in, self.lut_idx, self.small, self.pbs_out = [], [], [], [], []
+
+
+def run_program_exact(orc, ir, accs, p, ksk, inputs, pbs, trace=None):
+    """Replay a recorded program (Program.ir(), Program.accumulators()) level by level the way enqueue_levels runs it: the linear
+    instructions with wrapping u64 arithmetic and int64 coefficients, then the level's keyswitch (orc_keyswitch, exact integers) and
+    pbs(small, accs, lut_idx) -- orc.pbs_exact_batch with an explicit BSK, or orc.pbs_f64_batch with a FourierKey -- written to the output
+    slots.  Returns the output rows; a ProgramTrace given as `trace` is filled level by level."""
+    L = p.big_dim + 1
+    ksk = np.ascontiguousarray(ksk, dtype=np.uint64)
+    inputs = np.ascontiguousarray(inputs, dtype=np.uint64).reshape(-1, L)
+    assert inputs.shape[0] == ir.n_inputs
+    arena = np.zeros((ir.n_slots, L), dtype=np.uint64)
+    arena[: ir.n_inputs] = inputs
+    with np.errstate(over="ignore"):
+        for lv in range(len(ir.level_lin_off) - 1):
+            for li in range(int(ir.level_lin_off[lv]), int(ir.level_lin_off[lv + 1])):
+                out, tb, te = (int(v) for v in ir.lin[li])
+                acc = np.zeros(L, dtype=np.uint64)
+                for t in range(tb, te):
+                    acc += arena[ir.term_slot[t]] * np.uint64(int(ir.term_coef[t]) % 2**64)
+                acc[-1] += ir.lin_body[li]
+                arena[out] = acc
+            p0, p1 = int(ir.level_pbs_off[lv]), int(ir.level_pbs_off[lv + 1])
+            if p1 == p0:
+                continue
+            jobs = ir.pbs[p0:p1]
+            big = arena[jobs[:, 0]]
+            idx = np.ascontiguousarray(jobs[:, 2], dtype=np.uint32)
+            small = keyswitch_rows(orc, p, ksk, big)
+            res = pbs(small, accs, idx)
+            arena[jobs[:, 1]] = res
+            if trace is not None:
+                trace.levels.append(lv)
+                trace.big_in.append(big)
+                trace.lut_idx.append(idx)
+                trace.small.append(small)
+                trace.pbs_out.append(res)
+    return arena[ir.outputs]
+
+
+def max_coef_sum(ir):
+    """the largest sum |coef| of one linear instruction (1 if there is none: a PBS output read directly)"""
+    best = 1
+    for out, tb, te in ir.lin:
+        best = max(best, int(np.abs(ir.term_coef[int(tb):int(te)]).sum()))
+    return best
+
+
+def modulus_switched(p, small):
+    """the values the blind rotation reads from small LWEs: every word switched to 2N (orc_modulus_switch, round half up)"""
+    lg = int(p.poly_size).bit_length() - 1
+    x = np.ascontiguousarray(small, dtype=np.uint64)
+    return (((x >> np.uint64(62 - lg)) + np.uint64(1)) >> np.uint64(1)) & np.uint64(2 * p.poly_size - 1)
