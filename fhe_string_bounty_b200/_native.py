@@ -1,7 +1,8 @@
 """ctypes loader for libtfhe_b200.so and a small numpy-facing wrapper around the C ABI.
 
 Nothing here computes: every method forwards to an ``extern "C"`` entry point declared in
-``include/tfhe_b200.h``.  Missing library or missing GPU raises NativeError (no fallback).
+``include/tfhe_b200.h`` (EXPORTS) or ``include/tfhe_b200_sharded.h`` (SHARDED_EXPORTS).  Missing library or missing GPU
+raises NativeError (no fallback).
 """
 from __future__ import annotations
 
@@ -15,7 +16,7 @@ import numpy as np
 _PKG = Path(__file__).resolve().parent
 _SO = _PKG / "libtfhe_b200.so"
 _SOURCES = ["csrc/pbs_v4.cu", "csrc/pbs_v8.cu", "csrc/pbs_multibit_v4.cu", "csrc/pbs_multibit_v8.cu", "csrc/pbs_generic.cu", "csrc/pbs_n512.cu", "csrc/pbs_n8192.cu", "csrc/keyswitch.cu", "csrc/keyswitch_mma.cu", "csrc/keyswitch_tc.cu", "csrc/leveled.cu", "csrc/seeded.cu", "csrc/probe.cu", "csrc/exchange.cu", "csrc/c_api.cu", "csrc/host_api.cu"]
-_HEADERS = ["csrc/fft_core.cuh", "csrc/fft16_core.cuh", "csrc/fft8_core.cuh", "csrc/fft16x_slots.cuh", "csrc/pbs16_common.cuh", "csrc/pbs8_common.cuh", "csrc/ring_helpers.cuh", "csrc/kernels.h", "csrc/ctx.h", "csrc/host/program.h", "csrc/host/radix.h", "csrc/host/strings.h", "csrc/host/padded.h", "../include/tfhe_b200.h"]
+_HEADERS = ["csrc/fft_core.cuh", "csrc/fft16_core.cuh", "csrc/fft8_core.cuh", "csrc/fft16x_slots.cuh", "csrc/pbs16_common.cuh", "csrc/pbs8_common.cuh", "csrc/ring_helpers.cuh", "csrc/kernels.h", "csrc/ctx.h", "csrc/host/program.h", "csrc/host/radix.h", "csrc/host/strings.h", "csrc/host/padded.h", "../include/tfhe_b200.h", "../include/tfhe_b200_sharded.h"]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
@@ -224,6 +225,15 @@ EXPORTS = {
     "tfhe_b200_exchange_destroy": (C.c_int, [C.c_void_p]),
 }
 
+# include/tfhe_b200_sharded.h: any recorded program across the ranks of an exchange
+SHARDED_EXPORTS = {
+    "tfhe_b200_program_shard_plan": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, C.c_void_p]),
+    "tfhe_b200_program_level_share": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p]),
+    "tfhe_b200_program_run_sharded": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "tfhe_b200_program_run_sharded_group": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint32,
+                                                      C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint64, C.c_void_p]),
+}
+
 _lib = None
 
 
@@ -235,7 +245,7 @@ def load_native():
     if not _SO.exists():
         raise NativeError(f"{_SO} is missing: run __graft_entry__.build() (nvcc, sm_100a). There is no CPU fallback.")
     lib = C.CDLL(str(_SO))
-    for name, (res, args) in EXPORTS.items():
+    for name, (res, args) in {**EXPORTS, **SHARDED_EXPORTS}.items():
         try:
             fn = getattr(lib, name)
         except AttributeError as e:

@@ -104,4 +104,42 @@ int do_keyswitch(tfhe_b200_ctx *c, const uint64_t *d_in, uint64_t *d_small, size
                  const uint32_t *in_slot = nullptr, DevBuf *digits = nullptr, bool fused = false);
 int do_pbs(tfhe_b200_ctx *c, const uint64_t *d_small, const uint32_t *d_idx, const uint64_t *d_luts, uint64_t *d_out, size_t batch,
            uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot = nullptr, bool fused = false);
+
+// rank r's PBS jobs [lo, hi) of a split level of w jobs: contiguous and balanced, the first w % world ranks take one more
+// (multi_gpu.shard_range; the scatter kernel inverts it on the device)
+__host__ __device__ inline void shard_range(size_t w, uint32_t r, uint32_t world, size_t &lo, size_t &hi) {
+    const size_t base = w / world, rem = w % world;
+    lo = r * base + (r < rem ? r : rem);
+    hi = lo + base + (r < rem ? 1 : 0);
+}
+}  // namespace tbc
+
+// the symmetric exchange buffer of one rank (csrc/exchange.cu); here so that the program executor (host_api.cu) can validate it
+struct tfhe_b200_exchange {
+    tfhe_b200_ctx *ctx = nullptr;
+    int device = 0;
+    uint32_t rank = 0, world = 1, max_rows = 0;
+    size_t lwe_len = 0, flags_bytes = 0, area_bytes = 0;
+    tbc::DevBuf local;                         // the symmetric buffer of this rank
+    std::vector<void *> peer;                  // peer[r] = rank r's buffer as mapped into this process (peer[rank] = local.p)
+    std::vector<bool> opened;                  // mapped through cudaIpcOpenMemHandle (must be closed)
+    tbc::DevBuf d_peers;                       // device copy of `peer`
+    tbc::DevBuf d_group;                       // per-rank arguments of a single-GPU group launch
+    uint64_t epoch = 0;
+    bool attached = false;
+    bool shares_device = false;                // some peer lives on this very GPU: only tfhe_b200_exchange_group_run may run the exchange
+};
+
+namespace tbc {
+// send area of the NEXT exchange of `ex`
+inline uint64_t *exchange_next_send_area(const tfhe_b200_exchange *ex) {
+    return reinterpret_cast<uint64_t *>(static_cast<char *>(ex->local.p) + ex->flags_bytes + (size_t)((ex->epoch + 1) & 1) * ex->area_bytes);
+}
+// The scatter exchange after a split level of w PBS jobs (csrc/exchange.cu): every rank's share (shard_range) is pulled from that rank's
+// send area and row i of rank r's share lands in arena row out_slot[lo_r + i].  No validation and no locking: the caller holds the
+// context's mutex and has checked the exchange.  exchange_scatter: one rank of a one-process-per-GPU world; exchange_scatter_group: all
+// `world` ranks of one GPU in one cooperative launch (arenas[r] / out_slots[r] are rank r's).
+int exchange_scatter(tfhe_b200_exchange *ex, uint32_t w, const uint32_t *out_slot, uint64_t *arena, cudaStream_t s);
+int exchange_scatter_group(tfhe_b200_exchange *const *group, uint32_t world, uint32_t w, const uint32_t *const *out_slots,
+                           uint64_t *const *arenas, cudaStream_t s);
 }  // namespace tbc

@@ -18,6 +18,8 @@
 // flag to finish an exchange, and the peer raises flag e+1 only after its own exchange-e kernel has completed in stream order), so
 // epoch e+2 never overwrites rows that a peer is still reading for epoch e.
 // A peer that never arrives turns into a launch failure after ~20 s (__trap), never into a hung GPU.
+// The scatter kernels below use the same publish / wait steps after every split level of a sharded program (tfhe_b200_program_run_sharded):
+// every rank pulls every rank's PBS share and writes each row to its own arena slot.
 #include "ctx.h"
 
 #include <memory>
@@ -25,21 +27,6 @@
 using tbc::DevBuf;
 using tbc::DeviceGuard;
 using tbc::fail;
-
-struct tfhe_b200_exchange {
-    tfhe_b200_ctx *ctx = nullptr;
-    int device = 0;
-    uint32_t rank = 0, world = 1, max_rows = 0;
-    size_t lwe_len = 0, flags_bytes = 0, area_bytes = 0;
-    DevBuf local;                              // the symmetric buffer of this rank
-    std::vector<void *> peer;                  // peer[r] = rank r's buffer as mapped into this process (peer[rank] = local.p)
-    std::vector<bool> opened;                  // mapped through cudaIpcOpenMemHandle (must be closed)
-    DevBuf d_peers;                            // device copy of `peer`
-    DevBuf d_group;                            // per-rank arguments of a single-GPU group launch
-    uint64_t epoch = 0;
-    bool attached = false;
-    bool shares_device = false;                // some peer lives on this very GPU: only tfhe_b200_exchange_group_run may run the exchange
-};
 
 namespace {
 
@@ -58,9 +45,14 @@ __device__ __forceinline__ ulonglong2 ld_relaxed_sys_v2(const ulonglong2 *p) {
     return v;
 }
 
-// words16 = number of 16-byte units per rank (rows * lwe_len words rounded up to even, / 2); out is 16-byte aligned
-__device__ __forceinline__ void exchange_body(void *const *__restrict__ peers, uint32_t rank, uint32_t world, uint64_t epoch, size_t flags_bytes,
-                                              size_t area_bytes, size_t words16, int reduce, ulonglong2 *__restrict__ out) {
+__device__ __forceinline__ uint64_t ld_relaxed_sys(const uint64_t *p) {
+    uint64_t v;
+    asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+
+// steps 1 and 2 of every exchange kernel; on return every peer's rows of `epoch` are readable by this CTA
+__device__ __forceinline__ void publish_and_wait(void *const *__restrict__ peers, uint32_t rank, uint32_t world, uint64_t epoch) {
     // 1. publish (one CTA): everything the previous kernels of this stream wrote to my send area is visible system-wide first
     if (blockIdx.x == 0 && threadIdx.x < world) {
         __threadfence_system();
@@ -74,6 +66,12 @@ __device__ __forceinline__ void exchange_body(void *const *__restrict__ peers, u
             if (clock64() - t0 > kSpinLimitCycles) __trap();
     }
     __syncthreads();
+}
+
+// words16 = number of 16-byte units per rank (rows * lwe_len words rounded up to even, / 2); out is 16-byte aligned
+__device__ __forceinline__ void exchange_body(void *const *__restrict__ peers, uint32_t rank, uint32_t world, uint64_t epoch, size_t flags_bytes,
+                                              size_t area_bytes, size_t words16, int reduce, ulonglong2 *__restrict__ out) {
+    publish_and_wait(peers, rank, world, epoch);
     // 3. pull
     const size_t off = flags_bytes + (size_t)(epoch & 1) * area_bytes;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
@@ -108,6 +106,62 @@ exchange_group_kernel(const GroupRank *__restrict__ ranks, uint32_t world, size_
     exchange_body(g.peers, blockIdx.y, world, g.epoch, flags_bytes, area_bytes, words16, reduce, g.out);
 }
 
+// ---- scatter: the exchange after a split level of a sharded program (tfhe_b200_program_run_sharded*) ----------------------------------
+// Rank r's PBS share of a level of w jobs, rows [lo_r, hi_r) of tbc::shard_range, sits contiguously in r's send area; every rank pulls
+// every share (its own included) and writes job g's row to ITS arena row out_slot[g].  Rows are k*N+1 words, an odd count at every
+// parameter set, so a row and the arena slot it goes to need not share their 16-byte alignment: 8-byte loads and stores, kUnroll of them
+// in flight per thread (peer loads take a NVLink round trip).
+// The double buffer still holds with one exchange after every split level: whatever runs between two exchanges (the next levels' linear,
+// keyswitch and PBS kernels, or nothing for a rank with an empty share), a rank finishes exchange e + 1 only once every peer has raised
+// flag e + 1, which a peer does only after its exchange-e kernel -- the last reader of the epoch-e rows -- has completed in stream order.
+// So the PBS of the level after exchange e + 1 may overwrite the parity-e send area.  The epochs stay in step because every rank runs
+// an exchange after every split level, with or without a share: the plan depends only on (program, world, min_shard_width).
+constexpr int kUnroll = 8;
+
+__device__ __forceinline__ void scatter_body(void *const *__restrict__ peers, uint32_t rank, uint32_t world, uint64_t epoch, size_t flags_bytes,
+                                             size_t area_bytes, size_t lwe_len, uint32_t w, const uint32_t *__restrict__ out_slot,
+                                             uint64_t *__restrict__ arena) {
+    publish_and_wait(peers, rank, world, epoch);
+    const size_t off = flags_bytes + (size_t)(epoch & 1) * area_bytes;
+    const uint32_t base = w / world, rem = w % world, big = rem * (base + 1);   // jobs [0, big) belong to the ranks with base + 1 jobs
+    for (uint32_t g = blockIdx.x; g < w; g += gridDim.x) {
+        const uint32_t r = g < big ? g / (base + 1) : rem + (g - big) / base;
+        size_t lo, hi;
+        tbc::shard_range(w, r, world, lo, hi);
+        const uint64_t *src = reinterpret_cast<const uint64_t *>(static_cast<const char *>(peers[r]) + off) + (g - lo) * lwe_len;
+        uint64_t *dst = arena + (size_t)out_slot[g] * lwe_len;
+        for (size_t j0 = threadIdx.x; j0 < lwe_len; j0 += (size_t)kUnroll * blockDim.x) {
+            uint64_t v[kUnroll];
+#pragma unroll
+            for (int u = 0; u < kUnroll; ++u) {
+                const size_t j = j0 + (size_t)u * blockDim.x;
+                if (j < lwe_len) v[u] = ld_relaxed_sys(src + j);
+            }
+#pragma unroll
+            for (int u = 0; u < kUnroll; ++u) {
+                const size_t j = j0 + (size_t)u * blockDim.x;
+                if (j < lwe_len) dst[j] = v[u];
+            }
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256)
+scatter_kernel(void *const *__restrict__ peers, uint32_t rank, uint32_t world, uint64_t epoch, size_t flags_bytes, size_t area_bytes,
+               size_t lwe_len, uint32_t w, const uint32_t *__restrict__ out_slot, uint64_t *__restrict__ arena) {
+    scatter_body(peers, rank, world, epoch, flags_bytes, area_bytes, lwe_len, w, out_slot, arena);
+}
+
+// several ranks on one GPU: one cooperative launch, blockIdx.y = rank, as exchange_group_kernel.  The per-rank arguments travel by value
+// (64 x 32 bytes fit the kernel parameter space), so a launch needs no upload and no synchronisation.
+struct ScatterRank { void *const *peers; const uint32_t *out_slot; uint64_t *arena; uint64_t epoch; };
+struct ScatterGroup { ScatterRank r[kMaxWorld]; };
+__global__ void __launch_bounds__(256)
+scatter_group_kernel(const ScatterGroup g, uint32_t world, size_t flags_bytes, size_t area_bytes, size_t lwe_len, uint32_t w) {
+    const ScatterRank &m = g.r[blockIdx.y];
+    scatter_body(m.peers, blockIdx.y, world, m.epoch, flags_bytes, area_bytes, lwe_len, w, m.out_slot, m.arena);
+}
+
 size_t round_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 int run_exchange(tfhe_b200_exchange *ex, uint32_t rows, uint64_t *d_out, void *stream, int reduce) {
@@ -130,6 +184,35 @@ int run_exchange(tfhe_b200_exchange *ex, uint32_t rows, uint64_t *d_out, void *s
 }
 
 }  // namespace
+
+namespace tbc {
+
+int exchange_scatter(tfhe_b200_exchange *ex, uint32_t w, const uint32_t *out_slot, uint64_t *arena, cudaStream_t s) {
+    ex->epoch += 1;
+    const int blocks = (int)std::max<uint32_t>(1, std::min<uint32_t>((uint32_t)ex->ctx->sms, w));
+    scatter_kernel<<<blocks, 256, 0, s>>>((void *const *)ex->d_peers.p, ex->rank, ex->world, ex->epoch, ex->flags_bytes, ex->area_bytes,
+                                          ex->lwe_len, w, out_slot, arena);
+    TB_CUDA(cudaGetLastError());
+    ex->ctx->launches += 1;
+    return 0;
+}
+
+int exchange_scatter_group(tfhe_b200_exchange *const *group, uint32_t world, uint32_t w, const uint32_t *const *out_slots,
+                           uint64_t *const *arenas, cudaStream_t s) {
+    tfhe_b200_exchange *lead = group[0];
+    ScatterGroup g{};
+    for (uint32_t r = 0; r < world; ++r) {
+        group[r]->epoch += 1;
+        g.r[r] = ScatterRank{(void *const *)group[r]->d_peers.p, out_slots[r], arenas[r], group[r]->epoch};
+    }
+    const unsigned bx = std::max<unsigned>(1, std::min<unsigned>((unsigned)lead->ctx->sms / world, w));
+    void *args[] = {(void *)&g, (void *)&world, (void *)&lead->flags_bytes, (void *)&lead->area_bytes, (void *)&lead->lwe_len, (void *)&w};
+    TB_CUDA(cudaLaunchCooperativeKernel((const void *)scatter_group_kernel, dim3(bx, world), dim3(256), args, 0, s));
+    lead->ctx->launches += 1;
+    return 0;
+}
+
+}  // namespace tbc
 
 extern "C" {
 
@@ -223,7 +306,7 @@ int tfhe_b200_exchange_attach_local(tfhe_b200_exchange *ex, tfhe_b200_exchange *
  * stream the exchange is then called with (e.g. tfhe_b200_program_run_device(..., d_outputs = this pointer, stream)). */
 int tfhe_b200_exchange_send_rows(tfhe_b200_exchange *ex, uint64_t **d_rows) {
     if (!ex || !d_rows) return fail("null argument");
-    *d_rows = reinterpret_cast<uint64_t *>(static_cast<char *>(ex->local.p) + ex->flags_bytes + (size_t)((ex->epoch + 1) & 1) * ex->area_bytes);
+    *d_rows = tbc::exchange_next_send_area(ex);
     return 0;
 }
 

@@ -5,6 +5,7 @@
 // (integer/server_key/radix_parallel/*.rs -> shortint apply_lookup_table) that north_star asks for.
 #include "ctx.h"
 #include "host/padded.h"
+#include "../../include/tfhe_b200_sharded.h"
 
 #include <cstring>
 #include <memory>
@@ -388,35 +389,108 @@ int bind_program(tfhe_b200_ctx *c, tfhe_b200_program *h) {
     return 0;
 }
 
-// enqueues every level of the program on stream `s`: inputs are already in arena rows [0, n_inputs); the output rows end up in `d_out`
-int enqueue_levels(tfhe_b200_ctx *c, tfhe_b200_program *h, uint64_t *d_out, cudaStream_t s) {
-    const tbh::Program &pg = *h->prog;
-    const size_t L = c->big_len();
-    uint64_t *arena = (uint64_t *)h->d_arena.p;
-    TB_CUDA(cudaEventRecord(h->ev0, s));
+// The shard plan of a level: a level of w PBS jobs is split across `world` ranks when w > min_shard_width (and world > 1); rank `rank`
+// then runs jobs [lo, hi) of it (tbc::shard_range, possibly empty).  Every other level is replicated: every rank runs [0, w).  It depends
+// only on (program, world, min_shard_width), so all ranks agree on it without talking.
+bool level_share(const tfhe_b200_program *h, size_t lv, uint32_t rank, uint32_t world, uint64_t min_shard_width, size_t &lo, size_t &hi) {
+    const size_t w = h->pbs_off[lv + 1] - h->pbs_off[lv];
+    const bool split = world > 1 && w > min_shard_width;
+    lo = 0; hi = w;
+    if (split) tbc::shard_range(w, rank, world, lo, hi);
+    return split;
+}
+
+// {split levels, largest share in rows (the exchange's max_rows), rows each rank receives over all split levels}
+void shard_plan(const tfhe_b200_program *h, uint32_t world, uint64_t min_shard_width, uint64_t out[3]) {
+    out[0] = out[1] = out[2] = 0;
+    for (size_t lv = 0; lv + 1 < h->pbs_off.size(); ++lv) {
+        size_t lo, hi;
+        if (!level_share(h, lv, 0, world, min_shard_width, lo, hi)) continue;   // rank 0 has the largest share
+        out[0] += 1;
+        out[1] = std::max<uint64_t>(out[1], hi - lo);
+        out[2] += h->pbs_off[lv + 1] - h->pbs_off[lv];
+    }
+}
+
+// one rank of a run: its context, its program (bound to that context), its exchange (nullptr: an unsharded run) and its output rows
+struct Member { tfhe_b200_ctx *c; tfhe_b200_program *h; tfhe_b200_exchange *ex; uint64_t *d_out; };
+
+// Enqueues every level of the program on stream `s` for each of the `n` members: inputs are already in arena rows [0, n_inputs); the output
+// rows end up in each member's d_out.  n == 1 without exchange: the plain run.  n == 1 with an exchange: rank ex->rank of a world of one
+// process per GPU.  n == world > 1: every rank of one GPU, each level's shares enqueued rank after rank, then one cooperative scatter.
+// A split level runs the linear instructions in full, the keyswitch and PBS of the member's share only (the PBS writes its rows
+// contiguously into the exchange's send area), then the scatter that puts every share's rows into every member's arena.
+int enqueue_levels(const Member *m, uint32_t n, uint64_t min_shard_width, cudaStream_t s) {
+    const tbh::Program &pg = *m[0].h->prog;
+    const uint32_t world = m[0].ex ? m[0].ex->world : 1;
     size_t max_w = 0;
     for (auto &l : pg.levels()) max_w = std::max(max_w, l.pbs.size());
-    TB_CUDA(c->d_small.reserve_on(std::max<size_t>(max_w, 1) * c->small_len() * 8, s));
+    for (uint32_t i = 0; i < n; ++i) {
+        TB_CUDA(cudaEventRecord(m[i].h->ev0, s));
+        TB_CUDA(m[i].c->d_small.reserve_on(std::max<size_t>(max_w, 1) * m[i].c->small_len() * 8, s));
+    }
+    std::vector<tfhe_b200_exchange *> exs(n);
+    std::vector<const uint32_t *> out_slots(n);
+    std::vector<uint64_t *> arenas(n);
     for (size_t lv = 0; lv < pg.levels().size(); ++lv) {
-        const uint32_t l0 = h->lin_off[lv], l1 = h->lin_off[lv + 1], p0 = h->pbs_off[lv], p1 = h->pbs_off[lv + 1];
-        if (l1 > l0) {
-            TB_CUDA(tbk::launch_linear(arena, (const tbk::LinInstr *)h->d_lin.p + l0, (const tbk::LinTerm *)h->d_terms.p, int(l1 - l0), int(L), s));
-            c->launches += 1;
+        const uint32_t l0 = m[0].h->lin_off[lv], l1 = m[0].h->lin_off[lv + 1], p0 = m[0].h->pbs_off[lv], p1 = m[0].h->pbs_off[lv + 1];
+        bool split = false;
+        for (uint32_t i = 0; i < n; ++i) {
+            tfhe_b200_ctx *c = m[i].c;
+            tfhe_b200_program *h = m[i].h;
+            const size_t L = c->big_len();
+            uint64_t *arena = (uint64_t *)h->d_arena.p;
+            if (l1 > l0) {
+                TB_CUDA(tbk::launch_linear(arena, (const tbk::LinInstr *)h->d_lin.p + l0, (const tbk::LinTerm *)h->d_terms.p, int(l1 - l0), int(L), s));
+                c->launches += 1;
+            }
+            size_t lo, hi;
+            split = level_share(h, lv, m[i].ex ? m[i].ex->rank : 0, world, min_shard_width, lo, hi);
+            if (hi > lo) {
+                const size_t w = hi - lo;
+                const bool fused = tbc::fused_supported(c);
+                if (tbc::do_keyswitch(c, arena, (uint64_t *)c->d_small.p, w, s, (const uint32_t *)h->d_pbs_in.p + p0 + lo, nullptr, fused)) return 1;
+                if (tbc::do_pbs(c, (const uint64_t *)c->d_small.p, (const uint32_t *)h->d_pbs_lut.p + p0 + lo, (const uint64_t *)h->d_luts.p,
+                                split ? tbc::exchange_next_send_area(m[i].ex) : arena, w, c->p.lwe_dim, s,
+                                split ? nullptr : (const uint32_t *)h->d_pbs_out.p + p0, fused))
+                    return 1;
+            }
+            exs[i] = m[i].ex;
+            out_slots[i] = (const uint32_t *)h->d_pbs_out.p + p0;
+            arenas[i] = arena;
         }
-        if (p1 > p0) {
-            const size_t w = p1 - p0;
-            const bool fused = tbc::fused_supported(c);
-            if (tbc::do_keyswitch(c, arena, (uint64_t *)c->d_small.p, w, s, (const uint32_t *)h->d_pbs_in.p + p0, nullptr, fused)) return 1;
-            if (tbc::do_pbs(c, (const uint64_t *)c->d_small.p, (const uint32_t *)h->d_pbs_lut.p + p0, (const uint64_t *)h->d_luts.p, arena, w,
-                            c->p.lwe_dim, s, (const uint32_t *)h->d_pbs_out.p + p0, fused))
+        if (split) {
+            if (n > 1 ? tbc::exchange_scatter_group(exs.data(), n, p1 - p0, out_slots.data(), arenas.data(), s)
+                      : tbc::exchange_scatter(exs[0], p1 - p0, out_slots[0], arenas[0], s))
                 return 1;
         }
     }
-    TB_CUDA(cudaEventRecord(h->ev1, s));
-    if (!pg.outputs().empty()) {   // gather the output rows on the device
-        TB_CUDA(tbk::launch_gather_rows(arena, (const uint32_t *)h->d_out_slots.p, d_out, (int)pg.outputs().size(), (int)L, s));
-        c->launches += 1;
+    for (uint32_t i = 0; i < n; ++i) {
+        TB_CUDA(cudaEventRecord(m[i].h->ev1, s));
+        if (!pg.outputs().empty()) {   // gather the output rows on the device
+            TB_CUDA(tbk::launch_gather_rows((uint64_t *)m[i].h->d_arena.p, (const uint32_t *)m[i].h->d_out_slots.p, m[i].d_out,
+                                            (int)pg.outputs().size(), (int)m[i].c->big_len(), s));
+            m[i].c->launches += 1;
+        }
     }
+    return 0;
+}
+
+// everything a sharded run checks about one rank before it enqueues anything
+int check_sharded_member(const char *who, tfhe_b200_ctx *c, tfhe_b200_program *h, tfhe_b200_exchange *ex, const uint64_t *d_inputs,
+                         uint64_t *d_outputs, uint64_t min_shard_width) {
+    const std::string w = who;
+    if (!c || !h || !ex) return fail(w + ": null argument");
+    const tbh::Program &pg = *h->prog;
+    if ((pg.n_inputs() && !d_inputs) || (!pg.outputs().empty() && !d_outputs)) return fail(w + ": null buffer");
+    if (!same_params(c->p, h->p)) return fail(w + ": program was recorded for other parameters than the context");
+    if (ex->ctx != c) return fail(w + ": the exchange of rank " + std::to_string(ex->rank) + " belongs to another context");
+    if (!ex->attached) return fail(w + ": exchange peers not attached yet (tfhe_b200_exchange_attach)");
+    uint64_t plan[3];
+    shard_plan(h, ex->world, min_shard_width, plan);
+    if (plan[1] > ex->max_rows)
+        return fail(w + ": " + h->op + " at world " + std::to_string(ex->world) + " and min_shard_width " + std::to_string(min_shard_width) +
+                    " needs an exchange of max_rows >= " + std::to_string(plan[1]) + ", this one holds " + std::to_string(ex->max_rows));
     return 0;
 }
 
@@ -525,7 +599,8 @@ int tfhe_b200_program_run(tfhe_b200_ctx *c, tfhe_b200_program *h, const uint64_t
     const size_t L = c->big_len();
     if (bind_program(c, h)) return 1;
     if (pg.n_inputs()) TB_CUDA(cudaMemcpyAsync(h->d_arena.p, inputs, (size_t)pg.n_inputs() * L * 8, cudaMemcpyHostToDevice, s));
-    if (enqueue_levels(c, h, (uint64_t *)h->d_out_rows.p, s)) return 1;
+    const Member m{c, h, nullptr, (uint64_t *)h->d_out_rows.p};
+    if (enqueue_levels(&m, 1, 0, s)) return 1;
     if (!pg.outputs().empty())     // one copy back
         TB_CUDA(cudaMemcpyAsync(outputs, h->d_out_rows.p, pg.outputs().size() * L * 8, cudaMemcpyDeviceToHost, s));
     TB_CUDA(cudaStreamSynchronize(s));
@@ -549,7 +624,92 @@ int tfhe_b200_program_run_device(tfhe_b200_ctx *c, tfhe_b200_program *h, const u
     if (bind_program(c, h)) return 1;
     if (pg.n_inputs()) TB_CUDA(cudaMemcpyAsync(h->d_arena.p, d_inputs, (size_t)pg.n_inputs() * L * 8, cudaMemcpyDeviceToDevice, s));
     h->last_ms = -1.f;    // not synchronised: tfhe_b200_program_last_ms reads the events on demand
-    return enqueue_levels(c, h, d_outputs, s);
+    const Member m{c, h, nullptr, d_outputs};
+    return enqueue_levels(&m, 1, 0, s);
+}
+
+/* {split levels, largest share in rows, rows each rank receives} of a sharded run at (world, min_shard_width); pure host arithmetic. */
+int tfhe_b200_program_shard_plan(const tfhe_b200_program *h, uint32_t world, uint64_t min_shard_width, uint64_t out[3]) {
+    if (!h || !out) return fail("null argument");
+    if (world < 1) return fail("program_shard_plan: world must be >= 1");
+    shard_plan(h, world, min_shard_width, out);
+    return 0;
+}
+
+/* Rank `rank`'s PBS jobs of level `level` in a sharded run: out = {lo, hi, split}, jobs [lo, hi) counted from the level's first job.
+ * A replicated level (split = 0) gives [0, width) to every rank. */
+int tfhe_b200_program_level_share(const tfhe_b200_program *h, uint32_t level, uint32_t rank, uint32_t world, uint64_t min_shard_width,
+                                  uint64_t out[3]) {
+    if (!h || !out) return fail("null argument");
+    if (world < 1 || rank >= world) return fail("program_level_share: need world >= 1 and rank < world");
+    if ((size_t)level + 1 >= h->pbs_off.size()) return fail("program_level_share: no level " + std::to_string(level));
+    size_t lo, hi;
+    out[2] = level_share(h, level, rank, world, min_shard_width, lo, hi);
+    out[0] = lo; out[1] = hi;
+    return 0;
+}
+
+/* One rank of a program run across the ranks of `ex` (one process per GPU): levels wider than min_shard_width are split, every rank runs
+ * its share and the scatter exchange hands every row to every rank; the other levels run in full on every rank.  Every rank passes all
+ * inputs and receives all outputs; device buffers, enqueued on `cuda_stream` (NULL = the context's stream) without synchronising. */
+int tfhe_b200_program_run_sharded(tfhe_b200_ctx *c, tfhe_b200_program *h, tfhe_b200_exchange *ex, const uint64_t *d_inputs, uint64_t *d_outputs,
+                                  uint64_t min_shard_width, void *cuda_stream) {
+    if (check_sharded_member("program_run_sharded", c, h, ex, d_inputs, d_outputs, min_shard_width)) return 1;
+    if (ex->shares_device)
+        return fail("program_run_sharded: ranks that share a GPU must use tfhe_b200_program_run_sharded_group (kernels that wait on one another "
+                    "cannot be separate launches on one device)");
+    const tbh::Program &pg = *h->prog;
+    std::lock_guard<std::mutex> lk(c->mu);
+    DeviceGuard g(c->device);
+    cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
+    if (bind_program(c, h)) return 1;
+    if (pg.n_inputs()) TB_CUDA(cudaMemcpyAsync(h->d_arena.p, d_inputs, (size_t)pg.n_inputs() * c->big_len() * 8, cudaMemcpyDeviceToDevice, s));
+    h->last_ms = -1.f;
+    const Member m{c, h, ex, d_outputs};
+    return enqueue_levels(&m, 1, min_shard_width, s);
+}
+
+/* Every rank of one GPU in one call on one stream (ctxs[r], progs[r], exs[r]: rank r's context, its own program object -- a program binds
+ * to one context -- and its exchange, attached with tfhe_b200_exchange_attach_local).  Per split level every rank's share is enqueued,
+ * then one cooperative scatter serves all ranks. */
+int tfhe_b200_program_run_sharded_group(tfhe_b200_ctx *const *ctxs, tfhe_b200_program *const *progs, tfhe_b200_exchange *const *exs, uint32_t world,
+                                        const uint64_t *const *d_inputs, uint64_t *const *d_outputs, uint64_t min_shard_width, void *cuda_stream) {
+    const char *who = "program_run_sharded_group";
+    if (!ctxs || !progs || !exs || !d_inputs || !d_outputs || world < 1) return fail(std::string(who) + ": null argument");
+    for (uint32_t r = 0; r < world; ++r) {
+        if (check_sharded_member(who, ctxs[r], progs[r], exs[r], d_inputs[r], d_outputs[r], min_shard_width)) return 1;
+        if (exs[r]->world != world || exs[r]->rank != r)
+            return fail(std::string(who) + ": exchange " + std::to_string(r) + " is rank " + std::to_string(exs[r]->rank) + " of " +
+                        std::to_string(exs[r]->world) + ", not rank " + std::to_string(r) + " of " + std::to_string(world));
+        if (exs[0]->peer[r] != exs[r]->local.p)
+            return fail(std::string(who) + ": exchange " + std::to_string(r) + " is not attached to exchange 0 (tfhe_b200_exchange_attach_local)");
+        if (ctxs[r]->device != ctxs[0]->device)
+            return fail(std::string(who) + ": rank " + std::to_string(r) + " is on device " + std::to_string(ctxs[r]->device) + ", rank 0 on device " +
+                        std::to_string(ctxs[0]->device) + ": a group runs on one GPU (use tfhe_b200_program_run_sharded, one process per GPU)");
+        if (progs[r]->op != progs[0]->op || progs[r]->pbs_off != progs[0]->pbs_off || progs[r]->lin_off != progs[0]->lin_off ||
+            !same_params(ctxs[r]->p, progs[0]->p))
+            return fail(std::string(who) + ": rank " + std::to_string(r) + " runs another program or parameter set than rank 0");
+        for (uint32_t q = 0; q < r; ++q)
+            if (progs[q] == progs[r] || ctxs[q] == ctxs[r])
+                return fail(std::string(who) + ": ranks " + std::to_string(q) + " and " + std::to_string(r) +
+                            " share a context or a program object (each rank needs its own; a program binds to one context)");
+    }
+    const tbh::Program &pg = *progs[0]->prog;
+    std::vector<std::unique_lock<std::mutex>> locks;
+    for (uint32_t r = 0; r < world; ++r) locks.emplace_back(ctxs[r]->mu);
+    DeviceGuard g(ctxs[0]->device);
+    cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : ctxs[0]->stream;
+    std::vector<Member> m(world);
+    for (uint32_t r = 0; r < world; ++r) {
+        if (bind_program(ctxs[r], progs[r])) return 1;
+        m[r] = Member{ctxs[r], progs[r], exs[r], d_outputs[r]};
+    }
+    for (uint32_t r = 0; r < world; ++r) {
+        if (pg.n_inputs())
+            TB_CUDA(cudaMemcpyAsync(progs[r]->d_arena.p, d_inputs[r], (size_t)pg.n_inputs() * ctxs[r]->big_len() * 8, cudaMemcpyDeviceToDevice, s));
+        progs[r]->last_ms = -1.f;
+    }
+    return enqueue_levels(m.data(), world, min_shard_width, s);
 }
 
 /* Device time (ms, CUDA events on the context stream) of the kernels of the last tfhe_b200_program_run. */

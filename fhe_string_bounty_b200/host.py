@@ -95,6 +95,18 @@ class Program:
     def level_widths(self):
         return self.ir().level_widths
 
+    def shard_plan(self, world: int, min_shard_width: int) -> tuple[int, int, int]:
+        """(split levels, largest share in rows, rows each rank receives) of a run across `world` ranks (tfhe_b200_program_shard_plan)"""
+        out = np.zeros(3, dtype=np.uint64)
+        self._check(self.lib.tfhe_b200_program_shard_plan(self.h, world, min_shard_width, out.ctypes.data))
+        return tuple(int(x) for x in out)
+
+    def level_share(self, level: int, rank: int, world: int, min_shard_width: int) -> tuple[int, int, bool]:
+        """(lo, hi, split): the PBS jobs of level `level` that `rank` runs, counted from the level's first job"""
+        out = np.zeros(3, dtype=np.uint64)
+        self._check(self.lib.tfhe_b200_program_level_share(self.h, level, rank, world, min_shard_width, out.ctypes.data))
+        return int(out[0]), int(out[1]), bool(out[2])
+
     def accumulators(self) -> np.ndarray:
         acc = np.zeros((max(self.n_luts, 1), self.p.lut_len), dtype=np.uint64)
         if self.n_luts:

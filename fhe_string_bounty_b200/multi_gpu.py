@@ -105,6 +105,16 @@ class PeerExchange:
             handles = np.ascontiguousarray(out.cpu().numpy())
             eng._check(self.lib.tfhe_b200_exchange_attach(self.h, handles.ctypes.data))
 
+    @classmethod
+    def local(cls, eng: Engine, rank: int, world: int, max_rows: int) -> "PeerExchange":
+        """an exchange of a rank driven by this process; the caller attaches the group (tfhe_b200_exchange_attach_local)"""
+        ex = cls.__new__(cls)
+        ex.eng, ex.lib, ex.rank, ex.world, ex.max_rows = eng, eng.lib, rank, world, max_rows
+        h = C.c_void_p()
+        eng._check(eng.lib.tfhe_b200_exchange_create(eng.h, rank, world, max_rows, C.byref(h)))
+        ex.h = h
+        return ex
+
     def send_rows_ptr(self) -> int:
         p = C.c_void_p()
         self.eng._check(self.lib.tfhe_b200_exchange_send_rows(self.h, C.byref(p)))
@@ -169,6 +179,7 @@ class DeviceComm:
         self._host_out: dict = {}                    # page-locked result buffers, by shape
         self._group = None                           # set by local_group(): several ranks of one process on one GPU
         self.peer = PeerExchange(eng, self.rank, self.world, max_rows) if (exchange == "peer" and self.world > 1) else None
+        self._program_peer: PeerExchange | None = None   # the exchange of run_program_sharded, sized by the shard plan on first need
 
     @classmethod
     def local_group(cls, engines: list, max_rows: int = 16) -> list:
@@ -182,16 +193,12 @@ class DeviceComm:
         if world > 1:
             for c in comms:
                 c.exchange = "peer"
-                c.peer = PeerExchange.__new__(PeerExchange)
-                c.peer.eng, c.peer.lib, c.peer.rank, c.peer.world, c.peer.max_rows = c.eng, c.eng.lib, c.rank, world, max_rows
-                h = C.c_void_p()
-                c.eng._check(c.eng.lib.tfhe_b200_exchange_create(c.eng.h, c.rank, world, max_rows, C.byref(h)))
-                c.peer.h = h
+                c.peer = PeerExchange.local(c.eng, c.rank, world, max_rows)
             arr = (C.c_void_p * world)(*[c.peer.h for c in comms])
             for c in comms:
                 c.eng._check(c.eng.lib.tfhe_b200_exchange_attach_local(c.peer.h, arr))
             group = {"barrier": threading.Barrier(world), "handles": arr, "events": [None] * world, "outs": [None] * world, "done": None,
-                     "error": None}
+                     "error": None, "args": [None] * world}
             for c in comms:
                 c._group = group
         return comms
@@ -351,7 +358,62 @@ class DeviceComm:
         out = buf.numpy().view(np.uint64)
         return out if out.nbytes > (1 << 20) else out.copy()
 
+    def _program_exchange(self, max_rows: int) -> PeerExchange:
+        """the exchange of run_program_sharded, holding at least `max_rows` rows per rank.  Creating or replacing it is collective: every
+        rank runs the same program at the same min_shard_width, so every rank arrives here with the same max_rows."""
+        old = self._program_peer
+        if old is not None and old.max_rows >= max_rows:
+            return old
+        g = self._group
+        barrier = g["barrier"].wait if g is not None else dist.barrier
+        if old is not None:
+            # a peer may still be reading this rank's send area in its last scatter: free it once every rank's stream has drained
+            self.stream.synchronize()
+            barrier()
+            old.close()
+            self._program_peer = None
+        if g is None:
+            self._program_peer = PeerExchange(self.eng, self.rank, self.world, max_rows)
+            return self._program_peer
+        ex = PeerExchange.local(self.eng, self.rank, self.world, max_rows)
+        g["args"][self.rank] = ex.h
+        barrier()
+        arr = (C.c_void_p * self.world)(*g["args"])
+        self.eng._check(self.eng.lib.tfhe_b200_exchange_attach_local(ex.h, arr))
+        barrier()                      # nobody reuses g["args"] before every rank has attached
+        self._program_peer = ex
+        return ex
+
+    def _group_run_sharded(self, prog: Program, ex: PeerExchange, d_in, out: torch.Tensor):
+        """single-GPU group: as _group_exchange, rank 0 issues the one tfhe_b200_program_run_sharded_group call for every rank"""
+        g = self._group
+        stream = self.stream
+        ev = torch.cuda.Event()
+        ev.record(stream)
+        g["events"][self.rank] = ev
+        g["args"][self.rank] = (self.eng.h, prog.h, ex.h, d_in.data_ptr() if d_in is not None else None, out.data_ptr() if out.numel() else None)
+        g["barrier"].wait()
+        if self.rank == 0:
+            try:
+                for e in g["events"]:
+                    stream.wait_event(e)
+                ptrs = lambda i: (C.c_void_p * self.world)(*[a[i] for a in g["args"]])
+                self.eng._check(self.eng.lib.tfhe_b200_program_run_sharded_group(ptrs(0), ptrs(1), ptrs(2), self.world, ptrs(3), ptrs(4),
+                                                                                 self.min_shard_width, stream.cuda_stream))
+                done = torch.cuda.Event()
+                done.record(stream)
+                g["done"], g["error"] = done, None
+            except Exception as e:      # the other ranks' threads must not be left at the barrier
+                g["error"] = e
+        g["barrier"].wait()
+        if g["error"] is not None:
+            raise NativeError(f"sharded group run failed: {g['error']}")
+        stream.wait_event(g["done"])
+
     def close(self):
+        if self._program_peer is not None:
+            self._program_peer.close()
+            self._program_peer = None
         if self.peer is not None:
             self.peer.close()
             self.peer = None
@@ -540,3 +602,41 @@ def sharded_find(comm, params: dict, hay, pat, hay_len: int, pat_len: int, rank:
         mine = comm.zeros(1 + nb, hay.shape[1])
     parts = comm.all_gather(mine)[:active]
     return comm.to_host(comm.run(comm.program("find_combine", (active, nb), params), parts.reshape(active * (1 + nb), -1)))
+
+
+# ---- any recorded program, its wide levels split across the ranks ------------------------------------------------------------------
+
+@_on_comm_stream
+def run_program_sharded(comm: DeviceComm, prog: Program, inputs) -> torch.Tensor:
+    """Any recorded program across the ranks of `comm`; every rank calls it with the same program (under DeviceComm.local_group each rank
+    with its own Program object, e.g. comm.program(...): a program binds to one context) and the same inputs, and gets all outputs as a
+    CUDA tensor (n_outputs, k*N+1) of int64 words on the comm's stream.
+
+    Levels wider than comm.min_shard_width are split: each rank keyswitches and bootstraps its shard_range share of the level and one
+    scatter kernel hands every row to every rank over NVLink peer memory (tfhe_b200_program_run_sharded).  Narrower levels run in full on
+    every rank, with no communication.
+
+    The scatter uses an exchange of its own, created collectively on first need and sized by the shard plan; the `peer` exchange of the
+    sharded_* operations stays as it is.  Its send area is double-buffered, so it takes 2 x (largest share) x (k*N+1) x 8 bytes per rank:
+    string_eq_many {8, 8, 4096} at world 2 has a widest level of 131 072 PBS, so a share of 65 536 rows and about 2.1 GB per rank."""
+    if not isinstance(comm, DeviceComm):
+        raise TypeError("run_program_sharded runs on a DeviceComm")
+    if comm.world == 1:
+        return comm.run(prog, inputs)
+    if comm.exchange != "peer":
+        raise ValueError("run_program_sharded: exchange='nccl' is not supported; the per-level scatter runs over peer memory only "
+                         "(DeviceComm(exchange='peer'))")
+    _, max_rows, _ = prog.shard_plan(comm.world, comm.min_shard_width)
+    ex = comm._program_exchange(max(1, max_rows))
+    d_in = comm._to_device(inputs).reshape(-1, comm.L) if prog.n_inputs else None
+    if prog.n_inputs and d_in.shape[0] != prog.n_inputs:
+        raise ValueError(f"{prog.op}: expected {prog.n_inputs} input blocks, got {d_in.shape[0]}")
+    out = torch.empty((prog.n_outputs, comm.L), dtype=torch.int64, device=comm.dev)
+    if comm._group is not None:
+        comm._group_run_sharded(prog, ex, d_in, out)
+    else:
+        comm.eng._check(comm.eng.lib.tfhe_b200_program_run_sharded(comm.eng.h, prog.h, ex.h, d_in.data_ptr() if d_in is not None else None,
+                                                                   out.data_ptr() if out.numel() else None, comm.min_shard_width,
+                                                                   comm._stream()))
+    comm._keep = d_in          # the upload must outlive the enqueued copy
+    return out

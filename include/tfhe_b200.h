@@ -217,6 +217,9 @@ int tfhe_b200_exchange_group_run(tfhe_b200_exchange *const *group, uint32_t worl
                                  void *cuda_stream);
 int tfhe_b200_exchange_destroy(tfhe_b200_exchange *ex);
 
+/* Running any recorded program across the ranks of an exchange (wide levels split, rows scattered back after each) is declared in
+ * tfhe_b200_sharded.h, which includes this header. */
+
 /* Kernel selection (A/B comparisons and the parity tests that pin one kernel instance); the same keys are read from the environment at
  * context creation as TFHE_B200_<KEY>.  Keys: "narrow_kernel" (8 = pbs_v8.cu / pbs_multibit_v8.cu serve levels of at most narrow_max
  * ciphertexts and level tails, 0 = the 1- / 2-ciphertext instances of the wide kernels), "narrow_max" (0 = default: 2 x SM count
