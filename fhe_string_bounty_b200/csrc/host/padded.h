@@ -316,7 +316,10 @@ class PaddedStringServerKey {
     }
 
     // some suffix of the haystack equals the pattern as padded strings (the empty suffix included)
-    BooleanBlock ends_with(const FheString &hay, const FheString &pat) {
+    BooleanBlock ends_with(const FheString &hay, const FheString &pat) { return isk.is_at_least_one_comparisons_block_true(suffix_matches(hay, pat)); }
+    // per[w], w = 0 ..= capacity: hay[w..] equals the pattern as padded strings.  A non-empty pattern fires at w = len - len(pat) only, the
+    // empty one at every w >= len
+    std::vector<Ct> suffix_matches(const FheString &hay, const FheString &pat) {
         const size_t n = hay.len(), m = pat.len();
         std::vector<Ct> pz = zero_flags(pat), hz = zero_flags(hay), per;
         for (size_t w = 0; w <= n; ++w) {
@@ -332,8 +335,31 @@ class PaddedStringServerKey {
             }
             per.push_back(isk.are_all_comparisons_block_true(flags));
         }
-        return isk.is_at_least_one_comparisons_block_true(per);
+        return per;
     }
+
+    // ---- strip_prefix / strip_suffix with a PADDED pattern: (matched, string) ---------------------------------------------------------
+    // prefix: a left shift by len(pat), every bit of the amount gated by the flag
+    std::pair<BooleanBlock, FheString> strip_prefix(const FheString &s, const FheString &pat) {
+        BooleanBlock flag = starts_with(s, pat);
+        if (pat.len() == 0) return {flag, s};
+        size_t n_bits = 1;
+        while ((size_t(1) << n_bits) <= pat.len()) ++n_bits;
+        std::vector<Ct> bits = bits_of(len(pat), n_bits);
+        for (auto &b : bits) b = and_flags(b, flag);
+        return {flag, shift(s, bits, true)};
+    }
+    // suffix: the chars at and after the window where the pattern is the suffix are dropped (the first such window for the empty pattern)
+    std::pair<BooleanBlock, FheString> strip_suffix(const FheString &s, const FheString &pat) {
+        const size_t n = s.len();
+        std::vector<Ct> drop = prefix_or(suffix_matches(s, pat), true);
+        FheString out = s;
+        for (size_t i = 0; i < n; ++i) out.chars[i] = keep(s.chars[i], isk.boolean_bitnot(drop[i]));
+        return {drop[n], out};
+    }
+
+    // ---- eq_ignore_case of two padded strings: the fused ASCII case fold of both (the padding byte folds to itself), then eq -----------
+    BooleanBlock eq_ignore_case(const FheString &a, const FheString &b) { return eq(ssk.to_lowercase(a), ssk.to_lowercase(b)); }
 
     // ---- concat / repeat: the second operand moves right by the secret length of the first; the supports are disjoint, so the result is a
     // leveled sum of blocks -----------------------------------------------------------------------------------------------------------------------
@@ -362,6 +388,29 @@ class PaddedStringServerKey {
         FheString acc = s;
         for (size_t k = 1; k < count; ++k) acc = concat(acc, s);
         return acc;
+    }
+    // repeat by a secret count: s repeated min(count, max_count) times in capacity * max_count chars.  Copy k is s masked by
+    // [k < count], and the copies are concatenated: an empty copy moves nothing.  Every concat adds one unit of noise to the chars it
+    // keeps, so they are cleaned before len() would sum four blocks of more than 3 units, and at the end
+    FheString repeat(const FheString &s, const Radix &count, size_t max_count) {
+        FheString acc;
+        if (max_count == 0) return acc;
+        const Radix limit = clamp_radix(count, digits_for(max_count));
+        for (size_t k = 0; k < max_count; ++k) {
+            const Ct more = pg.pbs(scalar_sign(limit, k), [](uint64_t x) { return uint64_t(x == IntegerServerKey::IS_SUPERIOR); });
+            FheString copy;
+            for (auto &c : s.chars) copy.chars.push_back(keep(c, more));
+            acc = k == 0 ? copy : concat(cleaned(acc, 3), copy);
+        }
+        return cleaned(acc, 1);
+    }
+    // every block of noise above max_noise through a message-extract PBS
+    FheString cleaned(const FheString &s, uint64_t max_noise) {
+        FheString out = s;
+        for (auto &c : out.chars)
+            for (auto &blk : c)
+                if (blk.noise > max_noise || blk.degree >= p.msg_mod) blk = pg.pbs(blk, [this](uint64_t x) { return x % p.msg_mod; });
+        return out;
     }
 
     // ---- replace / replacen / split / splitn / split_once / rsplit_once: str's methods with a &str pattern ------------------------------
@@ -539,6 +588,72 @@ class PaddedStringServerKey {
         return lim;
     }
 
+    // ---- secret integer arguments: a radix of any number of digits, little endian ---------------------------------------------------
+    // the low nd digits, zero-extended, or all maximal when a higher digit is set: min(x, 4^nd - 1), so one comparison on nd digits decides
+    Radix clamp_radix(const Radix &x, size_t nd) {
+        Radix lo = resized(Radix(x.begin(), x.begin() + std::min(nd, x.size())), nd);
+        if (x.size() <= nd) return lo;
+        std::vector<Ct> high;
+        for (size_t j = nd; j < x.size(); ++j) high.push_back(pg.pbs(x[j], [](uint64_t v) { return uint64_t(v != 0); }));
+        const Ct over = isk.is_at_least_one_comparisons_block_true(high);
+        const uint64_t top = p.msg_mod - 1;
+        for (auto &d : lo) d = pg.pbs_bivariate(d, over, [top](uint64_t v, uint64_t o) { return (o & 1) ? top : v; });
+        return lo;
+    }
+    // sign of (a - b) for radixes of the same length: block signs by bivariate lookup, reduced with the comparator's tree; as in
+    // scalar_sign nothing is subtracted
+    Ct radix_sign(const Radix &a, const Radix &b) {
+        std::vector<Ct> signs;
+        for (size_t i = 0; i < a.size(); ++i)
+            signs.push_back(pg.pbs_bivariate(a[i], b[i], [](uint64_t x, uint64_t y) {
+                return x < y ? IntegerServerKey::IS_INFERIOR : (x == y ? IntegerServerKey::IS_EQUAL : IntegerServerKey::IS_SUPERIOR);
+            }));
+        return isk.reduce_signs(signs);
+    }
+    Radix resized(Radix r, size_t nd) {
+        while (r.size() < nd) r.push_back(pg.create_trivial(0));
+        r.resize(nd);
+        return r;
+    }
+    // first_matches with a secret limit (at least as many digits as the counts): acc[w] AND [cnt[w] < limit] (strict) or [cnt[w] <= limit]
+    std::vector<Ct> first_matches_below(const std::vector<Ct> &acc, const std::vector<Radix> &cnt, const Radix &limit, bool strict) {
+        std::vector<Ct> lim(acc.size());
+        for (size_t w = 0; w < acc.size(); ++w) {
+            if (is_const(acc[w], 0)) { lim[w] = acc[w]; continue; }
+            const Ct sign = radix_sign(resized(cnt[w], limit.size()), limit);
+            lim[w] = pg.pbs_bivariate(sign, acc[w], [strict](uint64_t s, uint64_t a) {
+                return uint64_t((strict ? s == IntegerServerKey::IS_INFERIOR : s != IntegerServerKey::IS_SUPERIOR) && (a & 1));
+            });
+        }
+        return lim;
+    }
+
+    // ends[e], e = 0 ..= capacity: one of the matches `starts` (window order, non-overlapping) ends at e.  A clear pattern of length m:
+    // starts[e - m].  A padded one: OR_d (starts[e - d] AND [len(pat) == d]); one length is true, so the terms are disjoint (built as
+    // `covered` is)
+    std::vector<Ct> match_ends(const std::vector<Ct> &starts, const Pattern &pt) {
+        const size_t n = starts.size() - 1, m = pt.chars.len();
+        std::vector<Ct> ends(n + 1, pg.create_trivial(0));
+        if (pt.clear) {
+            for (size_t e = m; e <= n; ++e) ends[e] = starts[e - m];
+            return ends;
+        }
+        const std::vector<Ct> is_len = length_onehot(nonzero_flags(pt.chars));   // d = 0 ..= cap_pat
+        for (size_t e = 0; e <= n; ++e) {
+            std::vector<Ct> t;
+            for (size_t d = 0; d <= std::min(e, m); ++d) t.push_back(and_flags(starts[e - d], is_len[d]));
+            ends[e] = onehot_sum(t, 1);
+        }
+        return ends;
+    }
+    // [the part at the end of the string is empty]: the string is empty, or one of the matches ends at its end
+    Ct end_part_empty(const FheString &s, const std::vector<Ct> &ends) {
+        const std::vector<Ct> at_len = length_onehot(nonzero_flags(s));
+        std::vector<Ct> t{at_len[0]};
+        for (size_t e = 1; e <= s.len(); ++e) t.push_back(and_flags(at_len[e], ends[e]));
+        return onehot_sum(t, 1);
+    }
+
     // removes the zero chars of s in order and returns the first out_len positions.  Char j moves left by the number D_j of zero chars
     // before it, one bit of D_j per stage, least significant first.  For non-zero chars j < j', D_j' - D_j <= j' - j - 1, so their
     // positions stay strictly increasing after every stage: no two chars ever meet, a stage is a sum of two keep_if per block, and the
@@ -584,16 +699,19 @@ class PaddedStringServerKey {
         return extend(out, out_len);
     }
 
-    // replacen (count = SIZE_MAX: replace).  Slot i of the expanded string holds `to` if an accepted match starts at i, then s[i] unless a
-    // match covers it; compacting the zero chars away gives the result
-    FheString replace(const FheString &s, const Pattern &pt, const FheString &to, size_t count) {
+    // replacen (count = SIZE_MAX: replace; secret_count: the first *secret_count matches, sized as replace).  Slot i of the expanded string
+    // holds `to` if an accepted match starts at i, then s[i] unless a match covers it; compacting the zero chars away gives the result
+    FheString replace(const FheString &s, const Pattern &pt, const FheString &to, size_t count, const Radix *secret_count = nullptr) {
         const size_t n = s.len(), m_min = pt.min_len(), M = max_matches(n, m_min);
         count = std::min(count, M);
         const size_t out_len = n + count * (to.len() > m_min ? to.len() - m_min : 0);
         if (count == 0) return s;
         Matches mt = find_all(s, pt);
         std::vector<Ct> acc = non_overlapping(mt.raw, mt.over);
-        if (count < M) acc = first_matches(acc, prefix_count(acc, digits_for(M)), count);
+        if (secret_count) {
+            std::vector<Radix> cnt = prefix_count(acc, digits_for(M));
+            acc = first_matches_below(acc, cnt, clamp_radix(*secret_count, digits_for(M)), false);
+        } else if (count < M) acc = first_matches(acc, prefix_count(acc, digits_for(M)), count);
         std::vector<Ct> cov = covered(acc, mt.cov, n);
         FheString ex;   // chars known to be zero are left out: compaction removes them anyway
         for (size_t i = 0; i <= n; ++i) {
@@ -622,33 +740,105 @@ class PaddedStringServerKey {
 
     // splitn (n_parts = SIZE_MAX: split): (part count as digits_for(P) digits, P parts of capacity chars), P = min(M + 1, n_parts).  Char i
     // belongs to part min(#accepted matches at or before i, P - 1) unless a match covers it; parts past the count are empty.
-    std::pair<Radix, std::vector<FheString>> split(const FheString &s, const Pattern &pt, size_t n_parts) {
+    //   reverse      rsplit / rsplitn: the rightmost non-overlapping matches (the reverse searcher: the chain runs from window `capacity`
+    //                down), and char i belongs to part #accepted matches after i, part 0 being the one at the end of the string
+    //   terminator   split_terminator / rsplit_terminator: the part at the end of the string is dropped when it is empty.  For split that
+    //                is the last part, which is then all zero already, so only the count drops; for rsplit it is part 0, so every char's
+    //                part index drops by that flag
+    //   secret_n     splitn_enc / rsplitn_enc: n is a radix, P = M + 1; the first n - 1 matches split, part n - 1 is the unsplit rest
+    std::pair<Radix, std::vector<FheString>> split(const FheString &s, const Pattern &pt, size_t n_parts, bool reverse = false,
+                                                   bool terminator = false, const Radix *secret_n = nullptr) {
         const size_t n = s.len(), M = max_matches(n, pt.min_len()), P = std::min(M + 1, n_parts), nd = digits_for(P);
         std::vector<FheString> parts;
         if (P == 0) return {trivial_radix(0, nd), parts};
-        if (P == 1) { parts.push_back(s); return {trivial_radix(1, nd), parts}; }
+        if (P == 1 && !terminator && !secret_n) { parts.push_back(s); return {trivial_radix(1, nd), parts}; }
         const size_t last = P - 1;
         Matches mt = find_all(s, pt);
-        std::vector<Ct> acc = non_overlapping(mt.raw, mt.over);
+        std::vector<Ct> raw = mt.raw;                                 // in the order the searcher meets the windows
+        if (reverse) std::reverse(raw.begin(), raw.end());
+        std::vector<Ct> acc = non_overlapping(raw, mt.over);
         std::vector<Radix> cnt = prefix_count(acc, digits_for(M));   // counts of every accepted match, up to M
-        std::vector<Ct> lim = last < M ? first_matches(acc, cnt, last) : acc;
+        const Radix limit = secret_n ? clamp_radix(*secret_n, nd) : Radix();
+        std::vector<Ct> lim = secret_n ? first_matches_below(acc, cnt, limit, true) : last < M ? first_matches(acc, cnt, last) : acc;
+        if (reverse) std::reverse(lim.begin(), lim.end());           // back to window order
         std::vector<Ct> cov = covered(lim, mt.cov, n);
+        // matches before char i in the searcher's order: at or before i, or (reverse) after i
+        auto count_at = [&](size_t i) -> const Radix & { return cnt[reverse ? n - 1 - i : i]; };
         // count = min(#matches, last) + 1: when there are fewer than `last` matches, their number fits nd digits
         Radix total(cnt[n].begin(), cnt[n].begin() + std::min(nd, cnt[n].size()));
         while (total.size() < nd) total.push_back(pg.create_trivial(0));
-        Radix count = isk.add(total, trivial_radix(1, nd));
-        if (last < M) {
+        Radix count;
+        Ct dropped;                                                    // terminator: the part at the end is empty
+        if (terminator) {
+            dropped = end_part_empty(s, match_ends(lim, pt));
+            count = isk.add(total, resized({isk.boolean_bitnot(dropped)}, nd));
+        } else count = isk.add(total, trivial_radix(1, nd));
+        if (secret_n) {                                                // min(#matches + 1, n)
+            Ct less = pg.pbs(radix_sign(count, limit), [](uint64_t x) { return uint64_t(x == IntegerServerKey::IS_INFERIOR); });
+            count = isk.if_then_else(less, count, limit);
+        } else if (last < M) {
             Ct more = pg.pbs(scalar_sign(cnt[n], last), [](uint64_t x) { return uint64_t(x != 0); });
             count = isk.if_then_else(more, trivial_radix(P, nd), count);
         }
-        for (size_t k = 0; k < P; ++k) {
+        // member(k, i): char i is in part k (of split / rsplit / splitn / rsplitn); in_part(k)[i]: char i goes to part k of the result
+        auto member = [&](size_t k, size_t i) {
+            const bool tail = k == last;
+            return pg.pbs_bivariate(scalar_sign(count_at(i), k), cov[i], [tail](uint64_t sg, uint64_t c) {
+                return uint64_t((tail ? sg != 0 : sg == 1) && !(c & 1));
+            });
+        };
+        std::vector<std::vector<Ct>> members;                         // rsplit_terminator: [char i is in rsplit's part k], every k
+        if (reverse && terminator)
+            for (size_t k = 0; k < P; ++k) {
+                members.emplace_back(n);
+                for (size_t i = 0; i < n; ++i) members[k][i] = member(k, i);
+            }
+        std::vector<Ct> n_sign(P);                                     // secret n: sign of n - (k + 1)
+        if (secret_n)
+            for (size_t k = 0; k < P; ++k) n_sign[k] = scalar_sign(limit, k + 1);
+        auto in_part = [&](size_t k) {
             std::vector<Ct> in(n);
             for (size_t i = 0; i < n; ++i) {
-                const bool tail = k == last;
-                in[i] = pg.pbs_bivariate(scalar_sign(cnt[i], k), cov[i], [tail](uint64_t sg, uint64_t c) {
-                    return uint64_t((tail ? sg != 0 : sg == 1) && !(c & 1));
-                });
+                if (reverse && terminator) {                           // part k of the result is rsplit's part k + dropped
+                    const Ct next = k + 1 < P ? members[k + 1][i] : pg.create_trivial(0);
+                    in[i] = pg.pbs_bivariate(pg.unchecked_add(members[k][i], pg.unchecked_scalar_mul(next, 2)), dropped,
+                                             [](uint64_t x, uint64_t d) { return (d & 1) ? (x >> 1) & 1 : x & 1; });
+                } else if (secret_n) {                                 // [cnt == k and k < n - 1] or [cnt >= k and k == n - 1]
+                    Ct g = pg.pbs(pg.unchecked_add(scalar_sign(count_at(i), k), pg.unchecked_scalar_mul(n_sign[k], 3)), [](uint64_t x) {
+                        const uint64_t sg = x % 3, ns = x / 3;
+                        return uint64_t((ns == IntegerServerKey::IS_SUPERIOR && sg == IntegerServerKey::IS_EQUAL) ||
+                                        (ns == IntegerServerKey::IS_EQUAL && sg != IntegerServerKey::IS_INFERIOR));
+                    });
+                    in[i] = pg.pbs_bivariate(g, cov[i], [](uint64_t x, uint64_t c) { return uint64_t((x & 1) && !(c & 1)); });
+                } else in[i] = member(k, i);
             }
+            return in;
+        };
+        for (size_t k = 0; k < P; ++k) {
+            std::vector<Ct> in = in_part(k);
+            if (k == 0 && !reverse) {   // part 0 starts at 0
+                FheString p0;
+                for (size_t i = 0; i < n; ++i) p0.chars.push_back(keep(s.chars[i], in[i]));
+                parts.push_back(p0);
+            } else parts.push_back(part(s, in));
+        }
+        return {count, parts};
+    }
+
+    // split_inclusive: the leftmost matches, each part keeping the match that ends it, and a trailing empty part dropped.  Char i belongs to
+    // part #matches ending at or before i (covered chars included); count = #matches + [the part at the end is not empty]; P = M + 1.
+    std::pair<Radix, std::vector<FheString>> split_inclusive(const FheString &s, const Pattern &pt) {
+        const size_t n = s.len(), M = max_matches(n, pt.min_len()), P = M + 1, nd = digits_for(P);
+        Matches mt = find_all(s, pt);
+        const std::vector<Ct> ends = match_ends(non_overlapping(mt.raw, mt.over), pt);
+        std::vector<Radix> cnt = prefix_count(ends, digits_for(M));
+        const Ct trailing = isk.boolean_bitnot(end_part_empty(s, ends));
+        Radix count = isk.add(resized(cnt[n], nd), resized({trailing}, nd));
+        std::vector<FheString> parts;
+        for (size_t k = 0; k < P; ++k) {
+            std::vector<Ct> in(n);
+            for (size_t i = 0; i < n; ++i)
+                in[i] = pg.pbs(scalar_sign(cnt[i], k), [](uint64_t x) { return uint64_t(x == IntegerServerKey::IS_EQUAL); });
             if (k == 0) {   // part 0 starts at 0
                 FheString p0;
                 for (size_t i = 0; i < n; ++i) p0.chars.push_back(keep(s.chars[i], in[i]));
@@ -656,6 +846,37 @@ class PaddedStringServerKey {
             } else parts.push_back(part(s, in));
         }
         return {count, parts};
+    }
+
+    // split_ascii_whitespace: the non-empty runs of chars that are neither padding nor u8::is_ascii_whitespace (U+0009, U+000A, U+000C,
+    // U+000D, U+0020 -- not U+000B, which char::is_whitespace and char_class include).  Word k holds the chars after the (k + 1)-th word
+    // start; P = ceil(capacity / 2) parts.
+    Ct ascii_word_char(const Radix &c) {
+        Ct hi = pg.unchecked_add(pg.unchecked_scalar_mul(c[3], p.msg_mod), c[2]);
+        Ct lo = pg.unchecked_add(pg.unchecked_scalar_mul(c[1], p.msg_mod), c[0]);
+        Ct k = pg.pbs(hi, [](uint64_t x) { return x == 0 ? uint64_t(1) : (x == 2 ? uint64_t(2) : uint64_t(0)); });
+        Ct r = pg.pbs(lo, [](uint64_t x) { return x == 0 ? uint64_t(2) : ((x == 9 || x == 10 || x == 12 || x == 13) ? uint64_t(1) : uint64_t(0)); });
+        return pg.pbs_bivariate(k, r, [](uint64_t kk, uint64_t rr) {
+            return uint64_t(!((kk == 1 && rr != 0) || (kk == 2 && rr == 2)));   // 0x00, 0x09, 0x0A, 0x0C, 0x0D, 0x20
+        });
+    }
+    std::pair<Radix, std::vector<FheString>> split_ascii_whitespace(const FheString &s) {
+        const size_t n = s.len(), P = (n + 1) / 2, nd = digits_for(P);
+        std::vector<FheString> parts;
+        if (n == 0) return {trivial_radix(0, nd), parts};
+        std::vector<Ct> word(n), start(n);
+        for (size_t i = 0; i < n; ++i) word[i] = ascii_word_char(s.chars[i]);
+        start[0] = word[0];
+        for (size_t i = 1; i < n; ++i)
+            start[i] = pg.pbs(pg.unchecked_add(word[i], pg.unchecked_scalar_mul(word[i - 1], 2)), [](uint64_t x) { return uint64_t(x == 1); });
+        std::vector<Radix> cnt = prefix_count(start, nd);
+        for (size_t k = 0; k < P; ++k) {
+            std::vector<Ct> in(n);
+            for (size_t i = 0; i < n; ++i)
+                in[i] = pg.pbs_bivariate(scalar_sign(cnt[i], k + 1), word[i], [](uint64_t sg, uint64_t w) { return uint64_t(sg == IntegerServerKey::IS_EQUAL && (w & 1)); });
+            parts.push_back(part(s, in));
+        }
+        return {cnt[n - 1], parts};
     }
 
     // split_once / rsplit_once: (found, before, after) around the first (last: the last, as rfind finds it) match; both strings are empty

@@ -104,6 +104,106 @@ bool record_split_replace(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh
     return true;
 }
 
+// The rest of the split family, the ops with a secret integer argument, the padded-pattern strip_prefix / strip_suffix and the padded
+// eq_ignore_case; include/tfhe_b200.h gives every output layout.  A secret integer is a radix input of count_blocks blocks appended after
+// the strings.  Every argument is checked before anything is recorded.
+bool record_padded_extra(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh::StringServerKey &ssk, const std::string &op,
+                         const std::string &f, const uint64_t *a, size_t na, const char *clear, std::string &err) {
+    static const std::map<std::string, std::vector<std::string>> kArgs = {
+        {"rsplit", {"capacity", "capacity_pat"}}, {"rsplitn", {"capacity", "capacity_pat", "n"}},
+        {"split_terminator", {"capacity", "capacity_pat"}}, {"rsplit_terminator", {"capacity", "capacity_pat"}},
+        {"split_inclusive", {"capacity", "capacity_pat"}}, {"split_ascii_whitespace", {"capacity"}},
+        {"repeat_enc", {"capacity", "max_count", "count_blocks"}},
+        {"replacen_enc", {"capacity", "capacity_from", "capacity_to", "count_blocks"}},
+        {"splitn_enc", {"capacity", "capacity_pat", "n_blocks"}}, {"rsplitn_enc", {"capacity", "capacity_pat", "n_blocks"}},
+        {"strip_prefix", {"capacity", "capacity_pat"}}, {"strip_suffix", {"capacity", "capacity_pat"}},
+        {"eq_ignore_case", {"capacity_a", "capacity_b"}}};
+    const std::vector<std::string> &names = kArgs.at(f);
+    if (na < names.size()) {
+        std::string list;
+        for (auto &nm : names) list += (list.empty() ? "" : ", ") + nm;
+        err = op + ": expected " + std::to_string(names.size()) + " integer arguments {" + list + "}";
+        return false;
+    }
+    const bool has_pattern = names.size() > 1 && names[1] != "max_count";
+    if (clear && !has_pattern) {
+        err = op + ": takes no clear operand";
+        return false;
+    }
+    if (clear && std::strlen(clear) != a[1]) {
+        err = op + ": the pattern capacity " + std::to_string(a[1]) + " differs from the clear pattern's length " + std::to_string(std::strlen(clear));
+        return false;
+    }
+    const bool secret = f.size() > 4 && f.compare(f.size() - 4, 4, "_enc") == 0;
+    const uint64_t blocks = secret ? a[names.size() - 1] : 0;
+    if (secret && (blocks < 1 || blocks > 16)) {
+        err = op + ": " + names.back() + " must be 1 ..= 16, got " + std::to_string(blocks);
+        return false;
+    }
+    // sizes arrive from outside: bound every string and the result before anything is recorded (slot indices are 32-bit)
+    constexpr uint64_t kMaxChars = uint64_t(1) << 20;
+    const size_t n_sizes = names.size() - (secret || f == "rsplitn" ? 1 : 0);   // capacities (and repeat_enc's max_count)
+    for (size_t i = 0; i < n_sizes; ++i)
+        if (a[i] > kMaxChars) {
+            err = op + ": capacities are limited to " + std::to_string(kMaxChars) + " chars";
+            return false;
+        }
+    const uint64_t cap = a[0], m_min = clear ? a[1] : 0, M = tbh::PaddedStringServerKey::max_matches(cap, m_min);
+    unsigned __int128 chars = cap;   // the largest string the program holds at once
+    if (f == "repeat_enc") chars = (unsigned __int128)cap * a[1];
+    else if (f == "replacen_enc") {
+        const uint64_t cap_to = a[2];
+        chars = std::max((unsigned __int128)(cap + 1) * (cap_to + 1), (unsigned __int128)cap + (unsigned __int128)M * (cap_to > m_min ? cap_to - m_min : 0));
+    } else if (f == "split_ascii_whitespace") chars = (unsigned __int128)((cap + 1) / 2) * cap;
+    else if (f.find("split") != std::string::npos) chars = (unsigned __int128)(f == "rsplitn" ? std::min<uint64_t>(M + 1, a[2]) : M + 1) * cap;
+    if (chars > kMaxChars) {
+        err = op + ": the result or the expanded string would exceed " + std::to_string(kMaxChars) + " chars";
+        return false;
+    }
+
+    tbh::FheString s = ssk.input_string(cap);
+    if (f == "split_ascii_whitespace") {
+        auto r = psk.split_ascii_whitespace(s);
+        output_radix(pg, r.first);
+        for (auto &part : r.second) output_string(pg, part);
+        return true;
+    }
+    if (f == "repeat_enc") {
+        tbh::Radix count = input_radix(pg, blocks);
+        output_string(pg, psk.repeat(s, count, a[1]));
+        return true;
+    }
+    if (f == "eq_ignore_case") {
+        tbh::FheString t = clear ? ssk.trivial_string(clear) : ssk.input_string(a[1]);
+        pg.output(psk.eq_ignore_case(s, t));
+        return true;
+    }
+    if (f == "strip_prefix" || f == "strip_suffix") {   // the padded pattern (a clear one takes the form without capacity_pat)
+        tbh::FheString pat = ssk.input_string(a[1]);
+        auto r = f == "strip_prefix" ? psk.strip_prefix(s, pat) : psk.strip_suffix(s, pat);
+        pg.output(r.first);
+        output_string(pg, r.second);
+        return true;
+    }
+    const tbh::PaddedStringServerKey::Pattern pt = clear ? psk.clear_pattern(clear) : psk.padded_pattern(ssk.input_string(a[1]));
+    if (f == "replacen_enc") {
+        tbh::FheString to = ssk.input_string(a[2]);
+        tbh::Radix count = input_radix(pg, blocks);
+        output_string(pg, psk.replace(s, pt, to, SIZE_MAX, &count));
+        return true;
+    }
+    std::pair<tbh::Radix, std::vector<tbh::FheString>> r;
+    const bool reverse = f[0] == 'r';
+    if (f == "split_inclusive") r = psk.split_inclusive(s, pt);
+    else if (secret) {
+        tbh::Radix n = input_radix(pg, blocks);
+        r = psk.split(s, pt, SIZE_MAX, reverse, false, &n);
+    } else r = psk.split(s, pt, f == "rsplitn" ? a[2] : SIZE_MAX, reverse, f.find("terminator") != std::string::npos);
+    output_radix(pg, r.first);
+    for (auto &part : r.second) output_string(pg, part);
+    return true;
+}
+
 // records `op`; returns false with a message when the op / arguments are unknown
 bool record(tfhe_b200_program &h, const std::string &op_in, const uint64_t *a, size_t na, const char *clear, std::string &err) {
     tbh::Program &pg = *h.prog;
@@ -257,6 +357,14 @@ bool record(tfhe_b200_program &h, const std::string &op_in, const uint64_t *a, s
         const std::string f = op.substr(8);
         if (f == "replace" || f == "replacen" || f == "split" || f == "splitn" || f == "split_once" || f == "rsplit_once")
             return record_split_replace(pg, psk, ssk, op, f, a, na, clear, err);
+        if (f == "strip_prefix" || f == "strip_suffix") {
+            if (!clear && na < 2) { err = op + ": needs a clear pattern, or {capacity, capacity_pat} and a padded pattern input"; return false; }
+            if (!clear) return record_padded_extra(pg, psk, ssk, op, f, a, na, clear, err);
+        }
+        if (f == "rsplit" || f == "rsplitn" || f == "split_terminator" || f == "rsplit_terminator" || f == "split_inclusive" ||
+            f == "split_ascii_whitespace" || f == "repeat_enc" || f == "replacen_enc" || f == "splitn_enc" || f == "rsplitn_enc" ||
+            f == "eq_ignore_case")
+            return record_padded_extra(pg, psk, ssk, op, f, a, na, clear, err);
         tbh::FheString s = ssk.input_string(a[0]);
         if (f == "len") { output_radix(pg, psk.len(s)); return true; }
         if (f == "is_empty") { pg.output(psk.is_empty(s)); return true; }

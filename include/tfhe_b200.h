@@ -160,10 +160,28 @@ int tfhe_b200_pbs_batch_partial(tfhe_b200_ctx *ctx, const uint64_t *lwe_small, c
  *     blocks), then P parts of capacity chars, P = M + 1 (splitn: min(M + 1, n); the last part is the unsplit rest; n = 0: count 0)
  *   pstring_split_once / pstring_rsplit_once {capacity, capacity_pat}: inputs s, pat -> found, before, after (capacity chars each; both
  *     empty when nothing is found).  rsplit_once splits at the last match as rfind finds it
+ *   pstring_{rsplit,split_terminator,rsplit_terminator,split_inclusive} {capacity, capacity_pat}  pstring_rsplitn {capacity, capacity_pat, n}:
+ *     inputs s, pat -> the part count (ceil(log4(P + 1)) blocks), then P parts of capacity chars, P = M + 1 (rsplitn: min(M + 1, n)).
+ *     rsplit / rsplitn: the rightmost non-overlapping matches, parts in Rust's order from the end (rsplitn: the last part is the unsplit
+ *     prefix; n = 0: count 0).  split_terminator / rsplit_terminator: split / rsplit without the part at the end of the string when that
+ *     part is empty.  split_inclusive: each part keeps the match that ends it; an empty part at the end is dropped
+ *   pstring_split_ascii_whitespace {capacity}: input s -> the word count, then P = ceil(capacity / 2) words of capacity chars; words are
+ *     separated by the bytes of u8::is_ascii_whitespace (U+0009, U+000A, U+000C, U+000D, U+0020; not U+000B)
+ *   secret integers (the _enc ops): a radix of count_blocks 2-bit blocks (1 ..= 16, little endian), the last input
+ *   pstring_repeat_enc {capacity, max_count, count_blocks}: inputs s, count -> capacity * max_count chars: s repeated min(count, max_count)
+ *     times (a count above max_count is clamped to it)
+ *   pstring_replacen_enc {capacity, capacity_from, capacity_to, count_blocks}: inputs s, from, to, count -> the first `count` matches
+ *     replaced (all of them when count >= M), in the C = capacity + M * max(0, capacity_to - m_min) chars of replace
+ *   pstring_splitn_enc / pstring_rsplitn_enc {capacity, capacity_pat, n_blocks}: inputs s, pat, n -> the part count (ceil(log4(M + 2))
+ *     blocks), then M + 1 parts of capacity chars: splitn / rsplitn with n parts at most (n = 0: count 0)
+ *   pstring_{strip_prefix,strip_suffix} {capacity, capacity_pat} without a clear operand: inputs s, pat (padded) -> matched, the string
+ *   pstring_eq_ignore_case {capacity_a, capacity_b}: inputs a, b (or a and the clear b, capacity_b its length) -> one boolean block:
+ *     a and b equal after the ASCII case fold
  *     -- Rust's str methods with a &str pattern: leftmost non-overlapping matches, the empty pattern matching at every char boundary
  *        0 ..= len.  With clear_operand != NULL it is the pattern (from / pat, not an input) and capacity_from / capacity_pat must equal
  *        its length.  m_min is the least pattern length (0 for a padded pattern, the length of a clear one) and M the most matches:
- *        capacity + 1 when m_min = 0, else capacity / m_min.  Parts past the count are all zero.
+ *        capacity + 1 when m_min = 0, else capacity / m_min.  Parts past the count are all zero.  Capacities, and the chars of the result
+ *        and of replace's expanded string, are limited to 2^20.
  *     -- NULL-PADDED strings: public capacity, secret length, content followed by zero bytes (host/padded.h); len returns a radix of
  *        ceil(log4(capacity + 1)) blocks, the string-valued ops return 4 blocks per char of the result capacity
  * Appending "_packed" to a string op (or radix_eq) selects packed block equalities: one PBS per PAIR of blocks built from
