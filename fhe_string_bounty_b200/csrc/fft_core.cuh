@@ -273,6 +273,34 @@ TB_HD int32_t signed_digit_l1(uint64_t x, int base_log) {
     return (int32_t)r - (int32_t)((r > half) ? (1u << base_log) : 0u);
 }
 
+// Gather of the rotated polynomial: u = (j - a) << (31 - kLogN) carries the source index d = (j - a) mod 2N with its wrap bit
+// (d >= N: the word enters negated) on top.  Returns poly[d mod N] and sets `wrap` to all ones for a wrapped word, else 0; both are
+// shifts of u (no index masking, no 64-bit negation), and u for j + c is u + (c << (31 - kLogN)).
+TB_HD uint64_t rot_gather(const uint64_t *poly, uint32_t u, uint32_t &wrap) {
+    wrap = (uint32_t)((int32_t)u >> 31);
+    return *reinterpret_cast<const uint64_t *>(reinterpret_cast<const char *>(poly) + ((u << 1) >> (29 - kLogN)));
+}
+
+// signed_digit_l1(+-r - o, base_log) of the rotated gather (r: gathered word, wrap: rot_gather's mask, all ones when r enters
+// negated; o: own word),
+// computed from the high word of the complement only:
+//   ~(+-r - o) = o + (r ^ ~M) + M,  M = wrap in both words          (one three-input add with carry)
+//   signed_digit_l1(x) = -( (int32)(hi(~x) + 2^(31-B)) >> (32-B) )  (rounding half up on x is rounding half down on -x, and the
+//                                                                    arithmetic shift lands in [-B/2, B/2): no tie fix-up)
+// For 2 <= base_log <= 30 it equals signed_digit_l1 for every input (tests/test_rot_digit.py checks the classes that matter).
+TB_HD int32_t rot_sub_digit(uint64_t r, uint32_t wrap, uint64_t o, int base_log) {
+    uint32_t xl = (uint32_t)r, xh = (uint32_t)(r >> 32);
+#if defined(__CUDA_ARCH__)
+    // one LOP3 per word (the compiler splits ~(a ^ b) into two)
+    asm("lop3.b32 %0, %0, %2, 0, 0xC3;\n\tlop3.b32 %1, %1, %2, 0, 0xC3;" : "+r"(xl), "+r"(xh) : "r"(wrap));
+#else
+    xl = ~(xl ^ wrap); xh = ~(xh ^ wrap);
+#endif
+    const uint64_t M = ((uint64_t)wrap << 32) | wrap;
+    const uint32_t nh = (uint32_t)((o + (((uint64_t)xh << 32) | xl) + M) >> 32);
+    return -((int32_t)(nh + (1u << (31 - base_log))) >> (32 - base_log));
+}
+
 // commons/math/torus/mod.rs:72-78 with the x86 rounding the reference actually runs (half-to-even,
 // fft/x86.rs:859-867): fract = t - rint(t); (i64) rint(fract * 2^64).
 TB_HD uint64_t from_torus_f64(double t) {

@@ -14,7 +14,9 @@
 // registers: +9 % time), exchange A through Tensor Memory with a ciphertext's four warps in one lane quarter (shared-memory pipe 76 ->
 // 47 %, but +31 % instructions for uniform-register address moves, warp-part twiddles and spills: +34 % time).  Kept: the two
 // polynomials of a ciphertext in the two halves of each warp, so that the spectrum exchange of the external product is a lane ^ 16
-// shuffle (two barriers and 32 shared-memory instructions per thread and iteration fewer).
+// shuffle (two barriers and 32 shared-memory instructions per thread and iteration fewer).  The rotated gather takes its byte offset
+// and wrap mask as shifts of one index and its digit from the high word of one three-input add (fft_core.cuh rot_gather /
+// rot_sub_digit): the main loop of the 4-per-SM instance went from 2 815 to 2 623 instructions, 98.2 -> 95.0 ms per 8192 (B200).
 // Shared memory per 4-ciphertext CTA: 8 x 17 KiB polynomial tiles (rotated-gather source, then exchange tile) + 5 x 16 KiB ring.
 // TMEM: 64 columns per ciphertext (accumulator master copy) + 80 columns of per-thread FFT twiddles.
 // Named barriers: one per ciphertext (128 threads).
@@ -158,14 +160,12 @@ pbs_classic_kernel_v4(const uint64_t *__restrict__ lwe_small, const uint32_t *__
 #pragma unroll
         for (int m = 0; m < 16; ++m) {
             const int j = T + 64 * m;
-            const uint32_t s0 = ((uint32_t)j - a) & (2 * kN - 1);
-            const uint32_t s1 = (s0 + kM) & (2 * kN - 1);
-            uint64_t r0 = pb[s0 & (kN - 1)], r1 = pb[s1 & (kN - 1)];
-            r0 = (s0 >= (uint32_t)kN) ? (uint64_t)0 - r0 : r0;
-            r1 = (s1 >= (uint32_t)kN) ? (uint64_t)0 - r1 : r1;
             const uint64_t o0 = (uint64_t)__double_as_longlong(re[m]), o1 = (uint64_t)__double_as_longlong(im[m]);
-            re[m] = (double)signed_digit_l1(r0 - o0, base_log);
-            im[m] = (double)signed_digit_l1(r1 - o1, base_log);
+            const uint32_t u = ((uint32_t)j - a) << (31 - kLogN);
+            uint32_t wrap0, wrap1;
+            const uint64_t r0 = rot_gather(pb, u, wrap0), r1 = rot_gather(pb, u + ((uint32_t)kM << (31 - kLogN)), wrap1);
+            re[m] = (double)rot_sub_digit(r0, wrap0, o0, base_log);
+            im[m] = (double)rot_sub_digit(r1, wrap1, o1, base_log);
         }
         fft16_fwd(re, im, tile, twd, T, ct_sync);    // its first barrier also ends the rotated gather: nobody writes the tile before it
 

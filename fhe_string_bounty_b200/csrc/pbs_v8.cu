@@ -143,14 +143,12 @@ pbs_classic_kernel_v8(const uint64_t *__restrict__ lwe_small, const uint32_t *__
 #pragma unroll
         for (int m = 0; m < 8; ++m) {
             const int j = T + 128 * m;
-            const uint32_t s0 = ((uint32_t)j - a) & (2 * kN - 1);
-            const uint32_t s1 = (s0 + kM) & (2 * kN - 1);
-            uint64_t r0 = pb[s0 & (kN - 1)], r1 = pb[s1 & (kN - 1)];
-            r0 = (s0 >= (uint32_t)kN) ? (uint64_t)0 - r0 : r0;
-            r1 = (s1 >= (uint32_t)kN) ? (uint64_t)0 - r1 : r1;
             const uint64_t o0 = (uint64_t)__double_as_longlong(re[m]), o1 = (uint64_t)__double_as_longlong(im[m]);
-            re[m] = (double)signed_digit_l1(r0 - o0, base_log);
-            im[m] = (double)signed_digit_l1(r1 - o1, base_log);
+            const uint32_t u = ((uint32_t)j - a) << (31 - kLogN);
+            uint32_t wrap0, wrap1;
+            const uint64_t r0 = rot_gather(pb, u, wrap0), r1 = rot_gather(pb, u + ((uint32_t)kM << (31 - kLogN)), wrap1);
+            re[m] = (double)rot_sub_digit(r0, wrap0, o0, base_log);
+            im[m] = (double)rot_sub_digit(r1, wrap1, o1, base_log);
         }
 
         if (REGS) fft8_fwd(re, im, tile, twd_r, T, poly_sync); else fft8_fwd(re, im, tile, twd_t, T, poly_sync);
