@@ -37,6 +37,9 @@ int check_params(const tfhe_b200_params &p) {
     if (p.pbs_base_log < 2 || p.pbs_base_log > 30) return fail("unsupported pbs_base_log");
     if (p.ks_level < 1 || p.ks_base_log < 2 || p.ks_base_log > 7 || p.ks_base_log * p.ks_level > 31)
         return fail("unsupported keyswitch decomposition");
+    if ((int)p.ks_level > tbk::ks_max_level())    // the IMAD kernel (the only one above 7 levels) stages 8 * ks_level key rows per step
+        return fail("unsupported ks_level " + std::to_string(p.ks_level) + ": at most " + std::to_string(tbk::ks_max_level()) +
+                    " levels (the keyswitch's shared-memory stages need 17 408 bytes per level, 227 KB per block)");
     if (p.lwe_dim < 1 || p.lwe_dim > 4096) return fail("unsupported lwe_dim");
     if (p.grouping_factor != 0 && p.grouping_factor != 2 && p.grouping_factor != 3)
         return fail("unsupported grouping_factor (0 = classic, 2 or 3 = multi-bit)");
@@ -249,7 +252,8 @@ int tfhe_b200_ctx_create(int cuda_device, const tfhe_b200_params *params, tfhe_b
     c->tuned512 = c->generic && tbk::pbs_n512_supported((int)params->poly_size, (int)params->glwe_dim, (int)params->pbs_level, (int)params->grouping_factor);
     if (const char *e = std::getenv("TFHE_B200_TUNED512")) if (e[0] == '0') c->tuned512 = false;
     if (c->tuned512) TB_CUDA(tbk::pbs_n512_configure());
-    c->tuned8192 = c->generic && tbk::pbs_n8192_supported((int)params->poly_size, (int)params->glwe_dim, (int)params->pbs_level, (int)params->grouping_factor);
+    c->tuned8192 = c->generic && tbk::pbs_n8192_supported((int)params->poly_size, (int)params->glwe_dim, (int)params->pbs_level, (int)params->pbs_base_log,
+                                                              (int)params->grouping_factor);
     if (const char *e = std::getenv("TFHE_B200_TUNED8192")) if (e[0] == '0') c->tuned8192 = false;
     if (c->tuned8192) TB_CUDA(tbk::pbs_n8192_configure());
     TB_CUDA(tbk::pbs_v4_configure());
@@ -267,7 +271,7 @@ int tfhe_b200_ctx_create(int cuda_device, const tfhe_b200_params *params, tfhe_b
         TB_CUDA(c->roots.reserve(r.size() * 8));
         TB_CUDA(cudaMemcpy(c->roots.p, r.data(), r.size() * 8, cudaMemcpyHostToDevice));
     }
-    TB_CUDA(tbk::ks_configure((int)params->ks_level));
+    TB_CUDA(tbk::ks_configure());
     // twiddle tables of the 16- and 8-points-per-thread FFTs
     std::vector<double> tbl16(c->tuned8192 ? 2 * 4352 : 2 * (tb::kM + 64));
     if (c->tuned8192) tbk::pbs_n8192_make_table(tbl16.data());
@@ -309,7 +313,8 @@ int tfhe_b200_set_tuning(tfhe_b200_ctx *c, const char *key, int value) {
         c->narrow_max = value;
     } else if (k == "tuned8192") {
         if (value != 0 && value != 1) return fail("tuned8192 must be 0 or 1");
-        if (value == 1 && !(c->bskf8.p && tbk::pbs_n8192_supported((int)c->p.poly_size, (int)c->p.glwe_dim, (int)c->p.pbs_level, (int)c->p.grouping_factor)))
+        if (value == 1 && !(c->bskf8.p && tbk::pbs_n8192_supported((int)c->p.poly_size, (int)c->p.glwe_dim, (int)c->p.pbs_level,
+                                                                        (int)c->p.pbs_base_log, (int)c->p.grouping_factor)))
             return fail("tuned8192: not this parameter shape, or the key was uploaded without the tuned copy");
         c->tuned8192 = value;
     } else if (k == "tuned512_min") {

@@ -8,7 +8,8 @@ namespace tbk {
 
 // keyswitch.cu
 int ks_padded_cols(int n);
-cudaError_t ks_configure(int level);
+int ks_max_level();          // the largest level count whose two pipeline stages fit in 227 KB of shared memory
+cudaError_t ks_configure();
 cudaError_t launch_ksk_pack(const uint64_t *ksk, uint64_t *packed, uint64_t *colsum, int rows, int n, cudaStream_t stream);
 cudaError_t launch_keyswitch(const uint64_t *lwe_in, const uint32_t *in_slot, const uint64_t *ksk_packed, const uint64_t *colsum, uint64_t *lwe_out,
                              int batch, int in_dim, int n, int base_log, int level, cudaStream_t stream);
@@ -90,7 +91,7 @@ cudaError_t launch_bsk_convert_n512(const uint64_t *bsk_std, void *bskf, const v
 
 // pbs_n8192.cu: tuned blind rotation for N = 8192, k = 1, two levels (PARAM_MESSAGE_3_CARRY_3_KS_PBS and siblings): one ciphertext per
 // two-SM cluster; tbl = 4096 + 256 complex twiddles
-bool pbs_n8192_supported(int poly_size, int glwe_dim, int pbs_level, int grouping_factor);
+bool pbs_n8192_supported(int poly_size, int glwe_dim, int pbs_level, int pbs_base_log, int grouping_factor);
 void pbs_n8192_make_table(double *t /* 2 * 4352 doubles */);
 cudaError_t pbs_n8192_configure();
 cudaError_t launch_pbs_n8192(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskf, const void *tbl,

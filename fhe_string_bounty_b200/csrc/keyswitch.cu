@@ -169,9 +169,17 @@ namespace tbk {
 
 int ks_padded_cols(int n) { return ((n + 1 + tbks::TILE_J - 1) / tbks::TILE_J) * tbks::TILE_J; }
 
-cudaError_t ks_configure(int level) {
+int ks_max_level() {
+    int level = 1;
+    while (tbks::ks_smem_bytes(level + 1) <= 227 * 1024) ++level;
+    return level;                                   // 13: 17 408 bytes per level
+}
+
+// The limit is a property of the kernel on the current device, shared by every context of the process: it is set to what the largest
+// supported level count needs, so that a context created later (with fewer levels) cannot lower it below an earlier context's launch.
+cudaError_t ks_configure() {
     return cudaFuncSetAttribute(tbks::keyswitch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)tbks::ks_smem_bytes(level));
+                                (int)tbks::ks_smem_bytes(ks_max_level()));
 }
 
 cudaError_t launch_ksk_pack(const uint64_t *ksk, uint64_t *packed, uint64_t *colsum, int rows, int n, cudaStream_t stream) {

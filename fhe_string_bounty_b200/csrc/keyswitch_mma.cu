@@ -3,7 +3,9 @@
 // Same result, bit for bit, as keyswitch.cu / core_crypto/algorithms/lwe_keyswitch.rs:96-170: the keyswitch IS a dense
 // integer GEMM  out[b][j] = body_b*[j==n] - sum_r digit[b][r] * KSK[r][j]  (r = mask element x level) in Z/2^64.  The
 // u64 key is split into its 8 byte planes, the signed digits are biased to unsigned bytes (d' = d + B/2), and
-//     S_p[b][j] = sum_r d'[b][r] * byte_p(KSK[r][j])            (u8 x u8 -> s32, exact: <= 10240*8*255 < 2^31)
+//     S_p[b][j] = sum_r d'[b][r] * byte_p(KSK[r][j])            (u8 x u8 -> s32, wrapping; < 2^32, u32 zero-extended: exact)
+// S_p <= K * B * 255 with d' <= B = 2^base_log; the worst accepted shape, kN = 32768 at (base_log, level) = (7, 4), bounds it by
+// 4.28e9 (4.25e9 reachable), above 2^31: the epilogue reads each plane sum as a u32.
 // runs as 8 interleaved int8 GEMM columns on mma.sync.m16n8k32 (one n8 tile = the 8 planes of one KSK column), then
 //     sum_r d' * KSK = sum_p S_p << 8p  (mod 2^64),    out = body*[j==n] + B/2 * colsum[j] - that.
 // Two kernels: ks_digits_kernel writes the digit matrix once (decomposer.rs:98-152, iter.rs:120-127), ks_mma_kernel is a

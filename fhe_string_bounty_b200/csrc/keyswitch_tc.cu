@@ -1,7 +1,9 @@
 // keyswitch_tc.cu -- the keyswitch GEMM on the 5th-generation tensor cores: tcgen05.mma kind::i8, operands staged by TMA, accumulators in
 // Tensor Memory.  Same arithmetic, bit for bit, as keyswitch_mma.cu (the mma.sync version, kept as the A/B reference) and as
 // core_crypto/algorithms/lwe_keyswitch.rs:96-170:
-//     S_p[b][j] = sum_r d'[b][r] * byte_p(KSK[r][j])      u8 x u8 -> s32, exact (<= K * 255 * 255 < 2^31 for every supported set)
+//     S_p[b][j] = sum_r d'[b][r] * byte_p(KSK[r][j])      u8 x u8 -> s32 accumulator, read back as u32 and zero-extended: exact, since
+//                                                          S_p <= K * B * 255 < 2^32 for every accepted shape (d' <= B = 2^base_log; worst
+//                                                          kN = 32768 at (base_log, level) = (7, 4): 4.28e9 bound, 4.25e9 reachable)
 //     out[b][j] = body_b * [j == n] + B/2 * colsum[j] - sum_p S_p << 8p          (mod 2^64)
 // with d' = signed digit + B/2 written once per batch by ks_digits_kernel, and the key split into its 8 byte planes at upload
 // (bmat[n = 8 j + p][k], k contiguous): both operands are K-major byte matrices, exactly what the tensor core wants.

@@ -431,8 +431,10 @@ bsk_convert_n8192_kernel(const uint64_t *__restrict__ bsk_std, cplx *__restrict_
 
 namespace tbk {
 
-bool pbs_n8192_supported(int poly_size, int glwe_dim, int pbs_level, int grouping_factor) {
-    return poly_size == tb8192::N && glwe_dim == 1 && pbs_level == tb8192::LEVELS && grouping_factor == 0;
+// signed_digits2 works on the top 32 bits of a word: base_log * LEVELS <= 31.  Larger bases (accepted up to B * l = 52) run on
+// pbs_generic.cu, whose decomposition is 64-bit.
+bool pbs_n8192_supported(int poly_size, int glwe_dim, int pbs_level, int pbs_base_log, int grouping_factor) {
+    return poly_size == tb8192::N && glwe_dim == 1 && pbs_level == tb8192::LEVELS && pbs_base_log * tb8192::LEVELS <= 31 && grouping_factor == 0;
 }
 
 void pbs_n8192_make_table(double *t) { tb16x_make_table_8192(t); }
