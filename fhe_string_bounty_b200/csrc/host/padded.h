@@ -523,7 +523,8 @@ class PaddedStringServerKey {
         std::vector<Ct> raw;         // windows 0 ..= capacity: the pattern occurs at w (and w is inside the string or at its end)
         std::vector<Ct> over, cov;   // d = 0 .. cap_pat - 1: matches d apart can overlap (d >= 1) / a match covers the char d after its start
     };
-    Matches find_all(const FheString &hay, const Pattern &pt) {
+    // hay_nz: where given, receives nonzero_flags(hay) when a padded pattern needs them (left untouched otherwise)
+    Matches find_all(const FheString &hay, const Pattern &pt, std::vector<Ct> *hay_nz = nullptr) {
         const size_t n = hay.len(), m = pt.chars.len();
         Matches r;
         r.raw.assign(n + 1, pg.create_trivial(0));
@@ -550,6 +551,7 @@ class PaddedStringServerKey {
             Ct mw = w < n ? window_match(hay, pt.chars, w, pz) : isk.are_all_comparisons_block_true(pz);
             r.raw[w] = w > 0 ? isk.boolean_bitand(mw, nz[w - 1]) : mw;
         }
+        if (hay_nz) *hay_nz = nz;
         for (size_t d = 0; d < m; ++d) r.cov.push_back(isk.boolean_bitnot(pz[d]));   // [the pattern is longer than d]
         r.over = r.cov;
         return r;
@@ -861,11 +863,17 @@ class PaddedStringServerKey {
         });
     }
     std::pair<Radix, std::vector<FheString>> split_ascii_whitespace(const FheString &s) {
+        if (s.len() == 0) return words(s, {});
+        std::vector<Ct> word(s.len());
+        for (size_t i = 0; i < s.len(); ++i) word[i] = ascii_word_char(s.chars[i]);
+        return words(s, word);
+    }
+    // the words of s given the flags [char i is a word char] (padding is not): count, then P = ceil(capacity / 2) words
+    std::pair<Radix, std::vector<FheString>> words(const FheString &s, const std::vector<Ct> &word) {
         const size_t n = s.len(), P = (n + 1) / 2, nd = digits_for(P);
         std::vector<FheString> parts;
         if (n == 0) return {trivial_radix(0, nd), parts};
-        std::vector<Ct> word(n), start(n);
-        for (size_t i = 0; i < n; ++i) word[i] = ascii_word_char(s.chars[i]);
+        std::vector<Ct> start(n);
         start[0] = word[0];
         for (size_t i = 1; i < n; ++i)
             start[i] = pg.pbs(pg.unchecked_add(word[i], pg.unchecked_scalar_mul(word[i - 1], 2)), [](uint64_t x) { return uint64_t(x == 1); });
@@ -904,6 +912,237 @@ class PaddedStringServerKey {
         for (size_t i = 0; i < n; ++i) b.chars.push_back(keep(s.chars[i], before[i]));
         return {found, b, part(s, after)};
     }
+
+    // ---- matches / match_indices / rmatch_indices / trim_start_matches / trim_end_matches: the rest of str's &str-pattern methods ------
+    // matches(pat) always yields the pattern itself, so its iterator carries only a count.  There is no separate rmatches count: with
+    // every match of one length, greedy selection from the left and from the right both find a largest set of non-overlapping matches,
+    // so the two counts are equal (the empty pattern: len + 1 either way).
+    // the number of set flags as nd digits (a tree of radix additions, each on as many digits as its partial sums can fill)
+    Radix count_flags(const std::vector<Ct> &f, size_t nd) {
+        std::vector<std::pair<Radix, size_t>> c;   // partial sums and their largest value
+        for (auto &x : f)
+            if (!is_const(x, 0)) c.push_back({Radix{x}, 1});
+        if (c.empty()) return trivial_radix(0, nd);
+        while (c.size() > 1) {
+            std::vector<std::pair<Radix, size_t>> nxt;
+            for (size_t i = 0; i + 1 < c.size(); i += 2) {
+                const size_t bound = c[i].second + c[i + 1].second, used = std::min(nd, digits_for(bound));
+                nxt.push_back({isk.add(resized(c[i].first, used), resized(c[i + 1].first, used)), bound});
+            }
+            if (c.size() % 2) nxt.push_back(c.back());
+            c.swap(nxt);
+        }
+        return resized(c[0].first, nd);
+    }
+    // s.matches(pat).count(), digits_for(M) digits
+    Radix matches(const FheString &s, const Pattern &pt) {
+        const size_t M = max_matches(s.len(), pt.min_len());
+        if (M == 0) return trivial_radix(0, 1);
+        Matches mt = find_all(s, pt);
+        return count_flags(non_overlapping(mt.raw, mt.over), digits_for(M));
+    }
+    // (count, M byte indices of digits_for(capacity) digits): the leftmost non-overlapping matches in order, or (reverse) the rightmost
+    // ones from the end, as rsplit's reverse searcher finds them.  Index k is the window w with acc[w] and cnt[w] == k + 1 (in the
+    // searcher's order), its radix the window's byte index; indices past the count are zero
+    std::pair<Radix, std::vector<Radix>> match_indices(const FheString &s, const Pattern &pt, bool reverse) {
+        const size_t n = s.len(), m_min = pt.min_len(), M = max_matches(n, m_min), nd = digits_for(M), ni = digits_for(n);
+        std::vector<Radix> idx;
+        if (M == 0) return {trivial_radix(0, nd), idx};
+        Matches mt = find_all(s, pt);
+        std::vector<Ct> raw = mt.raw;                                // in the order the searcher meets the windows
+        if (reverse) std::reverse(raw.begin(), raw.end());
+        const std::vector<Ct> acc = non_overlapping(raw, mt.over);
+        const std::vector<Radix> cnt = prefix_count(acc, nd);
+        for (size_t k = 0; k < M; ++k) {
+            std::vector<Ct> sel(n + 1, pg.create_trivial(0));
+            for (size_t r = 0; r <= n; ++r) {
+                // matches are at least m_min apart: at most r / m_min + 1 of them (r + 1 for m_min = 0) up to the r-th window
+                if (is_const(acc[r], 0) || k > (m_min ? r / m_min : r)) continue;
+                sel[r] = pg.pbs_bivariate(scalar_sign(cnt[r], k + 1), acc[r], [](uint64_t sg, uint64_t a) {
+                    return uint64_t(sg == IntegerServerKey::IS_EQUAL && (a & 1));
+                });
+            }
+            idx.push_back(onehot_to_radix(sel, ni, [=](size_t r) { return uint64_t(reverse ? n - r : r); }));
+        }
+        return {cnt[n], idx};
+    }
+    // [len(pat) == d], d = 0 ..= capacity_pat, of a padded pattern
+    std::vector<Ct> pattern_length_onehot(const Pattern &pt) { return length_onehot(nonzero_flags(pt.chars)); }
+    // trim_start_matches: the run of back-to-back matches at the start goes (next_reject).  For a pattern length d the run covers chars
+    // i < d j_d, j_d the first window 0, d, 2 d, ... that does not match; a padded pattern computes every d = 1 ..= capacity_pat and
+    // selects with [len(pat) == d], so no chain over the string is needed.  The rest moves to the start in one `part`
+    FheString trim_start_matches(const FheString &s, const Pattern &pt) {
+        const size_t n = s.len(), m = pt.chars.len();
+        if (m == 0 || (pt.clear && m > n)) return s;   // the empty pattern, or no match fits
+        std::vector<Ct> raw(n + 1, pg.create_trivial(0)), is_len;
+        if (pt.clear)   // only the windows at multiples of m
+            for (size_t w = 0; w + m <= n; w += m) raw[w] = ssk.window_matches(s, pt.chars, w, w + 1)[0];
+        else {
+            raw = find_all(s, pt).raw;
+            is_len = pattern_length_onehot(pt);
+        }
+        std::vector<std::vector<Ct>> terms(n);          // [char i is in the run] for each candidate length: at most one is set
+        for (size_t d = pt.clear ? m : 1; d <= m && d <= n; ++d) {
+            std::vector<Ct> fail;
+            for (size_t w = 0; w + d <= n; w += d) fail.push_back(isk.boolean_bitnot(raw[w]));
+            const std::vector<Ct> broken = prefix_or(fail, true);    // some window 0, d, ..., j d does not match
+            const Ct sel = pt.clear ? pg.create_trivial(1) : is_len[d];
+            for (size_t i = 0; i < fail.size() * d; ++i) terms[i].push_back(and_flags(sel, isk.boolean_bitnot(broken[i / d])));
+        }
+        std::vector<Ct> in(n);
+        for (size_t i = 0; i < n; ++i) in[i] = isk.boolean_bitnot(onehot_sum(terms[i], 5));   // part() adds 3 in[]: <= 15
+        return part(s, in);
+    }
+    // trim_end_matches: the run of back-to-back matches that ends at the secret end of the string goes (next_reject_back).  For a
+    // pattern length d the run consists of the windows w = len - d, len - 2 d, ... down to the first that does not match.  Char i lies in
+    // the window w_r(i) = the largest w <= i with w == r (mod d), r = len mod d, and goes iff no window w' >= w_r(i) of that residue class
+    // below len fails: a suffix OR over the class, with one term per residue selected by [len == r (mod d)] (from length_onehot) and, for
+    // a padded pattern, by [len(pat) == d].  Only a suffix is masked; nothing moves
+    FheString trim_end_matches(const FheString &s, const Pattern &pt) {
+        const size_t n = s.len(), m = pt.chars.len();
+        if (m == 0 || (pt.clear && m > n)) return s;
+        std::vector<Ct> nz, is_len;
+        const std::vector<Ct> raw = find_all(s, pt, &nz).raw;
+        if (pt.clear) nz = nonzero_flags(s);
+        else is_len = pattern_length_onehot(pt);
+        const std::vector<Ct> at_len = length_onehot(nz);
+        std::vector<Ct> fail(n);                        // [w < len and no match at w]
+        for (size_t w = 0; w < n; ++w)
+            fail[w] = is_const(raw[w], 0) ? nz[w] : pg.pbs_bivariate(raw[w], nz[w], [](uint64_t r, uint64_t z) { return uint64_t(!(r & 1) && (z & 1)); });
+        std::vector<std::vector<Ct>> terms(n);          // at most one term per char is set: one length, one residue
+        for (size_t d = pt.clear ? m : 1; d <= m && d <= n; ++d) {
+            const Ct sel = pt.clear ? pg.create_trivial(1) : is_len[d];
+            for (size_t r = 0; r < d; ++r) {
+                std::vector<Ct> t;
+                for (size_t e = r; e <= n; e += d) t.push_back(at_len[e]);
+                const Ct res = and_flags(sel, onehot_sum(t, 1));           // [len(pat) == d and len == r (mod d)]
+                if (is_const(res, 0)) continue;
+                std::vector<Ct> chain;                                     // the windows r, r + d, ... < n, last first
+                for (size_t w = r; w < n; w += d) chain.push_back(fail[w]);
+                std::reverse(chain.begin(), chain.end());
+                std::vector<Ct> bad = prefix_or(chain, true);             // some failure at or after the window
+                std::reverse(bad.begin(), bad.end());
+                for (size_t i = r; i < n; ++i) terms[i].push_back(and_flags(res, isk.boolean_bitnot(bad[(i - r) / d])));
+            }
+        }
+        FheString out = s;
+        for (size_t i = 0; i < n; ++i) out.chars[i] = keep(s.chars[i], isk.boolean_bitnot(onehot_sum(terms[i], p.total_mod() - 1 - 4)));
+        return out;
+    }
+
+    // ---- lines / split_whitespace -------------------------------------------------------------------------------------------------
+    // a property of the byte c as one table lookup on hcode(high nibble) * mul + lcode(low nibble), given the two nibble codes (PBS
+    // outputs).  The table is derived from the property over all 256 bytes; two bytes it tells apart must differ in their codes
+    Ct byte_lookup(const Ct &hc, const Ct &lc, uint64_t mul, uint64_t (*hcode)(uint64_t), uint64_t (*lcode)(uint64_t), uint64_t (*prop)(uint64_t)) {
+        std::vector<int> table(p.total_mod(), -1);
+        for (uint64_t b = 0; b < 256; ++b) {
+            const uint64_t x = hcode(b >> 4) * mul + lcode(b & 15), v = prop(b);
+            if (x >= table.size() || (table[x] >= 0 && uint64_t(table[x]) != v)) throw std::logic_error("byte_lookup: the nibble codes do not separate the property");
+            table[x] = int(v);
+        }
+        return pg.pbs(pg.unchecked_add(pg.unchecked_scalar_mul(hc, mul), lc), [table](uint64_t x) { return uint64_t(std::max(table[x], 0)); });
+    }
+    Ct high_nibble(const Radix &c) { return pg.unchecked_add(pg.unchecked_scalar_mul(c[3], p.msg_mod), c[2]); }
+    Ct low_nibble(const Radix &c) { return pg.unchecked_add(pg.unchecked_scalar_mul(c[1], p.msg_mod), c[0]); }
+    Ct nibble_code(const Ct &nib, uint64_t (*code)(uint64_t)) { return pg.pbs(nib, [code](uint64_t x) { return code(x); }); }
+
+    // lines: split_inclusive on "\n", then a trailing "\n" or "\r\n" stripped from each line (a bare "\r" at the end stays).  Char i
+    // belongs to line #("\n" before i) unless it is a "\n" or the "\r" of a "\r\n"; count = #"\n" + [the part at the end is not empty].
+    // (count as digits_for(capacity) digits, capacity lines of capacity chars)
+    std::pair<Radix, std::vector<FheString>> lines(const FheString &s) {
+        const size_t n = s.len(), nd = digits_for(n);
+        std::vector<FheString> parts;
+        if (n == 0) return {trivial_radix(0, nd), parts};
+        static uint64_t (*const h0)(uint64_t) = [](uint64_t h) { return uint64_t(h == 0); };
+        static uint64_t (*const lnr)(uint64_t) = [](uint64_t l) { return l == 0xA ? uint64_t(1) : (l == 0xD ? uint64_t(2) : uint64_t(0)); };
+        std::vector<Ct> nl(n), cr(n);
+        for (size_t i = 0; i < n; ++i) {
+            const Ct hc = nibble_code(high_nibble(s.chars[i]), h0), lc = nibble_code(low_nibble(s.chars[i]), lnr);
+            nl[i] = byte_lookup(hc, lc, 3, h0, lnr, [](uint64_t b) { return uint64_t(b == '\n'); });
+            cr[i] = byte_lookup(hc, lc, 3, h0, lnr, [](uint64_t b) { return uint64_t(b == '\r'); });
+        }
+        std::vector<Ct> in_line(n), ends(n + 1, pg.create_trivial(0));
+        for (size_t i = 0; i < n; ++i) {
+            Ct y = pg.unchecked_add(nl[i], pg.unchecked_scalar_mul(cr[i], 2));
+            if (i + 1 < n) y = pg.unchecked_add(y, pg.unchecked_scalar_mul(nl[i + 1], 4));
+            in_line[i] = pg.pbs(y, [](uint64_t x) { return uint64_t(!(x & 1) && (x & 6) != 6); });
+            ends[i + 1] = nl[i];
+        }
+        const std::vector<Radix> cnt = prefix_count(nl, nd);
+        const Ct trailing = isk.boolean_bitnot(end_part_empty(s, ends));
+        const Radix count = isk.add(resized(cnt[n - 1], nd), resized({trailing}, nd));
+        for (size_t k = 0; k < n; ++k) {
+            std::vector<Ct> in(n, pg.create_trivial(0));
+            for (size_t i = k; i < n; ++i) {                           // before char i there are at most i newlines
+                const Radix before = i > 0 ? cnt[i - 1] : trivial_radix(0, nd);
+                in[i] = pg.pbs_bivariate(scalar_sign(before, k), in_line[i], [](uint64_t sg, uint64_t l) {
+                    return uint64_t(sg == IntegerServerKey::IS_EQUAL && (l & 1));
+                });
+            }
+            if (k == 0) {   // line 0 starts at 0
+                FheString p0;
+                for (size_t i = 0; i < n; ++i) p0.chars.push_back(keep(s.chars[i], in[i]));
+                parts.push_back(p0);
+            } else parts.push_back(part(s, in));
+        }
+        return {count, parts};
+    }
+
+    // split_whitespace: the words between runs of char::is_whitespace, the 25 code points of Unicode White_Space: U+0009 ..= U+000D,
+    // U+0020, U+0085, U+00A0, U+1680, U+2000 ..= U+200A, U+2028, U+2029, U+202F, U+205F, U+3000.  Every occurrence of their UTF-8
+    // sequences is a separator: 09 ..= 0D, 20; C2 85, C2 A0; E1 9A 80, E2 80 80 ..= E2 80 8A, E2 80 A8, E2 80 A9, E2 80 AF, E2 81 9F,
+    // E3 80 80.  For valid UTF-8 that is Rust's result (UTF-8 is self-synchronising); for other bytes this rule is the definition.  The
+    // occurrences never overlap (each starts at an ASCII or lead byte, the rest are continuation bytes).
+    // Each byte is classified once: two high-nibble and five low-nibble codes, then seven table lookups give its roles (separator byte or
+    // padding, C2, lead E1 / E2 / E3, second byte 9A / 80 / 81, C2's second byte 85 / A0, third byte 80 / {81 ..= 8A, A8, A9, AF} / 9F);
+    // neighbours are combined by three more lookups ("second and third byte", "lead and tail", "C2 and its second byte") and the word
+    // flag is one lookup on the sum of the covering occurrences: 18 PBS per byte
+    std::vector<Ct> unicode_word_chars(const FheString &s) {
+        const size_t n = s.len();
+        static uint64_t (*const hW)(uint64_t) = [](uint64_t h) { return h == 0 ? uint64_t(1) : h == 2 ? uint64_t(2) : h == 0xC ? uint64_t(3) : h == 0xE ? uint64_t(4) : uint64_t(0); };
+        static uint64_t (*const hK)(uint64_t) = [](uint64_t h) { return h == 8 ? uint64_t(1) : h == 9 ? uint64_t(2) : h == 0xA ? uint64_t(3) : uint64_t(0); };
+        static uint64_t (*const lW)(uint64_t) = [](uint64_t l) { return l == 0 ? uint64_t(1) : (l >= 9 && l <= 0xD) ? uint64_t(2) : uint64_t(0); };
+        static uint64_t (*const lL)(uint64_t) = [](uint64_t l) { return l >= 1 && l <= 3 ? l : uint64_t(0); };
+        static uint64_t (*const lA)(uint64_t) = [](uint64_t l) { return l == 0 ? uint64_t(1) : l == 1 ? uint64_t(2) : l == 0xA ? uint64_t(3) : uint64_t(0); };
+        static uint64_t (*const lB)(uint64_t) = [](uint64_t l) { return (l >= 2 && l <= 7) ? uint64_t(1) : (l == 8 || l == 9) ? uint64_t(2) : l == 0xF ? uint64_t(3) : uint64_t(0); };
+        static uint64_t (*const lE)(uint64_t) = [](uint64_t l) { return l == 0 ? uint64_t(1) : l == 5 ? uint64_t(2) : uint64_t(0); };
+        std::vector<Ct> brk(n), lead(n), c2(n), sec(n), s2(n), thd(n);
+        for (size_t i = 0; i < n; ++i) {
+            const Ct hi = high_nibble(s.chars[i]), lo = low_nibble(s.chars[i]);
+            const Ct hw = nibble_code(hi, hW), hk = nibble_code(hi, hK);
+            const Ct lw = nibble_code(lo, lW), ll = nibble_code(lo, lL), la = nibble_code(lo, lA), lb = nibble_code(lo, lB), le = nibble_code(lo, lE);
+            brk[i] = byte_lookup(hw, lw, 3, hW, lW, [](uint64_t b) { return uint64_t(b == 0 || (b >= 0x09 && b <= 0x0D) || b == 0x20); });
+            lead[i] = byte_lookup(hw, ll, 3, hW, lL, [](uint64_t b) { return b >= 0xE1 && b <= 0xE3 ? b - 0xE0 : uint64_t(0); });
+            c2[i] = byte_lookup(hw, ll, 3, hW, lL, [](uint64_t b) { return uint64_t(b == 0xC2); });
+            sec[i] = byte_lookup(hk, la, 4, hK, lA, [](uint64_t b) { return b == 0x9A ? uint64_t(1) : b == 0x80 ? uint64_t(2) : b == 0x81 ? uint64_t(3) : uint64_t(0); });
+            s2[i] = byte_lookup(hk, le, 3, hK, lE, [](uint64_t b) { return uint64_t(b == 0x85 || b == 0xA0); });
+            // third byte: 1 = 80, 2 = 81 ..= 8A, A8, A9, AF, 3 = 9F; the two lookups see disjoint low nibbles, so their sum is the code
+            const Ct ta = byte_lookup(hk, la, 4, hK, lA, [](uint64_t b) { return b == 0x80 ? uint64_t(1) : (b == 0x81 || b == 0x8A) ? uint64_t(2) : uint64_t(0); });
+            const Ct tb = byte_lookup(hk, lb, 4, hK, lB, [](uint64_t b) {
+                return (b >= 0x82 && b <= 0x89) || b == 0xA8 || b == 0xA9 || b == 0xAF ? uint64_t(2) : b == 0x9F ? uint64_t(3) : uint64_t(0);
+            });
+            thd[i] = add_disjoint(ta, tb, 3);
+        }
+        // tail[j]: bytes j, j + 1 are 9A 80 (1: after E1), 80 80 (2: after E2 or E3), 80 {81 ..= 8A, A8, A9, AF} or 81 9F (3: after E2)
+        std::vector<Ct> tail(n, pg.create_trivial(0)), occ3(n, pg.create_trivial(0)), occ2(n, pg.create_trivial(0));
+        for (size_t j = 0; j + 1 < n; ++j)
+            tail[j] = pg.pbs_bivariate(sec[j], thd[j + 1], [](uint64_t a, uint64_t t) {
+                return a == 1 && t == 1 ? uint64_t(1) : a == 2 && t == 1 ? uint64_t(2) : (a == 2 && t == 2) || (a == 3 && t == 3) ? uint64_t(3) : uint64_t(0);
+            });
+        for (size_t i = 0; i + 2 < n; ++i)
+            occ3[i] = pg.pbs_bivariate(lead[i], tail[i + 1], [](uint64_t l, uint64_t t) { return uint64_t((l == 1 && t == 1) || (l == 2 && t >= 2) || (l == 3 && t == 2)); });
+        for (size_t i = 0; i + 1 < n; ++i)
+            occ2[i] = pg.pbs_bivariate(c2[i], s2[i + 1], [](uint64_t a, uint64_t b) { return uint64_t((a & 1) && (b & 1)); });
+        std::vector<Ct> word(n);
+        for (size_t i = 0; i < n; ++i) {
+            Ct y = pg.unchecked_add(brk[i], pg.unchecked_add(occ2[i], occ3[i]));
+            if (i >= 1) y = pg.unchecked_add(y, pg.unchecked_add(occ2[i - 1], occ3[i - 1]));
+            if (i >= 2) y = pg.unchecked_add(y, occ3[i - 2]);
+            word[i] = pg.pbs(y, [](uint64_t x) { return uint64_t(x == 0); });
+        }
+        return word;
+    }
+    std::pair<Radix, std::vector<FheString>> split_whitespace(const FheString &s) { return words(s, unicode_word_chars(s)); }
 
     Program &pg;
     IntegerServerKey isk;

@@ -104,8 +104,9 @@ bool record_split_replace(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh
     return true;
 }
 
-// The rest of the split family, the ops with a secret integer argument, the padded-pattern strip_prefix / strip_suffix and the padded
-// eq_ignore_case; include/tfhe_b200.h gives every output layout.  A secret integer is a radix input of count_blocks blocks appended after
+// The rest of the split family, the ops with a secret integer argument, the padded-pattern strip_prefix / strip_suffix, the padded
+// eq_ignore_case, matches / match_indices / rmatch_indices / trim_start_matches / trim_end_matches, lines and split_whitespace;
+// include/tfhe_b200.h gives every output layout.  A secret integer is a radix input of count_blocks blocks appended after
 // the strings.  Every argument is checked before anything is recorded.
 bool record_padded_extra(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh::StringServerKey &ssk, const std::string &op,
                          const std::string &f, const uint64_t *a, size_t na, const char *clear, std::string &err) {
@@ -117,7 +118,10 @@ bool record_padded_extra(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh:
         {"replacen_enc", {"capacity", "capacity_from", "capacity_to", "count_blocks"}},
         {"splitn_enc", {"capacity", "capacity_pat", "n_blocks"}}, {"rsplitn_enc", {"capacity", "capacity_pat", "n_blocks"}},
         {"strip_prefix", {"capacity", "capacity_pat"}}, {"strip_suffix", {"capacity", "capacity_pat"}},
-        {"eq_ignore_case", {"capacity_a", "capacity_b"}}};
+        {"eq_ignore_case", {"capacity_a", "capacity_b"}},
+        {"matches", {"capacity", "capacity_pat"}}, {"match_indices", {"capacity", "capacity_pat"}},
+        {"rmatch_indices", {"capacity", "capacity_pat"}}, {"trim_start_matches", {"capacity", "capacity_pat"}},
+        {"trim_end_matches", {"capacity", "capacity_pat"}}, {"lines", {"capacity"}}, {"split_whitespace", {"capacity"}}};
     const std::vector<std::string> &names = kArgs.at(f);
     if (na < names.size()) {
         std::string list;
@@ -154,7 +158,9 @@ bool record_padded_extra(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh:
     else if (f == "replacen_enc") {
         const uint64_t cap_to = a[2];
         chars = std::max((unsigned __int128)(cap + 1) * (cap_to + 1), (unsigned __int128)cap + (unsigned __int128)M * (cap_to > m_min ? cap_to - m_min : 0));
-    } else if (f == "split_ascii_whitespace") chars = (unsigned __int128)((cap + 1) / 2) * cap;
+    } else if (f == "split_ascii_whitespace" || f == "split_whitespace") chars = (unsigned __int128)((cap + 1) / 2) * cap;
+    else if (f == "lines") chars = (unsigned __int128)cap * cap;
+    else if (f == "match_indices" || f == "rmatch_indices") chars = (unsigned __int128)M * (cap + 1);   // one selection flag per match and window
     else if (f.find("split") != std::string::npos) chars = (unsigned __int128)(f == "rsplitn" ? std::min<uint64_t>(M + 1, a[2]) : M + 1) * cap;
     if (chars > kMaxChars) {
         err = op + ": the result or the expanded string would exceed " + std::to_string(kMaxChars) + " chars";
@@ -162,8 +168,8 @@ bool record_padded_extra(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh:
     }
 
     tbh::FheString s = ssk.input_string(cap);
-    if (f == "split_ascii_whitespace") {
-        auto r = psk.split_ascii_whitespace(s);
+    if (f == "split_ascii_whitespace" || f == "split_whitespace" || f == "lines") {
+        auto r = f == "lines" ? psk.lines(s) : f == "split_whitespace" ? psk.split_whitespace(s) : psk.split_ascii_whitespace(s);
         output_radix(pg, r.first);
         for (auto &part : r.second) output_string(pg, part);
         return true;
@@ -190,6 +196,20 @@ bool record_padded_extra(tbh::Program &pg, tbh::PaddedStringServerKey &psk, tbh:
         tbh::FheString to = ssk.input_string(a[2]);
         tbh::Radix count = input_radix(pg, blocks);
         output_string(pg, psk.replace(s, pt, to, SIZE_MAX, &count));
+        return true;
+    }
+    if (f == "matches") {
+        output_radix(pg, psk.matches(s, pt));
+        return true;
+    }
+    if (f == "match_indices" || f == "rmatch_indices") {
+        auto r = psk.match_indices(s, pt, f == "rmatch_indices");
+        output_radix(pg, r.first);
+        for (auto &idx : r.second) output_radix(pg, idx);
+        return true;
+    }
+    if (f == "trim_start_matches" || f == "trim_end_matches") {
+        output_string(pg, f == "trim_start_matches" ? psk.trim_start_matches(s, pt) : psk.trim_end_matches(s, pt));
         return true;
     }
     std::pair<tbh::Radix, std::vector<tbh::FheString>> r;
@@ -363,7 +383,8 @@ bool record(tfhe_b200_program &h, const std::string &op_in, const uint64_t *a, s
         }
         if (f == "rsplit" || f == "rsplitn" || f == "split_terminator" || f == "rsplit_terminator" || f == "split_inclusive" ||
             f == "split_ascii_whitespace" || f == "repeat_enc" || f == "replacen_enc" || f == "splitn_enc" || f == "rsplitn_enc" ||
-            f == "eq_ignore_case")
+            f == "eq_ignore_case" || f == "matches" || f == "match_indices" || f == "rmatch_indices" || f == "trim_start_matches" ||
+            f == "trim_end_matches" || f == "lines" || f == "split_whitespace")
             return record_padded_extra(pg, psk, ssk, op, f, a, na, clear, err);
         tbh::FheString s = ssk.input_string(a[0]);
         if (f == "len") { output_radix(pg, psk.len(s)); return true; }

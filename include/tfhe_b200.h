@@ -177,6 +177,21 @@ int tfhe_b200_pbs_batch_partial(tfhe_b200_ctx *ctx, const uint64_t *lwe_small, c
  *   pstring_{strip_prefix,strip_suffix} {capacity, capacity_pat} without a clear operand: inputs s, pat (padded) -> matched, the string
  *   pstring_eq_ignore_case {capacity_a, capacity_b}: inputs a, b (or a and the clear b, capacity_b its length) -> one boolean block:
  *     a and b equal after the ASCII case fold
+ *   pstring_matches {capacity, capacity_pat}: inputs s, pat -> s.matches(pat).count() as ceil(log4(M + 1)) blocks.  There is no separate
+ *     rmatches count: with every match of one length, greedy selection from the left and from the right both find a largest set of
+ *     non-overlapping matches, so the two counts are equal (the empty pattern: len + 1 either way)
+ *   pstring_match_indices / pstring_rmatch_indices {capacity, capacity_pat}: inputs s, pat -> the count (ceil(log4(M + 1)) blocks), then
+ *     M byte indices of ceil(log4(capacity + 1)) blocks each: the leftmost non-overlapping matches in order (rmatch_indices: the
+ *     rightmost ones as the reverse searcher finds them, last match first); indices past the count are zero.  M * (capacity + 1) is
+ *     limited to 2^20
+ *   pstring_trim_start_matches / pstring_trim_end_matches {capacity, capacity_pat}: inputs s, pat -> capacity chars: s without the run of
+ *     back-to-back matches at its start / at its (secret) end; the empty pattern returns s
+ *   pstring_lines {capacity}: input s -> the line count (ceil(log4(capacity + 1)) blocks), then capacity lines of capacity chars: s split
+ *     after every "\n", each line without its "\n" or "\r\n" (a bare "\r" at the end stays), no empty line after a final "\n"
+ *   pstring_split_whitespace {capacity}: input s -> the word count, then P = ceil(capacity / 2) words of capacity chars; words are separated
+ *     by char::is_whitespace (Unicode White_Space), i.e. every occurrence of the UTF-8 sequences 09 ..= 0D, 20, C2 85, C2 A0, E1 9A 80,
+ *     E2 80 80 ..= E2 80 8A, E2 80 A8, E2 80 A9, E2 80 AF, E2 81 9F, E3 80 80.  For valid UTF-8 that is Rust's result; for other bytes
+ *     this rule is the definition.  lines and split_whitespace take no clear operand
  *     -- Rust's str methods with a &str pattern: leftmost non-overlapping matches, the empty pattern matching at every char boundary
  *        0 ..= len.  With clear_operand != NULL it is the pattern (from / pat, not an input) and capacity_from / capacity_pat must equal
  *        its length.  m_min is the least pattern length (0 for a padded pattern, the length of a clear one) and M the most matches:
