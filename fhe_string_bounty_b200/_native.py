@@ -1,7 +1,8 @@
 """ctypes loader for libtfhe_b200.so and a small numpy-facing wrapper around the C ABI.
 
 Nothing here computes: every method forwards to an ``extern "C"`` entry point declared in
-``include/tfhe_b200.h`` (EXPORTS) or ``include/tfhe_b200_sharded.h`` (SHARDED_EXPORTS).  Missing library or missing GPU
+``include/tfhe_b200.h`` (EXPORTS), ``include/tfhe_b200_sharded.h`` (SHARDED_EXPORTS) or ``include/tfhe_b200_many_lut.h``
+(MANY_LUT_EXPORTS).  Missing library or missing GPU
 raises NativeError (no fallback).
 """
 from __future__ import annotations
@@ -16,7 +17,7 @@ import numpy as np
 _PKG = Path(__file__).resolve().parent
 _SO = _PKG / "libtfhe_b200.so"
 _SOURCES = ["csrc/pbs_v4.cu", "csrc/pbs_v8.cu", "csrc/pbs_multibit_v4.cu", "csrc/pbs_multibit_v8.cu", "csrc/pbs_generic.cu", "csrc/pbs_n512.cu", "csrc/pbs_n8192.cu", "csrc/keyswitch.cu", "csrc/keyswitch_mma.cu", "csrc/keyswitch_tc.cu", "csrc/leveled.cu", "csrc/seeded.cu", "csrc/probe.cu", "csrc/exchange.cu", "csrc/c_api.cu", "csrc/host_api.cu"]
-_HEADERS = ["csrc/fft_core.cuh", "csrc/fft16_core.cuh", "csrc/fft8_core.cuh", "csrc/fft16x_slots.cuh", "csrc/pbs16_common.cuh", "csrc/pbs8_common.cuh", "csrc/ring_helpers.cuh", "csrc/kernels.h", "csrc/ctx.h", "csrc/host/program.h", "csrc/host/radix.h", "csrc/host/strings.h", "csrc/host/padded.h", "../include/tfhe_b200.h", "../include/tfhe_b200_sharded.h"]
+_HEADERS = ["csrc/fft_core.cuh", "csrc/fft16_core.cuh", "csrc/fft8_core.cuh", "csrc/fft16x_slots.cuh", "csrc/pbs16_common.cuh", "csrc/pbs8_common.cuh", "csrc/ring_helpers.cuh", "csrc/sample_extract.cuh", "csrc/kernels.h", "csrc/ctx.h", "csrc/host/program.h", "csrc/host/radix.h", "csrc/host/strings.h", "csrc/host/padded.h", "../include/tfhe_b200.h", "../include/tfhe_b200_sharded.h", "../include/tfhe_b200_many_lut.h"]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
@@ -234,7 +235,40 @@ SHARDED_EXPORTS = {
                                                       C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint64, C.c_void_p]),
 }
 
+# include/tfhe_b200_many_lut.h: many-LUT PBS
+MANY_LUT_EXPORTS = {
+    "tfhe_b200_upload_many_luts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
+    "tfhe_b200_pbs_many_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
+    "tfhe_b200_pbs_many_batch_partial": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32]),
+    "tfhe_b200_ks_pbs_many_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
+    "tfhe_b200_pbs_many_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "tfhe_b200_ks_pbs_many_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+}
+
 _lib = None
+
+
+def many_lut_accumulator(params: dict | Params, fns) -> np.ndarray:
+    """tfhe-rs generate_many_lookup_table (shortint/server_key/mod.rs): the (k + 1) * N accumulator that stacks the F = len(fns)
+    functions, f_f(x) * Delta in box f * chunk + x for x < chunk = total // F (total = msg_mod * carry_mod), 0 in the boxes from F * chunk
+    on, then the half-box negation and rotation of generate_lookup_table.  Upload with Engine.upload_many_luts."""
+    p = params if isinstance(params, Params) else Params(**params)
+    total, N = p.msg_mod * p.carry_mod, p.poly_size
+    F = len(fns)
+    if not 2 <= F <= total:
+        raise ValueError(f"a many-LUT accumulator holds 2 ... msg_mod * carry_mod = {total} functions, not {F}")
+    chunk, box = total // F, N // total
+    delta = (1 << 63) // total
+    boxes = np.zeros(total, dtype=np.uint64)
+    for f, fn in enumerate(fns):
+        for x in range(chunk):
+            boxes[f * chunk + x] = (int(fn(x)) * delta) & (2**64 - 1)
+    body = np.repeat(boxes, box)
+    half = box // 2
+    body[:half] = np.uint64(0) - body[:half]
+    acc = np.zeros(p.lut_len, dtype=np.uint64)
+    acc[p.glwe_dim * N:] = np.roll(body, -half)
+    return acc
 
 
 def load_native():
@@ -245,7 +279,7 @@ def load_native():
     if not _SO.exists():
         raise NativeError(f"{_SO} is missing: run __graft_entry__.build() (nvcc, sm_100a). There is no CPU fallback.")
     lib = C.CDLL(str(_SO))
-    for name, (res, args) in {**EXPORTS, **SHARDED_EXPORTS}.items():
+    for name, (res, args) in {**EXPORTS, **SHARDED_EXPORTS, **MANY_LUT_EXPORTS}.items():
         try:
             fn = getattr(lib, name)
         except AttributeError as e:
@@ -283,6 +317,7 @@ class Engine:
         self._check(self.lib.tfhe_b200_ctx_create(device, C.byref(self.p), C.byref(h)))
         self.h = h
         self.device = device
+        self.many_stride = 0     # rows per ciphertext of the many-LUT entries (0: no many-LUT table uploaded)
 
     def _check(self, rc: int):
         if rc != 0:
@@ -331,6 +366,34 @@ class Engine:
         luts = np.ascontiguousarray(luts, dtype=np.uint64).reshape(-1, self.p.lut_len)
         self._check(self.lib.tfhe_b200_upload_luts(self.h, _ptr(luts), luts.shape[0]))
         self.n_luts = luts.shape[0]
+        self.many_stride = 0
+
+    def upload_many_luts(self, accs: np.ndarray, fn_count):
+        """many-LUT accumulators (many_lut_accumulator) and their function counts; replaces the uploaded lookup tables"""
+        accs = np.ascontiguousarray(accs, dtype=np.uint64).reshape(-1, self.p.lut_len)
+        fn = np.ascontiguousarray(np.broadcast_to(np.asarray(fn_count, dtype=np.uint32), (accs.shape[0],)))
+        self._check(self.lib.tfhe_b200_upload_many_luts(self.h, _ptr(accs), accs.shape[0], _ptr(fn)))
+        self.n_luts = accs.shape[0]
+        self.many_stride = int(fn.max())
+
+    def pbs_many_batch(self, small: np.ndarray, lut_idx=None, n_iters: int | None = None) -> np.ndarray:
+        """apply_many_lookup_table: (batch, S, k * N + 1), [i, f] = function f of ciphertext i (S = the largest function count)"""
+        small = np.ascontiguousarray(small, dtype=np.uint64).reshape(-1, self.p.small_len)
+        out = np.zeros((small.shape[0], max(self.many_stride, 1), self.p.big_len), dtype=np.uint64)
+        idx = None if lut_idx is None else np.ascontiguousarray(lut_idx, dtype=np.uint32)
+        if n_iters is None:
+            self._check(self.lib.tfhe_b200_pbs_many_batch(self.h, _ptr(small), _ptr(idx), _ptr(out), small.shape[0]))
+        else:
+            self._check(self.lib.tfhe_b200_pbs_many_batch_partial(self.h, _ptr(small), _ptr(idx), _ptr(out), small.shape[0], n_iters))
+        return out
+
+    def ks_pbs_many_batch(self, cts: np.ndarray, lut_idx=None) -> np.ndarray:
+        """keyswitch, then apply_many_lookup_table: (batch, S, k * N + 1)"""
+        cts = np.ascontiguousarray(cts, dtype=np.uint64).reshape(-1, self.p.big_len)
+        out = np.zeros((cts.shape[0], max(self.many_stride, 1), self.p.big_len), dtype=np.uint64)
+        idx = None if lut_idx is None else np.ascontiguousarray(lut_idx, dtype=np.uint32)
+        self._check(self.lib.tfhe_b200_ks_pbs_many_batch(self.h, _ptr(cts), _ptr(idx), _ptr(out), cts.shape[0]))
+        return out
 
     # host-buffer hot path -------------------------------------------------------------------------------
     def keyswitch_batch(self, cts: np.ndarray) -> np.ndarray:
@@ -382,6 +445,12 @@ class Engine:
 
     def pbs_batch_device(self, d_small, d_idx, d_out, batch: int, stream: int | None = None):
         self._check(self.lib.tfhe_b200_pbs_batch_device(self.h, _ptr(d_small), _ptr(d_idx), _ptr(d_out), batch, stream))
+
+    def pbs_many_batch_device(self, d_small, d_idx, d_out, batch: int, stream: int | None = None):
+        self._check(self.lib.tfhe_b200_pbs_many_batch_device(self.h, _ptr(d_small), _ptr(d_idx), _ptr(d_out), batch, stream))
+
+    def ks_pbs_many_batch_device(self, d_in, d_idx, d_out, batch: int, stream: int | None = None):
+        self._check(self.lib.tfhe_b200_ks_pbs_many_batch_device(self.h, _ptr(d_in), _ptr(d_idx), _ptr(d_out), batch, stream))
 
     def set_ciphertext_modulus_log2(self, log2_q: int):
         """non-native power-of-two ciphertext modulus 2^log2_q (64 = native): PBS outputs are rounded like bootstrap.rs:318-330"""

@@ -1,6 +1,7 @@
 // c_api.cu -- extern "C" boundary of libtfhe_b200.so (see include/tfhe_b200.h for the reference
 // interfaces each entry point replaces).  Plain pointers and sizes only; no torch types.
 #include "ctx.h"
+#include "../../include/tfhe_b200_many_lut.h"
 
 #include <atomic>
 #include <memory>
@@ -107,38 +108,39 @@ int do_keyswitch(tfhe_b200_ctx *c, const uint64_t *d_in, uint64_t *d_small, size
 }
 
 static int do_pbs_kernels(tfhe_b200_ctx *c, const uint64_t *d_small, const uint32_t *d_idx, const uint64_t *d_luts, uint64_t *d_out, size_t batch,
-                          uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot, bool fused);
+                          uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot, bool fused, tbk::ManyLut many);
 
 int do_pbs(tfhe_b200_ctx *c, const uint64_t *d_small, const uint32_t *d_idx, const uint64_t *d_luts, uint64_t *d_out, size_t batch,
-           uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot, bool fused) {
-    if (do_pbs_kernels(c, d_small, d_idx, d_luts, d_out, batch, n_iters, s, out_slot, fused)) return 1;
+           uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot, bool fused, tbk::ManyLut many) {
+    if (many.fn && !out_slot) return fail("internal: a many-LUT PBS needs output rows");
+    if (do_pbs_kernels(c, d_small, d_idx, d_luts, d_out, batch, n_iters, s, out_slot, fused, many)) return 1;
     if (c->log2_q < 64 && batch) {
-        TB_CUDA(tbk::launch_round_pow2(d_out, out_slot, (int)batch, (int)c->p.poly_size, (int)c->big_len(), c->log2_q, s));
+        TB_CUDA(tbk::launch_round_pow2(d_out, out_slot, d_idx, many, (int)batch, (int)c->p.poly_size, (int)c->big_len(), c->log2_q, s));
         c->launches += 1;
     }
     return 0;
 }
 
 static int do_pbs_kernels(tfhe_b200_ctx *c, const uint64_t *d_small, const uint32_t *d_idx, const uint64_t *d_luts, uint64_t *d_out, size_t batch,
-                          uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot, bool fused) {
+                          uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot, bool fused, tbk::ManyLut many) {
     if (fused && !fused_supported(c)) return fail("internal: fused PBS input requested on an unsupported configuration");
     if (!c->have_bsk) return fail("bootstrap key not uploaded");
     if (!d_luts) return fail("no lookup tables uploaded");
     if (c->tuned512 && batch >= (size_t)(c->tuned512_min ? c->tuned512_min : c->sms)) {
-        TB_CUDA(tbk::launch_pbs_n512(d_small, d_idx, d_luts, c->bskf8.p, c->tbl16.p, d_out, out_slot, (int)batch, (int)c->p.lwe_dim,
+        TB_CUDA(tbk::launch_pbs_n512(d_small, d_idx, d_luts, c->bskf8.p, c->tbl16.p, d_out, out_slot, many, (int)batch, (int)c->p.lwe_dim,
                                      (int)c->p.pbs_base_log, (int)(n_iters < c->p.lwe_dim ? n_iters : c->p.lwe_dim), s));
         c->launches += 1;
         return 0;
     }
     if (c->tuned8192) {
-        TB_CUDA(tbk::launch_pbs_n8192(d_small, d_idx, d_luts, c->bskf8.p, c->tbl16.p, d_out, out_slot, (int)batch, (int)c->p.lwe_dim,
+        TB_CUDA(tbk::launch_pbs_n8192(d_small, d_idx, d_luts, c->bskf8.p, c->tbl16.p, d_out, out_slot, many, (int)batch, (int)c->p.lwe_dim,
                                       (int)c->p.pbs_base_log, (int)(n_iters < c->p.lwe_dim ? n_iters : c->p.lwe_dim), (int)c->p.lwe_dim, s));
         c->launches += 1;
         return 0;
     }
     if (c->generic) {
         const uint32_t steps = c->p.grouping_factor ? c->p.lwe_dim / c->p.grouping_factor : c->p.lwe_dim;
-        TB_CUDA(tbk::launch_pbs_generic(d_small, d_idx, d_luts, c->bskf.p, c->tw_generic.p, d_out, out_slot, (int)batch, (int)c->p.lwe_dim,
+        TB_CUDA(tbk::launch_pbs_generic(d_small, d_idx, d_luts, c->bskf.p, c->tw_generic.p, d_out, out_slot, many, (int)batch, (int)c->p.lwe_dim,
                                         (int)c->p.poly_size, (int)c->p.glwe_dim, (int)c->p.pbs_base_log, (int)c->p.pbs_level,
                                         (int)c->p.grouping_factor, (int)(n_iters < steps ? n_iters : steps), s));
         c->launches += 1;
@@ -153,7 +155,7 @@ static int do_pbs_kernels(tfhe_b200_ctx *c, const uint64_t *d_small, const uint3
         const size_t tail = batch <= (size_t)2 * c->sms ? batch : (rem != 0 && rem <= (size_t)2 * c->sms) ? rem : 0, wide = batch - tail;
         const int steps = (int)(n_iters < groups ? n_iters : groups);
         if (wide) {
-            TB_CUDA(tbk::launch_pbs_multibit_v4(d_small, d_idx, d_luts, c->bskf.p, c->tbl16.p, c->roots.p, d_out, out_slot, (int)wide,
+            TB_CUDA(tbk::launch_pbs_multibit_v4(d_small, d_idx, d_luts, c->bskf.p, c->tbl16.p, c->roots.p, d_out, out_slot, many, (int)wide,
                                                 (int)c->p.lwe_dim, (int)c->p.pbs_base_log, steps, s));
             c->launches += 1;
         }
@@ -162,11 +164,11 @@ static int do_pbs_kernels(tfhe_b200_ctx *c, const uint64_t *d_small, const uint3
             uint64_t *t_out = out_slot ? d_out : d_out + wide * ((size_t)c->p.glwe_dim * c->p.poly_size + 1);
             if (c->narrow_kernel == 8 && tail <= (size_t)(c->narrow_max ? c->narrow_max : c->sms))
                 TB_CUDA(tbk::launch_pbs_multibit_v8(t_small, d_idx ? d_idx + wide : nullptr, d_luts, c->bskf8.p, c->tbl8.p, c->roots.p, t_out,
-                                                    out_slot ? out_slot + wide : nullptr, (int)tail, (int)c->p.lwe_dim,
+                                                    out_slot ? out_slot + wide : nullptr, many, (int)tail, (int)c->p.lwe_dim,
                                                     (int)c->p.pbs_base_log, steps, c->narrow_cluster ? c->sms / 2 : 0, s));
             else
                 TB_CUDA(tbk::launch_pbs_multibit_v4(t_small, d_idx ? d_idx + wide : nullptr, d_luts, c->bskf.p, c->tbl16.p, c->roots.p, t_out,
-                                                    out_slot ? out_slot + wide : nullptr, (int)tail, (int)c->p.lwe_dim,
+                                                    out_slot ? out_slot + wide : nullptr, many, (int)tail, (int)c->p.lwe_dim,
                                                     (int)c->p.pbs_base_log, steps, s));
             c->launches += 1;
         }
@@ -183,7 +185,7 @@ static int do_pbs_kernels(tfhe_b200_ctx *c, const uint64_t *d_small, const uint3
         auto wide_launch = [&](size_t count, int cts) -> int {
             const uint64_t *w_small = reinterpret_cast<const uint64_t *>(reinterpret_cast<const char *>(d_small) + done * in_stride);
             TB_CUDA(tbk::launch_pbs_classic_v4(w_small, d_idx ? d_idx + done : nullptr, d_luts, c->bskf.p, c->tbl16.p,
-                                               out_slot ? d_out : d_out + done * out_stride, out_slot ? out_slot + done : nullptr, (int)count,
+                                               out_slot ? d_out : d_out + done * out_stride, out_slot ? out_slot + done : nullptr, many, (int)count,
                                                (int)c->p.lwe_dim, (int)c->p.pbs_base_log, (int)n_iters, fused ? 1 : 0, cts, s));
             c->launches += 1;
             done += count;
@@ -194,7 +196,7 @@ static int do_pbs_kernels(tfhe_b200_ctx *c, const uint64_t *d_small, const uint3
         if (plan.tail) {
             const uint64_t *t_small = reinterpret_cast<const uint64_t *>(reinterpret_cast<const char *>(d_small) + done * in_stride);
             TB_CUDA(tbk::launch_pbs_classic_v8(t_small, d_idx ? d_idx + done : nullptr, d_luts, c->bskf8.p, c->tbl8.p,
-                                               out_slot ? d_out : d_out + done * out_stride, out_slot ? out_slot + done : nullptr, (int)plan.tail,
+                                               out_slot ? d_out : d_out + done * out_stride, out_slot ? out_slot + done : nullptr, many, (int)plan.tail,
                                                (int)c->p.lwe_dim, (int)c->p.pbs_base_log, (int)n_iters, fused ? 1 : 0,
                                                c->narrow_cluster ? c->sms / 2 : 0, s));
             c->launches += 1;
@@ -207,8 +209,15 @@ static int do_pbs_kernels(tfhe_b200_ctx *c, const uint64_t *d_small, const uint3
 
 using tbc::do_keyswitch;
 
+// the single-function entry points write one row per ciphertext: they cannot take a many-LUT table
+static int refuse_many(const tfhe_b200_ctx *c) {
+    return c->many_stride ? fail("a many-LUT table is uploaded (tfhe_b200_upload_many_luts): use the *_many_batch entry points, or upload "
+                                 "single-function tables with tfhe_b200_upload_luts") : 0;
+}
+
 static int do_pbs(tfhe_b200_ctx *c, const uint64_t *d_small, const uint32_t *d_idx, uint64_t *d_out, size_t batch, uint32_t n_iters,
                   cudaStream_t s) {
+    if (refuse_many(c)) return 1;
     return tbc::do_pbs(c, d_small, d_idx, c->n_luts ? (const uint64_t *)c->luts.p : nullptr, d_out, batch, n_iters, s, nullptr);
 }
 
@@ -339,7 +348,7 @@ int tfhe_b200_ctx_destroy(tfhe_b200_ctx *c) {
     if (!c) return 0;
     DeviceGuard g(c->device);
     cudaStreamSynchronize(c->stream);
-    for (DevBuf *b : {&c->ksk_packed, &c->ksk_colsum, &c->ksk_planes, &c->ks_digits, &c->bskf, &c->bskf8, &c->tbl16, &c->tbl8, &c->tw_generic, &c->roots, &c->luts, &c->d_in, &c->d_small, &c->d_out, &c->d_idx})
+    for (DevBuf *b : {&c->ksk_packed, &c->ksk_colsum, &c->ksk_planes, &c->ks_digits, &c->bskf, &c->bskf8, &c->tbl16, &c->tbl8, &c->tw_generic, &c->roots, &c->luts, &c->lut_fn, &c->d_in, &c->d_small, &c->d_out, &c->d_idx})
         b->release();
     for (auto &e : c->ev) if (e) cudaEventDestroy(e);
     for (auto &L : c->lane) {
@@ -580,6 +589,32 @@ int tfhe_b200_upload_luts(tfhe_b200_ctx *c, const uint64_t *luts, uint32_t n_lut
     TB_CUDA(cudaMemcpyAsync(c->luts.p, luts, bytes, cudaMemcpyHostToDevice, c->stream));
     TB_CUDA(cudaStreamSynchronize(c->stream));
     c->n_luts = n_luts;
+    c->many_stride = 0;
+    return 0;
+}
+
+int tfhe_b200_upload_many_luts(tfhe_b200_ctx *c, const uint64_t *accs, uint32_t n_luts, const uint32_t *fn_count) {
+    if (!c || !accs || !fn_count || n_luts == 0) return fail("null or empty many-LUT table");
+    const uint32_t total = c->p.msg_mod * c->p.carry_mod;
+    if (total < 2 || total > c->p.poly_size) return fail("many-LUT PBS needs 2 <= msg_mod * carry_mod <= poly_size");
+    uint32_t stride = 0;
+    for (uint32_t i = 0; i < n_luts; ++i) {
+        if (fn_count[i] < 2 || fn_count[i] > total)
+            return fail("fn_count[" + std::to_string(i) + "] = " + std::to_string(fn_count[i]) + ": a many-LUT accumulator holds 2 ... msg_mod * carry_mod = " +
+                        std::to_string(total) + " functions");
+        stride = std::max(stride, fn_count[i]);
+    }
+    std::lock_guard<std::mutex> lk(c->mu);
+    DeviceGuard g(c->device);
+    const size_t bytes = (size_t)n_luts * c->lut_len() * 8;
+    TB_CUDA(cudaStreamSynchronize(c->stream));
+    TB_CUDA(c->luts.reserve(bytes));
+    TB_CUDA(c->lut_fn.reserve((size_t)n_luts * 4));
+    TB_CUDA(cudaMemcpyAsync(c->luts.p, accs, bytes, cudaMemcpyHostToDevice, c->stream));
+    TB_CUDA(cudaMemcpyAsync(c->lut_fn.p, fn_count, (size_t)n_luts * 4, cudaMemcpyHostToDevice, c->stream));
+    TB_CUDA(cudaStreamSynchronize(c->stream));
+    c->n_luts = n_luts;
+    c->many_stride = stride;
     return 0;
 }
 
@@ -614,6 +649,7 @@ int tfhe_b200_ks_pbs_batch_device(tfhe_b200_ctx *c, const uint64_t *d_in, const 
     std::lock_guard<std::mutex> lk(c->mu);
     DeviceGuard g(c->device);
     cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
+    if (refuse_many(c)) return 1;
     TB_CUDA(c->d_small.reserve_on(batch * c->small_len() * 8, s));
     TB_CUDA(cudaEventRecord(c->ev[0], s));
     const bool fused = tbc::fused_supported(c);
@@ -690,7 +726,7 @@ int tfhe_b200_ks_pbs_batch(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t 
     if (!c->have_bsk) return fail("bootstrap key not uploaded");
     if (c->n_luts == 0) return fail("no lookup tables uploaded");
     std::lock_guard<std::mutex> lk(c->mu);
-    if (check_lut_indices(c, idx, batch)) return 1;
+    if (refuse_many(c) || check_lut_indices(c, idx, batch)) return 1;
     DeviceGuard g(c->device);
     // chunks of whole waves (classic: 4 ciphertexts per SM x 4 waves; multi-bit: 3 per SM x 5 waves), alternating between two lanes
     // (stream + staging buffers)
@@ -729,7 +765,7 @@ int tfhe_b200_pbs_ks_batch(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t 
     if (batch == 0) return 0;
     if (c->n_luts == 0) return fail("no lookup tables uploaded");
     std::lock_guard<std::mutex> lk(c->mu);
-    if (check_lut_indices(c, idx, batch)) return 1;
+    if (refuse_many(c) || check_lut_indices(c, idx, batch)) return 1;
     DeviceGuard g(c->device);
     cudaStream_t s = c->stream;
     TB_CUDA(c->d_small.reserve(batch * c->small_len() * 8));
@@ -749,6 +785,110 @@ int tfhe_b200_pbs_ks_batch(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t 
     TB_CUDA(cudaMemcpyAsync(out, c->d_in.p, batch * c->small_len() * 8, cudaMemcpyDeviceToHost, s));
     TB_CUDA(cudaStreamSynchronize(s));
     return 0;
+}
+
+// ---- many-LUT entry points: ciphertext i owns rows [i * S, (i + 1) * S) of the output, S = the largest function count of the uploaded
+// table; function f of its table lands in row i * S + f ----------------------------------------------------------------------------
+
+static int need_many(const tfhe_b200_ctx *c) {
+    return c->many_stride ? 0 : fail("no many-LUT table uploaded (tfhe_b200_upload_many_luts)");
+}
+
+static tbk::ManyLut ctx_many(const tfhe_b200_ctx *c) {
+    tbk::ManyLut m;
+    m.fn = (const uint32_t *)c->lut_fn.p;
+    m.total = (int)(c->p.msg_mod * c->p.carry_mod);
+    return m;
+}
+
+static int many_pbs(tfhe_b200_ctx *c, const uint64_t *d_in, const uint32_t *d_idx, uint64_t *d_out, size_t batch, uint32_t n_iters,
+                    cudaStream_t s, bool ks, const uint32_t *rows);
+
+// ks: the input rows are big-key ciphertexts, keyswitched first (fused modulus switch where the context supports it)
+static int many_batch(tfhe_b200_ctx *c, const uint64_t *d_in, const uint32_t *d_idx, uint64_t *d_out, size_t batch, uint32_t n_iters,
+                      cudaStream_t s, bool ks) {
+    if ((uint64_t)batch * c->many_stride > 0xFFFFFFFFull) return fail("many-LUT batch too large: batch * rows per ciphertext must fit 32 bits");
+    // row map i -> i * S, allocated and freed in the order of stream s: it lives exactly as long as the launches that read it
+    uint32_t *rows = nullptr;
+    TB_CUDA(cudaMallocAsync((void **)&rows, batch * 4, s));
+    const cudaError_t fill = tbk::launch_iota_rows(rows, batch, c->many_stride, s);
+    if (fill != cudaSuccess) { cudaFreeAsync(rows, s); return fail(std::string("launch_iota_rows: ") + cudaGetErrorString(fill)); }
+    const int rc = many_pbs(c, d_in, d_idx, d_out, batch, n_iters, s, ks, rows);
+    TB_CUDA(cudaFreeAsync(rows, s));
+    return rc;
+}
+
+static int many_pbs(tfhe_b200_ctx *c, const uint64_t *d_in, const uint32_t *d_idx, uint64_t *d_out, size_t batch, uint32_t n_iters,
+                    cudaStream_t s, bool ks, const uint32_t *rows) {
+    const uint64_t *d_small = d_in;
+    const bool fused = ks && tbc::fused_supported(c);
+    if (ks) {
+        TB_CUDA(c->d_small.reserve_on(batch * c->small_len() * 8, s));
+        if (tbc::do_keyswitch(c, d_in, (uint64_t *)c->d_small.p, batch, s, nullptr, nullptr, fused)) return 1;
+        d_small = (const uint64_t *)c->d_small.p;
+    }
+    return tbc::do_pbs(c, d_small, d_idx, (const uint64_t *)c->luts.p, d_out, batch, n_iters, s, rows, fused, ctx_many(c));
+}
+
+static int many_host(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t *idx, uint64_t *out, size_t batch, uint32_t n_iters, bool ks) {
+    if (!c || (batch && (!in || !out))) return fail("null argument");
+    if (batch == 0) return 0;
+    if (n_iters > c->p.lwe_dim) return fail("n_iters exceeds lwe_dim");
+    if (ks && !c->have_ksk) return fail("keyswitch key not uploaded");
+    std::lock_guard<std::mutex> lk(c->mu);
+    if (need_many(c) || check_lut_indices(c, idx, batch)) return 1;
+    DeviceGuard g(c->device);
+    const size_t in_len = ks ? c->big_len() : c->small_len(), out_words = batch * c->many_stride * c->big_len();
+    TB_CUDA(c->d_in.reserve(batch * in_len * 8));
+    TB_CUDA(c->d_out.reserve(out_words * 8));
+    TB_CUDA(cudaMemcpyAsync(c->d_in.p, in, batch * in_len * 8, cudaMemcpyHostToDevice, c->stream));
+    const uint32_t *d_idx = nullptr;
+    if (idx) {
+        TB_CUDA(c->d_idx.reserve(batch * 4));
+        TB_CUDA(cudaMemcpyAsync(c->d_idx.p, idx, batch * 4, cudaMemcpyHostToDevice, c->stream));
+        d_idx = (const uint32_t *)c->d_idx.p;
+    }
+    // rows past a table's function count are not written by the kernels: the caller receives them as zeros
+    TB_CUDA(cudaMemsetAsync(c->d_out.p, 0, out_words * 8, c->stream));
+    if (many_batch(c, (const uint64_t *)c->d_in.p, d_idx, (uint64_t *)c->d_out.p, batch, n_iters, c->stream, ks)) return 1;
+    TB_CUDA(cudaMemcpyAsync(out, c->d_out.p, out_words * 8, cudaMemcpyDeviceToHost, c->stream));
+    TB_CUDA(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int tfhe_b200_pbs_many_batch(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t *idx, uint64_t *out, size_t batch) {
+    if (!c) return fail("null context");
+    return many_host(c, in, idx, out, batch, c->p.lwe_dim, false);
+}
+
+int tfhe_b200_pbs_many_batch_partial(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t *idx, uint64_t *out, size_t batch,
+                                     uint32_t n_iters) {
+    return many_host(c, in, idx, out, batch, n_iters, false);
+}
+
+int tfhe_b200_ks_pbs_many_batch(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t *idx, uint64_t *out, size_t batch) {
+    if (!c) return fail("null context");
+    return many_host(c, in, idx, out, batch, c->p.lwe_dim, true);
+}
+
+static int many_device(tfhe_b200_ctx *c, const uint64_t *d_in, const uint32_t *d_idx, uint64_t *d_out, size_t batch, void *stream, bool ks) {
+    if (!c || (batch && (!d_in || !d_out))) return fail("null argument");
+    if (batch == 0) return 0;
+    if (ks && !c->have_ksk) return fail("keyswitch key not uploaded");
+    std::lock_guard<std::mutex> lk(c->mu);
+    if (need_many(c)) return 1;
+    DeviceGuard g(c->device);
+    return many_batch(c, d_in, d_idx, d_out, batch, c->p.lwe_dim, stream ? (cudaStream_t)stream : c->stream, ks);
+}
+
+int tfhe_b200_pbs_many_batch_device(tfhe_b200_ctx *c, const uint64_t *d_small, const uint32_t *d_idx, uint64_t *d_out, size_t batch,
+                                    void *stream) {
+    return many_device(c, d_small, d_idx, d_out, batch, stream, false);
+}
+
+int tfhe_b200_ks_pbs_many_batch_device(tfhe_b200_ctx *c, const uint64_t *d_in, const uint32_t *d_idx, uint64_t *d_out, size_t batch,
+                                       void *stream) {
+    return many_device(c, d_in, d_idx, d_out, batch, stream, true);
 }
 
 // ---- instrumentation --------------------------------------------------------------------------------

@@ -71,6 +71,10 @@ struct tfhe_b200_ctx {
     tbc::DevBuf ksk_packed, ksk_colsum, ksk_planes, ks_digits, bskf, bskf8, tbl16, tbl8, tw_generic, roots, luts;
     int ks_kernel = 2;    // 2: tcgen05 GEMM (keyswitch_tc.cu), 1: mma.sync GEMM (keyswitch_mma.cu), 0: IMAD GEMM (keyswitch.cu); env TFHE_B200_KS_KERNEL=tc|mma|imad
     uint32_t n_luts = 0;
+    // many-LUT table (tfhe_b200_upload_many_luts): lut_fn = the function count of every uploaded table, many_stride = the largest (rows
+    // per ciphertext of the many-LUT batch entries); 0 while the uploaded tables are single-function ones
+    tbc::DevBuf lut_fn;
+    uint32_t many_stride = 0;
     bool have_ksk = false, have_bsk = false;
     int narrow_kernel = 8;   // classic PBS, levels of <= 2 * SM count ciphertexts: 8 = pbs_v8.cu (8 FFT points per thread, 8 warps per ciphertext; keeps a second copy of the Fourier key in its own layout), 0 = the 1- / 2-ciphertext instances of pbs_v4.cu; env TFHE_B200_NARROW_KERNEL
     bool generic = false;    // parameter sets outside N = 2048, k = 1, l = 1 (or TFHE_B200_PBS_KERNEL=generic): pbs_generic.cu, no fused modulus switch
@@ -103,7 +107,7 @@ bool fused_supported(const tfhe_b200_ctx *c);
 int do_keyswitch(tfhe_b200_ctx *c, const uint64_t *d_in, uint64_t *d_small, size_t batch, cudaStream_t s,
                  const uint32_t *in_slot = nullptr, DevBuf *digits = nullptr, bool fused = false);
 int do_pbs(tfhe_b200_ctx *c, const uint64_t *d_small, const uint32_t *d_idx, const uint64_t *d_luts, uint64_t *d_out, size_t batch,
-           uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot = nullptr, bool fused = false);
+           uint32_t n_iters, cudaStream_t s, const uint32_t *out_slot = nullptr, bool fused = false, tbk::ManyLut many = {});
 
 // rank r's PBS jobs [lo, hi) of a split level of w jobs: contiguous and balanced, the first w % world ranks take one more
 // (multi_gpu.shard_range; the scatter kernel inverts it on the device)

@@ -48,25 +48,45 @@ namespace tblin {
 // SignedDecomposer(log2_q, 1).closest_representable BEFORE the sample extraction.  Applied to the extracted sample instead: the words
 // that sample extraction negated (glwe_sample_extraction.rs:91-147: every mask word except the first of each polynomial) are rounded as
 // -round(-x), the others as round(x), which is the same value bit for bit, ties included.
-__global__ void __launch_bounds__(256) round_pow2_kernel(uint64_t *__restrict__ out, const uint32_t *__restrict__ out_slot, int poly_size,
+// A many-LUT row of function f (kernels.h ManyLut) was extracted at monomial t_f: there the negated words are the mask words past t_f of
+// each polynomial.
+__global__ void __launch_bounds__(256) round_pow2_kernel(uint64_t *__restrict__ out, const uint32_t *__restrict__ out_slot,
+                                                         const uint32_t *__restrict__ lut_idx, const tbk::ManyLut many, int poly_size,
                                                          int lwe_len, int log2_q) {
-    uint64_t *row = out + (size_t)(out_slot ? out_slot[blockIdx.x] : blockIdx.x) * lwe_len;
+    const int nf = many.fn ? (int)many.fn[lut_idx ? lut_idx[blockIdx.x] : 0] : 1;
+    const int step = many.fn ? (many.total / nf) * (poly_size / many.total) : 0;
     const int shift = 64 - log2_q - 1;
-    for (int j = threadIdx.x; j < lwe_len; j += blockDim.x) {
-        const bool negated = j != lwe_len - 1 && (j % poly_size) != 0;
-        uint64_t x = row[j];
-        if (negated) x = (uint64_t)0 - x;
-        x = (((x >> shift) + 1) & ~(uint64_t)1) << shift;
-        row[j] = negated ? (uint64_t)0 - x : x;
+    for (int f = 0; f < nf; ++f) {
+        uint64_t *row = out + ((size_t)(out_slot ? out_slot[blockIdx.x] : blockIdx.x) + f) * lwe_len;
+        const int t = f * step;
+        for (int j = threadIdx.x; j < lwe_len; j += blockDim.x) {
+            const bool negated = j != lwe_len - 1 && (j % poly_size) > t;
+            uint64_t x = row[j];
+            if (negated) x = (uint64_t)0 - x;
+            x = (((x >> shift) + 1) & ~(uint64_t)1) << shift;
+            row[j] = negated ? (uint64_t)0 - x : x;
+        }
     }
+}
+
+__global__ void __launch_bounds__(256) iota_rows_kernel(uint32_t *__restrict__ rows, size_t n, uint32_t stride) {
+    const size_t i = (size_t)blockIdx.x * 256 + threadIdx.x;
+    if (i < n) rows[i] = (uint32_t)(i * stride);
 }
 }  // namespace tblin
 
 namespace tbk {
 
-cudaError_t launch_round_pow2(uint64_t *out, const uint32_t *out_slot, int batch, int poly_size, int lwe_len, int log2_q, cudaStream_t stream) {
+cudaError_t launch_round_pow2(uint64_t *out, const uint32_t *out_slot, const uint32_t *lut_idx, ManyLut many, int batch, int poly_size,
+                              int lwe_len, int log2_q, cudaStream_t stream) {
     if (batch <= 0 || log2_q >= 64) return cudaSuccess;
-    tblin::round_pow2_kernel<<<batch, 256, 0, stream>>>(out, out_slot, poly_size, lwe_len, log2_q);
+    tblin::round_pow2_kernel<<<batch, 256, 0, stream>>>(out, out_slot, lut_idx, many, poly_size, lwe_len, log2_q);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_iota_rows(uint32_t *rows, size_t n, uint32_t stride, cudaStream_t stream) {
+    if (n == 0) return cudaSuccess;
+    tblin::iota_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(rows, n, stride);
     return cudaGetLastError();
 }
 

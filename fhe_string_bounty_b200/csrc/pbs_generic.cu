@@ -20,6 +20,7 @@
 // This is the coverage kernel, not the tuned one: N = 2048, k = 1, one level stays on pbs_v4.cu / pbs_v8.cu (TFHE_B200_PBS_KERNEL=generic
 // forces this one for cross-checks).  Measured 2.4 ... 6.1 TFLOP/s algorithmic against 15.8 for the tuned kernels (DESIGN.md K12).
 #include "kernels.h"
+#include "sample_extract.cuh"
 #include <type_traits>
 #include "fft_core.cuh"
 #include "pbs16_common.cuh"      // Tensor Memory helpers (tcgen05.alloc / ld / st)
@@ -468,7 +469,7 @@ template <int LOGN, int K1, int GF>
 __global__ void __launch_bounds__(Shape<LOGN, K1>::T, Shape<LOGN, K1>::MINB)
 pbs_generic_kernel(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                    const cplx *__restrict__ bskf, const cplx *__restrict__ tw, uint64_t *__restrict__ out,
-                   const uint32_t *__restrict__ out_slot, int n, int base_log, int levels, int n_iters) {
+                   const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int n, int base_log, int levels, int n_iters) {
     using S = Shape<LOGN, K1>;
     constexpr int N = S::N, M = S::M, PER = S::PER, T = S::T;
     using F = typename std::conditional<S::R8, Fft8<M, T>, Fft4<M, T>>::type;
@@ -637,10 +638,15 @@ pbs_generic_kernel(const uint64_t *__restrict__ lwe_small, const uint32_t *__res
     }
 
     // sample extraction of coefficient 0 (glwe_sample_extraction.rs:91-147)
-    uint64_t *dst = out + (size_t)(out_slot ? out_slot[ct] : ct) * ((size_t)(K1 - 1) * N + 1);
-    for (int r = 0; r < K1 - 1; ++r)
-        for (int j = t; j < N; j += T) dst[r * N + j] = j == 0 ? acc[r * N] : (uint64_t)0 - acc[r * N + N - j];
-    if (t == 0) dst[(K1 - 1) * N] = acc[(K1 - 1) * N];
+    if (many.fn) {
+        const int nf = tbx::many_fn_count(many, lut_idx, ct);
+        tbx::extract_many_acc(out, out_slot[ct], nf, tbx::many_step(many, nf, N), acc, N, K1 - 1, t, T);
+    } else {
+        uint64_t *dst = out + (size_t)(out_slot ? out_slot[ct] : ct) * ((size_t)(K1 - 1) * N + 1);
+        for (int r = 0; r < K1 - 1; ++r)
+            for (int j = t; j < N; j += T) dst[r * N + j] = j == 0 ? acc[r * N] : (uint64_t)0 - acc[r * N + N - j];
+        if (t == 0) dst[(K1 - 1) * N] = acc[(K1 - 1) * N];
+    }
     if (TM) {
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
         __syncthreads();
@@ -675,7 +681,7 @@ bsk_convert_generic_kernel(const uint64_t *__restrict__ bsk_std, cplx *__restric
 
 template <int LOGN, int K1, int GF>
 cudaError_t launch(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskf, const void *tw,
-                   uint64_t *out, const uint32_t *out_slot, int batch, int n, int base_log, int levels, int n_iters, cudaStream_t stream) {
+                   uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n, int base_log, int levels, int n_iters, cudaStream_t stream) {
     using S = Shape<LOGN, K1>;
     using F = typename std::conditional<S::R8, Fft8<S::M, S::T>, Fft4<S::M, S::T>>::type;
     const size_t smem = (size_t)K1 * S::N * 8 + (size_t)S::M * 16 + (size_t)F::ENTRIES * 16 + 16;   // + the Tensor Memory base address slot
@@ -685,7 +691,7 @@ cudaError_t launch(const uint64_t *lwe_small, const uint32_t *lut_idx, const uin
     e = cudaFuncSetAttribute(pbs_generic_kernel<LOGN, K1, GF>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return e;
     pbs_generic_kernel<LOGN, K1, GF><<<batch, S::T, smem, stream>>>(lwe_small, lut_idx, luts, reinterpret_cast<const cplx *>(bskf),
-                                                                 reinterpret_cast<const cplx *>(tw), out, out_slot, n, base_log, levels, n_iters);
+                                                                 reinterpret_cast<const cplx *>(tw), out, out_slot, many, n, base_log, levels, n_iters);
     return cudaGetLastError();
 }
 
@@ -762,7 +768,7 @@ template <int LOGN, int K1>
 __global__ void __launch_bounds__(BIG_T, 2)
 pbs_generic_big_kernel(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                        const cplx *__restrict__ bskf, const cplx *__restrict__ tw, uint64_t *__restrict__ out,
-                       const uint32_t *__restrict__ out_slot, unsigned char *scratch, int batch, int n, int base_log, int levels,
+                       const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, unsigned char *scratch, int batch, int n, int base_log, int levels,
                        int n_iters) {
     constexpr int N = 1 << LOGN, M = N / 2, T = BIG_T;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -833,10 +839,15 @@ pbs_generic_big_kernel(const uint64_t *__restrict__ lwe_small, const uint32_t *_
             }
             __syncthreads();
         }
-        uint64_t *dst = out + (size_t)(out_slot ? out_slot[ct] : ct) * ((size_t)(K1 - 1) * N + 1);
-        for (int r = 0; r < K1 - 1; ++r)
-            for (int j = t; j < N; j += T) dst[r * N + j] = j == 0 ? acc[r * N] : (uint64_t)0 - acc[r * N + N - j];
-        if (t == 0) dst[(K1 - 1) * N] = acc[(K1 - 1) * N];
+        if (many.fn) {
+            const int nf = tbx::many_fn_count(many, lut_idx, ct);
+            tbx::extract_many_acc(out, out_slot[ct], nf, tbx::many_step(many, nf, N), acc, N, K1 - 1, t, T);
+        } else {
+            uint64_t *dst = out + (size_t)(out_slot ? out_slot[ct] : ct) * ((size_t)(K1 - 1) * N + 1);
+            for (int r = 0; r < K1 - 1; ++r)
+                for (int j = t; j < N; j += T) dst[r * N + j] = j == 0 ? acc[r * N] : (uint64_t)0 - acc[r * N + N - j];
+            if (t == 0) dst[(K1 - 1) * N] = acc[(K1 - 1) * N];
+        }
         __syncthreads();      // the next ciphertext overwrites the accumulator
     }
 }
@@ -863,7 +874,7 @@ bsk_convert_generic_big_kernel(const uint64_t *__restrict__ bsk_std, cplx *bskf,
 
 template <int LOGN, int K1>
 cudaError_t launch_big(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskf, const void *tw,
-                       uint64_t *out, const uint32_t *out_slot, int batch, int n, int base_log, int levels, int n_iters, cudaStream_t stream) {
+                       uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n, int base_log, int levels, int n_iters, cudaStream_t stream) {
     const size_t smem = (size_t)BIG_CH * 16 + (size_t)BigFft::ENTRIES * 16;
     cudaError_t e = cudaFuncSetAttribute(pbs_generic_big_kernel<LOGN, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
@@ -874,7 +885,7 @@ cudaError_t launch_big(const uint64_t *lwe_small, const uint32_t *lut_idx, const
     unsigned char *scratch = nullptr;     // stream-ordered: concurrent launches on other streams get their own area
     if ((e = cudaMallocAsync((void **)&scratch, (size_t)grid * big_scratch_bytes<LOGN, K1>(), stream)) != cudaSuccess) return e;
     pbs_generic_big_kernel<LOGN, K1><<<grid, BIG_T, smem, stream>>>(lwe_small, lut_idx, luts, reinterpret_cast<const cplx *>(bskf),
-                                                                    reinterpret_cast<const cplx *>(tw), out, out_slot, scratch, batch, n,
+                                                                    reinterpret_cast<const cplx *>(tw), out, out_slot, many, scratch, batch, n,
                                                                     base_log, levels, n_iters);
     e = cudaGetLastError();
     const cudaError_t e2 = cudaFreeAsync(scratch, stream);
@@ -906,26 +917,26 @@ bool pbs_generic_supported(int poly_size, int glwe_dim) {
 }
 
 cudaError_t launch_pbs_generic(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskf, const void *tw,
-                               uint64_t *out, const uint32_t *out_slot, int batch, int n, int poly_size, int glwe_dim, int base_log,
+                               uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n, int poly_size, int glwe_dim, int base_log,
                                int levels, int grouping_factor, int n_iters, cudaStream_t stream) {
     if (batch <= 0) return cudaSuccess;
 #define X(LOGN, K)                                                                                                                   \
     if (poly_size == (1 << LOGN) && glwe_dim == K) {                                                                                 \
         if (grouping_factor == 0)                                                                                                    \
-            return tbg::launch<LOGN, K + 1, 0>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, batch, n, base_log, levels, n_iters, stream); \
+            return tbg::launch<LOGN, K + 1, 0>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, many, batch, n, base_log, levels, n_iters, stream); \
         if (grouping_factor == 2)                                                                                                    \
-            return tbg::launch<LOGN, K + 1, 2>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, batch, n, base_log, levels, n_iters, stream); \
+            return tbg::launch<LOGN, K + 1, 2>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, many, batch, n, base_log, levels, n_iters, stream); \
         if (grouping_factor == 3)                                                                                                    \
-            return tbg::launch<LOGN, K + 1, 3>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, batch, n, base_log, levels, n_iters, stream); \
+            return tbg::launch<LOGN, K + 1, 3>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, many, batch, n, base_log, levels, n_iters, stream); \
         return cudaErrorInvalidValue;                                                                                                \
     }
     TBG_SHAPES(X)
 #undef X
     if (grouping_factor != 0) return cudaErrorInvalidValue;
     if (glwe_dim == 1 && poly_size == 16384)
-        return tbg::launch_big<14, 2>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, batch, n, base_log, levels, n_iters, stream);
+        return tbg::launch_big<14, 2>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, many, batch, n, base_log, levels, n_iters, stream);
     if (glwe_dim == 1 && poly_size == 32768)
-        return tbg::launch_big<15, 2>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, batch, n, base_log, levels, n_iters, stream);
+        return tbg::launch_big<15, 2>(lwe_small, lut_idx, luts, bskf, tw, out, out_slot, many, batch, n, base_log, levels, n_iters, stream);
     return cudaErrorInvalidValue;
 }
 

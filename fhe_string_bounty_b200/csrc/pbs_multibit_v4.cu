@@ -14,6 +14,7 @@
 // Key stream: 512 KiB per step through a ring of five 16 KiB pieces ([j & 1][out poly][sel][q 2][thread 64], two GGSWs of one
 // 2-frequency chunk each), fed by bulk asynchronous copies; shared memory = 8 x 17 KiB tiles + 80 KiB ring.
 #include "kernels.h"
+#include "sample_extract.cuh"
 #include "pbs16_common.cuh"
 #include <cstdlib>
 
@@ -52,7 +53,7 @@ template <int CTS>
 __global__ void __launch_bounds__(128 * CTS, 1)
 pbs_multibit_kernel_v4(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                        const cplx *__restrict__ bskm, const cplx *__restrict__ tbl16, const cplx *__restrict__ roots,   // roots[e] = exp(i*pi*e/2048)
-                       uint64_t *__restrict__ out, const uint32_t *__restrict__ out_slot, int batch, int n, int base_log, int n_groups) {
+                       uint64_t *__restrict__ out, const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int batch, int n, int base_log, int n_groups) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int WARPS = 4 * CTS, TMEM_COLS = 256, NSLOT = Smem<CTS>::NSLOT;   // twiddles in columns 0..79 (shared by the ciphertexts: same thread index, same values)
     Smem<CTS> &sm = *reinterpret_cast<Smem<CTS> *>(smem_raw);
@@ -272,7 +273,10 @@ pbs_multibit_kernel_v4(const uint64_t *__restrict__ lwe_small, const uint32_t *_
         }
     }
 
-    if (live) {
+    if (live && many.fn) {
+        const int nf = tbx::many_fn_count(many, lut_idx, ct);
+        tbx::extract_many_regs<16, 64, kN, 1>(out, out_slot[ct], nf, tbx::many_step(many, nf, kN), w, T, re, im);
+    } else if (live) {
         uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (kN + 1);
         if (w == 0) {
 #pragma unroll
@@ -340,7 +344,7 @@ cudaError_t pbs_multibit_v4_configure() {
 }
 
 cudaError_t launch_pbs_multibit_v4(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskm,
-                                   const void *tbl16, const void *roots, uint64_t *out, const uint32_t *out_slot, int batch, int n,
+                                   const void *tbl16, const void *roots, uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n,
                                    int base_log, int n_groups, cudaStream_t stream) {
     if (batch <= 0) return cudaSuccess;
     int sms = 148, dev = 0;
@@ -355,17 +359,17 @@ cudaError_t launch_pbs_multibit_v4(const uint64_t *lwe_small, const uint32_t *lu
     const int force = fe ? atoi(fe) : 0;
     const int cts = force ? force : batch <= sms ? 1 : batch <= 2 * sms ? 2 : 3;
     if (cts == 1)
-        tbm4::pbs_multibit_kernel_v4<1><<<batch, 128, sizeof(tbm4::Smem<1>), stream>>>(lwe_small, lut_idx, luts, bk, tb, rt, out, out_slot, batch,
+        tbm4::pbs_multibit_kernel_v4<1><<<batch, 128, sizeof(tbm4::Smem<1>), stream>>>(lwe_small, lut_idx, luts, bk, tb, rt, out, out_slot, many, batch,
                                                                                     n, base_log, n_groups);
     else if (cts == 2)
         tbm4::pbs_multibit_kernel_v4<2><<<(batch + 1) / 2, 256, sizeof(tbm4::Smem<2>), stream>>>(lwe_small, lut_idx, luts, bk, tb, rt, out,
-                                                                                              out_slot, batch, n, base_log, n_groups);
+                                                                                              out_slot, many, batch, n, base_log, n_groups);
     else if (cts == 3)
         tbm4::pbs_multibit_kernel_v4<3><<<(batch + 2) / 3, 384, sizeof(tbm4::Smem<3>), stream>>>(lwe_small, lut_idx, luts, bk, tb, rt, out,
-                                                                                              out_slot, batch, n, base_log, n_groups);
+                                                                                              out_slot, many, batch, n, base_log, n_groups);
     else
         tbm4::pbs_multibit_kernel_v4<4><<<(batch + 3) / 4, 512, sizeof(tbm4::Smem<4>), stream>>>(lwe_small, lut_idx, luts, bk, tb, rt, out,
-                                                                                              out_slot, batch, n, base_log, n_groups);
+                                                                                              out_slot, many, batch, n, base_log, n_groups);
     return cudaGetLastError();
 }
 

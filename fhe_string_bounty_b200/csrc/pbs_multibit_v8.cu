@@ -11,6 +11,7 @@
 // Key stream: 512 KiB per step through a ring of eleven 16 KiB pieces ([j & 1][out poly][sel][thread 128]: two GGSWs of ONE frequency);
 // the four pieces of a frequency are released together.
 #include "kernels.h"
+#include "sample_extract.cuh"
 #include "pbs8_common.cuh"
 
 namespace tbm8 {
@@ -43,7 +44,7 @@ __device__ __forceinline__ size_t bskm8_index(int grp, int j, int g, int c, int 
 __global__ void __launch_bounds__(256, 1)
 pbs_multibit_kernel_v8(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                        const cplx *__restrict__ bskm, const cplx *__restrict__ tbl8, const cplx *__restrict__ roots,   // roots[e] = exp(i*pi*e/2048)
-                       uint64_t *__restrict__ out, const uint32_t *__restrict__ out_slot, int batch, int n, int base_log, int n_groups) {
+                       uint64_t *__restrict__ out, const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int batch, int n, int base_log, int n_groups) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
     const int W = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -202,7 +203,10 @@ pbs_multibit_kernel_v8(const uint64_t *__restrict__ lwe_small, const uint32_t *_
         }
     }
 
-    if (blockIdx.x < batch) {
+    if (blockIdx.x < batch && many.fn) {
+        const int nf = tbx::many_fn_count(many, lut_idx, ct);
+        tbx::extract_many_regs<8, 128, kN, 1>(out, out_slot[ct], nf, tbx::many_step(many, nf, kN), w, T, re, im);
+    } else if (blockIdx.x < batch) {
         uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (kN + 1);
         if (w == 0) {
 #pragma unroll
@@ -252,7 +256,7 @@ constexpr int COMB_COLS = 128;     // Tensor Memory: [step parity 2][register g 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(288, 1)
 pbs_multibit_kernel_v8x2(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                          const cplx *__restrict__ bskm, const cplx *__restrict__ tbl8, const cplx *__restrict__ roots,
-                         uint64_t *__restrict__ out, const uint32_t *__restrict__ out_slot, int batch, int n, int base_log, int n_groups) {
+                         uint64_t *__restrict__ out, const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int batch, int n, int base_log, int n_groups) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     SmemX2 &sm = *reinterpret_cast<SmemX2 *>(smem_raw);
     const int T = threadIdx.x & 127, lane = threadIdx.x & 31;
@@ -474,17 +478,22 @@ pbs_multibit_kernel_v8x2(const uint64_t *__restrict__ lwe_small, const uint32_t 
                 im[m] = __longlong_as_double((long long)from_torus_f64(im[m]));
             }
         }
-        uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (kN + 1);
-        if (w == 0) {
+        if (many.fn) {
+            const int nf = tbx::many_fn_count(many, lut_idx, ct);
+            tbx::extract_many_regs<8, 128, kN, 1>(out, out_slot[ct], nf, tbx::many_step(many, nf, kN), w, T, re, im);
+        } else {
+            uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (kN + 1);
+            if (w == 0) {
 #pragma unroll
-            for (int m = 0; m < 8; ++m) {
-                const int j = T + 128 * m;
-                const uint64_t v0 = (uint64_t)__double_as_longlong(re[m]), v1 = (uint64_t)__double_as_longlong(im[m]);
-                if (j == 0) o[0] = v0; else o[kN - j] = (uint64_t)0 - v0;
-                o[kN - (j + kM)] = (uint64_t)0 - v1;
+                for (int m = 0; m < 8; ++m) {
+                    const int j = T + 128 * m;
+                    const uint64_t v0 = (uint64_t)__double_as_longlong(re[m]), v1 = (uint64_t)__double_as_longlong(im[m]);
+                    if (j == 0) o[0] = v0; else o[kN - j] = (uint64_t)0 - v0;
+                    o[kN - (j + kM)] = (uint64_t)0 - v1;
+                }
+            } else if (T == 0) {
+                o[kN] = (uint64_t)__double_as_longlong(re[0]);
             }
-        } else if (T == 0) {
-            o[kN] = (uint64_t)__double_as_longlong(re[0]);
         }
     }
     // nobody leaves while the partner could still address its shared memory
@@ -538,18 +547,18 @@ cudaError_t pbs_multibit_v8_configure() {
 
 // one ciphertext per CTA: for batch <= SM count (the caller dispatches wider levels to launch_pbs_multibit_v4)
 cudaError_t launch_pbs_multibit_v8(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskm8,
-                                   const void *tbl8, const void *roots, uint64_t *out, const uint32_t *out_slot, int batch, int n,
+                                   const void *tbl8, const void *roots, uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n,
                                    int base_log, int n_groups, int cluster_max, cudaStream_t stream) {
     if (batch <= 0) return cudaSuccess;
     if (batch <= cluster_max) {
         tbm8::pbs_multibit_kernel_v8x2<<<2 * batch, 288, sizeof(tbm8::SmemX2), stream>>>(
             lwe_small, lut_idx, luts, reinterpret_cast<const tb::cplx *>(bskm8), reinterpret_cast<const tb::cplx *>(tbl8),
-            reinterpret_cast<const tb::cplx *>(roots), out, out_slot, batch, n, base_log, n_groups);
+            reinterpret_cast<const tb::cplx *>(roots), out, out_slot, many, batch, n, base_log, n_groups);
         return cudaGetLastError();
     }
     tbm8::pbs_multibit_kernel_v8<<<batch, 256, sizeof(tbm8::Smem), stream>>>(
         lwe_small, lut_idx, luts, reinterpret_cast<const tb::cplx *>(bskm8), reinterpret_cast<const tb::cplx *>(tbl8),
-        reinterpret_cast<const tb::cplx *>(roots), out, out_slot, batch, n, base_log, n_groups);
+        reinterpret_cast<const tb::cplx *>(roots), out, out_slot, many, batch, n, base_log, n_groups);
     return cudaGetLastError();
 }
 

@@ -22,6 +22,7 @@
 #include <cstdlib>
 
 #include "kernels.h"
+#include "sample_extract.cuh"
 #include "pbs16_common.cuh"
 #include "fft16x_slots.cuh"
 
@@ -117,7 +118,7 @@ template <int CTS>
 __global__ void __launch_bounds__(64 * CTS, 1)
 pbs_n512_kernel(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                 const cplx *__restrict__ bskf, const cplx *__restrict__ tbl, uint64_t *__restrict__ out,
-                const uint32_t *__restrict__ out_slot, int batch, int n, int base_log, int n_iters) {
+                const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int batch, int n, int base_log, int n_iters) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int WARPS = 2 * CTS, WPQ = (WARPS + 3) / 4;        // warps that share a TMEM lane quarter
     constexpr int TW_COL = 64 * WPQ, NEED = TW_COL + 64;
@@ -297,7 +298,10 @@ pbs_n512_kernel(const uint64_t *__restrict__ lwe_small, const uint32_t *__restri
     }
 
     // sample extraction of coefficient 0 (glwe_sample_extraction.rs:91-147): mask polynomial r -> out[r N + 0] = A_r[0], out[r N + j] = -A_r[N - j]
-    if (live) {
+    if (live && many.fn) {
+        const int nf = tbx::many_fn_count(many, lut_idx, ct);
+        tbx::extract_many_regs<16, 16, N, K1 - 1>(out, out_slot[ct], nf, tbx::many_step(many, nf, N), r, T, re, im);
+    } else if (live) {
         uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * ((K1 - 1) * N + 1);
         if (r < K1 - 1) {
             uint64_t *base = o + r * N;
@@ -361,18 +365,18 @@ cudaError_t pbs_n512_configure() {
 }
 
 cudaError_t launch_pbs_n512(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskf, const void *tbl,
-                            uint64_t *out, const uint32_t *out_slot, int batch, int n, int base_log, int n_iters, cudaStream_t stream) {
+                            uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n, int base_log, int n_iters, cudaStream_t stream) {
     if (batch <= 0) return cudaSuccess;
     int sms = 148, dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const tb::cplx *bk = reinterpret_cast<const tb::cplx *>(bskf), *tb = reinterpret_cast<const tb::cplx *>(tbl);
     if (batch <= sms)
-        tb512::pbs_n512_kernel<1><<<batch, 64, sizeof(tb512::Smem<1>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, batch, n, base_log, n_iters);
+        tb512::pbs_n512_kernel<1><<<batch, 64, sizeof(tb512::Smem<1>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many, batch, n, base_log, n_iters);
     else if (batch <= 4 * sms)
-        tb512::pbs_n512_kernel<4><<<(batch + 3) / 4, 256, sizeof(tb512::Smem<4>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, batch, n, base_log, n_iters);
+        tb512::pbs_n512_kernel<4><<<(batch + 3) / 4, 256, sizeof(tb512::Smem<4>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many, batch, n, base_log, n_iters);
     else
-        tb512::pbs_n512_kernel<8><<<(batch + 7) / 8, 512, sizeof(tb512::Smem<8>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, batch, n, base_log, n_iters);
+        tb512::pbs_n512_kernel<8><<<(batch + 7) / 8, 512, sizeof(tb512::Smem<8>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many, batch, n, base_log, n_iters);
     return cudaGetLastError();
 }
 

@@ -28,6 +28,7 @@
 #include <cstdlib>
 
 #include "kernels.h"
+#include "sample_extract.cuh"
 #include "pbs16_common.cuh"
 #include "fft16x_slots.cuh"
 
@@ -194,7 +195,7 @@ __device__ __forceinline__ size_t key_piece(int n_ggsw, int w, int i, int lvslot
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 pbs_n8192_kernel(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                  const cplx *__restrict__ bskf, const cplx *__restrict__ tbl, uint64_t *__restrict__ out,
-                 const uint32_t *__restrict__ out_slot, int n, int base_log, int n_iters, int n_ggsw) {
+                 const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int n, int base_log, int n_iters, int n_ggsw) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
     const int T = threadIdx.x, W = T >> 5, lane = T & 31;
@@ -382,7 +383,10 @@ pbs_n8192_kernel(const uint64_t *__restrict__ lwe_small, const uint32_t *__restr
     }
 
     // sample extraction of coefficient 0: out[0] = A[0], out[N - j] = -A[j]; body = B[0]
-    {
+    if (many.fn) {
+        const int nf = tbx::many_fn_count(many, lut_idx, ct);
+        tbx::extract_many_regs<16, 256, N, 1>(out, out_slot[ct], nf, tbx::many_step(many, nf, N), w, T, re, im);
+    } else {
         uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (N + 1);
         if (w == 0) {
 #pragma unroll
@@ -446,11 +450,11 @@ cudaError_t pbs_n8192_configure() {
 }
 
 cudaError_t launch_pbs_n8192(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskf, const void *tbl,
-                             uint64_t *out, const uint32_t *out_slot, int batch, int n, int base_log, int n_iters, int n_ggsw,
+                             uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n, int base_log, int n_iters, int n_ggsw,
                              cudaStream_t stream) {
     if (batch <= 0) return cudaSuccess;
     tb8192::pbs_n8192_kernel<<<2 * batch, tb8192::THREADS, sizeof(tb8192::Smem), stream>>>(
-        lwe_small, lut_idx, luts, reinterpret_cast<const tb::cplx *>(bskf), reinterpret_cast<const tb::cplx *>(tbl), out, out_slot, n, base_log,
+        lwe_small, lut_idx, luts, reinterpret_cast<const tb::cplx *>(bskf), reinterpret_cast<const tb::cplx *>(tbl), out, out_slot, many, n, base_log,
         n_iters, n_ggsw);
     return cudaGetLastError();
 }

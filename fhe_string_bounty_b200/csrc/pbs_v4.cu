@@ -23,6 +23,7 @@
 #include <cstdlib>
 
 #include "kernels.h"
+#include "sample_extract.cuh"
 #include "pbs16_common.cuh"
 
 namespace tb4 {
@@ -57,7 +58,7 @@ template <int CTS>
 __global__ void __launch_bounds__(128 * CTS, 1)
 pbs_classic_kernel_v4(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                       const cplx *__restrict__ bskf4, const cplx *__restrict__ tbl16, uint64_t *__restrict__ out,
-                      const uint32_t *__restrict__ out_slot, int batch, int n, int base_log, int n_iters, int small_is_u16) {
+                      const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int batch, int n, int base_log, int n_iters, int small_is_u16) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int TMEM_COLS = CTS >= 3 ? 512 : 256, CONSUMERS = 4 * CTS;   // every warp reads every ring piece
     constexpr int NS = Smem<CTS>::NS;
@@ -241,7 +242,10 @@ pbs_classic_kernel_v4(const uint64_t *__restrict__ lwe_small, const uint32_t *__
     }
 
     // sample extraction (coefficient 0) straight from the registers: out[0] = A[0], out[N-j] = -A[j]; body = B[0]
-    if (live) {
+    if (live && many.fn) {
+        const int nf = tbx::many_fn_count(many, lut_idx, ct);
+        tbx::extract_many_regs<16, 64, kN, 1>(out, out_slot[ct], nf, tbx::many_step(many, nf, kN), w, T, re, im);
+    } else if (live) {
         uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (kN + 1);
         if (w == 0) {
 #pragma unroll
@@ -301,7 +305,7 @@ cudaError_t pbs_v4_configure() {
 }
 
 cudaError_t launch_pbs_classic_v4(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskf4,
-                                  const void *tbl16, uint64_t *out, const uint32_t *out_slot, int batch, int n, int base_log,
+                                  const void *tbl16, uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n, int base_log,
                                   int n_iters, int small_is_u16, int cts, cudaStream_t stream) {
     if (batch <= 0) return cudaSuccess;
     int sms = 148, dev = 0;
@@ -312,18 +316,18 @@ cudaError_t launch_pbs_classic_v4(const uint64_t *lwe_small, const uint32_t *lut
     if (cts == 0 && std::getenv("TFHE_B200_WIDE_CTS") && std::getenv("TFHE_B200_WIDE_CTS")[0] == '3' && batch > 2 * sms) cts = 3;
     if (cts == 0) cts = batch <= sms ? 1 : batch <= 2 * sms ? 2 : batch <= 3 * sms ? 3 : 4;
     if (cts == 1)
-        tb4::pbs_classic_kernel_v4<1><<<batch, 128, sizeof(tb4::Smem<1>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, batch, n,
+        tb4::pbs_classic_kernel_v4<1><<<batch, 128, sizeof(tb4::Smem<1>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many, batch, n,
                                                                                   base_log, n_iters, small_is_u16);
     else if (cts == 2)
-        tb4::pbs_classic_kernel_v4<2><<<(batch + 1) / 2, 256, sizeof(tb4::Smem<2>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot,
+        tb4::pbs_classic_kernel_v4<2><<<(batch + 1) / 2, 256, sizeof(tb4::Smem<2>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many,
                                                                                             batch, n, base_log, n_iters, small_is_u16);
     else if (cts == 3)
         // one wave of three ciphertexts per SM (152 registers, 7-slot ring) takes 5.5 ms against 7.25 ms for a -- then mostly empty -- wave
         // of four; TFHE_B200_WIDE_CTS=3 runs every wide batch on this instance (the A/B that showed equal throughput from 12 and 16 warps)
-        tb4::pbs_classic_kernel_v4<3><<<(batch + 2) / 3, 384, sizeof(tb4::Smem<3>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot,
+        tb4::pbs_classic_kernel_v4<3><<<(batch + 2) / 3, 384, sizeof(tb4::Smem<3>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many,
                                                                                             batch, n, base_log, n_iters, small_is_u16);
     else
-        tb4::pbs_classic_kernel_v4<4><<<(batch + 3) / 4, 512, sizeof(tb4::Smem<4>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot,
+        tb4::pbs_classic_kernel_v4<4><<<(batch + 3) / 4, 512, sizeof(tb4::Smem<4>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many,
                                                                                             batch, n, base_log, n_iters, small_is_u16);
     return cudaGetLastError();
 }

@@ -16,6 +16,7 @@
 // Shared memory: 17 KiB tile per polynomial + the key ring, double buffered by whole iterations (2 x 64 KiB).
 // Named barriers: 1..4 one per polynomial (128 threads), 5..6 one per ciphertext (256 threads).
 #include "kernels.h"
+#include "sample_extract.cuh"
 #include "pbs8_common.cuh"
 
 namespace tb8k {
@@ -47,7 +48,7 @@ template <int CTS>
 __global__ void __launch_bounds__(256 * CTS, 1)
 pbs_classic_kernel_v8(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                       const cplx *__restrict__ bskf8, const cplx *__restrict__ tbl8, uint64_t *__restrict__ out,
-                      const uint32_t *__restrict__ out_slot, int batch, int n, int base_log, int n_iters, int small_is_u16) {
+                      const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int batch, int n, int base_log, int n_iters, int small_is_u16) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int WARPS = 8 * CTS, TMEM_COLS = 256, TW_COL = 128;   // accumulators: 32 columns per (ciphertext, polynomial); twiddles: 96
     constexpr bool REGS = CTS == 1;     // one ciphertext per CTA: twiddles and the accumulator master copy live in registers, no TMEM
@@ -234,7 +235,10 @@ pbs_classic_kernel_v8(const uint64_t *__restrict__ lwe_small, const uint32_t *__
     }
 
     // sample extraction (coefficient 0) straight from the registers: out[0] = A[0], out[N-j] = -A[j]; body = B[0]
-    if (live) {
+    if (live && many.fn) {
+        const int nf = tbx::many_fn_count(many, lut_idx, ct);
+        tbx::extract_many_regs<8, 128, kN, 1>(out, out_slot[ct], nf, tbx::many_step(many, nf, kN), w, T, re, im);
+    } else if (live) {
         uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (kN + 1);
         if (w == 0) {
 #pragma unroll
@@ -278,7 +282,7 @@ struct SmemX2 {
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(160, 1)
 pbs_classic_kernel_v8x2(const uint64_t *__restrict__ lwe_small, const uint32_t *__restrict__ lut_idx, const uint64_t *__restrict__ luts,
                         const cplx *__restrict__ bskf8, const cplx *__restrict__ tbl8, uint64_t *__restrict__ out,
-                        const uint32_t *__restrict__ out_slot, int batch, int n, int base_log, int n_iters, int small_is_u16) {
+                        const uint32_t *__restrict__ out_slot, const tbk::ManyLut many, int batch, int n, int base_log, int n_iters, int small_is_u16) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     SmemX2 &sm = *reinterpret_cast<SmemX2 *>(smem_raw);
     const int T = threadIdx.x;
@@ -418,17 +422,22 @@ pbs_classic_kernel_v8x2(const uint64_t *__restrict__ lwe_small, const uint32_t *
         }
     }
 
-    uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (kN + 1);
-    if (w == 0) {
+    if (many.fn) {
+        const int nf = tbx::many_fn_count(many, lut_idx, ct);
+        tbx::extract_many_regs<8, 128, kN, 1>(out, out_slot[ct], nf, tbx::many_step(many, nf, kN), w, T, re, im);
+    } else {
+        uint64_t *o = out + (size_t)(out_slot ? out_slot[ct] : ct) * (kN + 1);
+        if (w == 0) {
 #pragma unroll
-        for (int m = 0; m < 8; ++m) {
-            const int j = T + 128 * m;
-            const uint64_t v0 = (uint64_t)__double_as_longlong(re[m]), v1 = (uint64_t)__double_as_longlong(im[m]);
-            if (j == 0) o[0] = v0; else o[kN - j] = (uint64_t)0 - v0;
-            o[kN - (j + kM)] = (uint64_t)0 - v1;
+            for (int m = 0; m < 8; ++m) {
+                const int j = T + 128 * m;
+                const uint64_t v0 = (uint64_t)__double_as_longlong(re[m]), v1 = (uint64_t)__double_as_longlong(im[m]);
+                if (j == 0) o[0] = v0; else o[kN - j] = (uint64_t)0 - v0;
+                o[kN - (j + kM)] = (uint64_t)0 - v1;
+            }
+        } else if (T == 0) {
+            o[kN] = (uint64_t)__double_as_longlong(re[0]);
         }
-    } else if (T == 0) {
-        o[kN] = (uint64_t)__double_as_longlong(re[0]);
     }
     cluster_sync_all();     // nobody leaves while the partner could still address its shared memory
 }
@@ -472,7 +481,7 @@ cudaError_t pbs_v8_configure() {
 
 // batch <= 2 * SM count only (the caller dispatches wider levels to launch_pbs_classic_v4)
 cudaError_t launch_pbs_classic_v8(const uint64_t *lwe_small, const uint32_t *lut_idx, const uint64_t *luts, const void *bskf8,
-                                  const void *tbl8, uint64_t *out, const uint32_t *out_slot, int batch, int n, int base_log,
+                                  const void *tbl8, uint64_t *out, const uint32_t *out_slot, tbk::ManyLut many, int batch, int n, int base_log,
                                   int n_iters, int small_is_u16, int cluster_max, cudaStream_t stream) {
     if (batch <= 0) return cudaSuccess;
     int sms = 148, dev = 0;
@@ -480,13 +489,13 @@ cudaError_t launch_pbs_classic_v8(const uint64_t *lwe_small, const uint32_t *lut
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const tb::cplx *bk = reinterpret_cast<const tb::cplx *>(bskf8), *tb = reinterpret_cast<const tb::cplx *>(tbl8);
     if (batch <= cluster_max && batch <= sms / 2)      // one ciphertext per two-SM cluster
-        tb8k::pbs_classic_kernel_v8x2<<<2 * batch, 160, sizeof(tb8k::SmemX2), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, batch, n,
+        tb8k::pbs_classic_kernel_v8x2<<<2 * batch, 160, sizeof(tb8k::SmemX2), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many, batch, n,
                                                                                      base_log, n_iters, small_is_u16);
     else if (batch <= sms)
-        tb8k::pbs_classic_kernel_v8<1><<<batch, 256, sizeof(tb8k::Smem<1>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, batch, n,
+        tb8k::pbs_classic_kernel_v8<1><<<batch, 256, sizeof(tb8k::Smem<1>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many, batch, n,
                                                                                    base_log, n_iters, small_is_u16);
     else
-        tb8k::pbs_classic_kernel_v8<2><<<(batch + 1) / 2, 512, sizeof(tb8k::Smem<2>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot,
+        tb8k::pbs_classic_kernel_v8<2><<<(batch + 1) / 2, 512, sizeof(tb8k::Smem<2>), stream>>>(lwe_small, lut_idx, luts, bk, tb, out, out_slot, many,
                                                                                              batch, n, base_log, n_iters, small_is_u16);
     return cudaGetLastError();
 }
