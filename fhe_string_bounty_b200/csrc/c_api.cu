@@ -244,6 +244,7 @@ int tfhe_b200_ctx_create(int cuda_device, const tfhe_b200_params *params, tfhe_b
     c->p = *params;
     TB_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     for (auto &e : c->ev) TB_CUDA(cudaEventCreate(&e));
+    TB_CUDA(cudaEventCreateWithFlags(&c->scratch_done, cudaEventDisableTiming));
     for (auto &L : c->lane) TB_CUDA(cudaStreamCreateWithFlags(&L.s, cudaStreamNonBlocking));
     if (const char *e = std::getenv("TFHE_B200_KS_KERNEL")) c->ks_kernel = (e[0] == 'i') ? 0 : (e[0] == 'm') ? 1 : 2;   // imad / mma / tc
     if (c->ks_kernel == 2 && !tbk::ks_tc_supported((int)(params->glwe_dim * params->poly_size), (int)params->ks_level)) c->ks_kernel = 1;
@@ -348,6 +349,7 @@ int tfhe_b200_ctx_destroy(tfhe_b200_ctx *c) {
     if (!c) return 0;
     DeviceGuard g(c->device);
     cudaStreamSynchronize(c->stream);
+    if (c->scratch_done) { cudaEventSynchronize(c->scratch_done); cudaEventDestroy(c->scratch_done); }   // calls pending on other streams
     for (DevBuf *b : {&c->ksk_packed, &c->ksk_colsum, &c->ksk_planes, &c->ks_digits, &c->bskf, &c->bskf8, &c->tbl16, &c->tbl8, &c->tw_generic, &c->roots, &c->luts, &c->lut_fn, &c->d_in, &c->d_small, &c->d_out, &c->d_idx})
         b->release();
     for (auto &e : c->ev) if (e) cudaEventDestroy(e);
@@ -629,9 +631,12 @@ int tfhe_b200_synchronize(tfhe_b200_ctx *c) {
 
 int tfhe_b200_keyswitch_batch_device(tfhe_b200_ctx *c, const uint64_t *d_in, uint64_t *d_small, size_t batch, void *stream) {
     if (!c || (batch && (!d_in || !d_small))) return fail("null argument");
-    std::lock_guard<std::mutex> lk(c->mu);   // the digit scratch buffer is per context
+    std::lock_guard<std::mutex> lk(c->mu);
     DeviceGuard g(c->device);
-    return do_keyswitch(c, d_in, d_small, batch, stream ? (cudaStream_t)stream : c->stream);
+    const cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
+    tbc::StreamOrder scratch(c->scratch_done, s);   // the digit buffer is per context
+    TB_CUDA(scratch.wait);
+    return do_keyswitch(c, d_in, d_small, batch, s);
 }
 
 int tfhe_b200_pbs_batch_device(tfhe_b200_ctx *c, const uint64_t *d_small, const uint32_t *d_idx, uint64_t *d_out, size_t batch,
@@ -650,6 +655,8 @@ int tfhe_b200_ks_pbs_batch_device(tfhe_b200_ctx *c, const uint64_t *d_in, const 
     DeviceGuard g(c->device);
     cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
     if (refuse_many(c)) return 1;
+    tbc::StreamOrder scratch(c->scratch_done, s);
+    TB_CUDA(scratch.wait);
     TB_CUDA(c->d_small.reserve_on(batch * c->small_len() * 8, s));
     TB_CUDA(cudaEventRecord(c->ev[0], s));
     const bool fused = tbc::fused_supported(c);
@@ -678,8 +685,10 @@ int tfhe_b200_keyswitch_batch(tfhe_b200_ctx *c, const uint64_t *in, uint64_t *ou
     if (batch == 0) return 0;
     std::lock_guard<std::mutex> lk(c->mu);
     DeviceGuard g(c->device);
+    tbc::StreamOrder scratch(c->scratch_done, c->stream);   // a device call on another stream may still use d_small / ks_digits
+    TB_CUDA(scratch.wait);
     TB_CUDA(c->d_in.reserve(batch * c->big_len() * 8));
-    TB_CUDA(c->d_small.reserve(batch * c->small_len() * 8));
+    TB_CUDA(c->d_small.reserve_on(batch * c->small_len() * 8, c->stream));
     TB_CUDA(cudaMemcpyAsync(c->d_in.p, in, batch * c->big_len() * 8, cudaMemcpyHostToDevice, c->stream));
     if (do_keyswitch(c, (const uint64_t *)c->d_in.p, (uint64_t *)c->d_small.p, batch, c->stream)) return 1;
     TB_CUDA(cudaMemcpyAsync(out, c->d_small.p, batch * c->small_len() * 8, cudaMemcpyDeviceToHost, c->stream));
@@ -694,7 +703,9 @@ static int pbs_host(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t *idx, u
     std::lock_guard<std::mutex> lk(c->mu);
     if (check_lut_indices(c, idx, batch)) return 1;
     DeviceGuard g(c->device);
-    TB_CUDA(c->d_small.reserve(batch * c->small_len() * 8));
+    tbc::StreamOrder scratch(c->scratch_done, c->stream);
+    TB_CUDA(scratch.wait);
+    TB_CUDA(c->d_small.reserve_on(batch * c->small_len() * 8, c->stream));
     TB_CUDA(c->d_out.reserve(batch * c->big_len() * 8));
     TB_CUDA(cudaMemcpyAsync(c->d_small.p, in, batch * c->small_len() * 8, cudaMemcpyHostToDevice, c->stream));
     const uint32_t *d_idx = nullptr;
@@ -768,7 +779,9 @@ int tfhe_b200_pbs_ks_batch(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t 
     if (refuse_many(c) || check_lut_indices(c, idx, batch)) return 1;
     DeviceGuard g(c->device);
     cudaStream_t s = c->stream;
-    TB_CUDA(c->d_small.reserve(batch * c->small_len() * 8));
+    tbc::StreamOrder scratch(c->scratch_done, s);
+    TB_CUDA(scratch.wait);
+    TB_CUDA(c->d_small.reserve_on(batch * c->small_len() * 8, s));
     TB_CUDA(c->d_out.reserve(batch * c->big_len() * 8));
     TB_CUDA(c->d_in.reserve(batch * c->small_len() * 8));
     TB_CUDA(cudaMemcpyAsync(c->d_small.p, in, batch * c->small_len() * 8, cudaMemcpyHostToDevice, s));
@@ -820,14 +833,13 @@ static int many_batch(tfhe_b200_ctx *c, const uint64_t *d_in, const uint32_t *d_
 
 static int many_pbs(tfhe_b200_ctx *c, const uint64_t *d_in, const uint32_t *d_idx, uint64_t *d_out, size_t batch, uint32_t n_iters,
                     cudaStream_t s, bool ks, const uint32_t *rows) {
-    const uint64_t *d_small = d_in;
-    const bool fused = ks && tbc::fused_supported(c);
-    if (ks) {
-        TB_CUDA(c->d_small.reserve_on(batch * c->small_len() * 8, s));
-        if (tbc::do_keyswitch(c, d_in, (uint64_t *)c->d_small.p, batch, s, nullptr, nullptr, fused)) return 1;
-        d_small = (const uint64_t *)c->d_small.p;
-    }
-    return tbc::do_pbs(c, d_small, d_idx, (const uint64_t *)c->luts.p, d_out, batch, n_iters, s, rows, fused, ctx_many(c));
+    if (!ks) return tbc::do_pbs(c, d_in, d_idx, (const uint64_t *)c->luts.p, d_out, batch, n_iters, s, rows, false, ctx_many(c));
+    const bool fused = tbc::fused_supported(c);
+    tbc::StreamOrder scratch(c->scratch_done, s);
+    TB_CUDA(scratch.wait);
+    TB_CUDA(c->d_small.reserve_on(batch * c->small_len() * 8, s));
+    if (tbc::do_keyswitch(c, d_in, (uint64_t *)c->d_small.p, batch, s, nullptr, nullptr, fused)) return 1;
+    return tbc::do_pbs(c, (const uint64_t *)c->d_small.p, d_idx, (const uint64_t *)c->luts.p, d_out, batch, n_iters, s, rows, fused, ctx_many(c));
 }
 
 static int many_host(tfhe_b200_ctx *c, const uint64_t *in, const uint32_t *idx, uint64_t *out, size_t batch, uint32_t n_iters, bool ks) {

@@ -58,6 +58,21 @@ struct DeviceGuard {
     ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
+// Orders the calls that share a device buffer across streams.  The constructor makes `s` wait for `done`, the event the previous user
+// recorded after its last launch that touched the buffer; the caller checks `wait` before it grows or touches the buffer, so a growth
+// (reserve_on) frees only memory that nothing still reads.  The destructor records `done` on `s` after everything the call enqueued,
+// on its error paths too.  The mutex only orders the enqueues: without this, a call on another stream overwrites the buffer while
+// kernels of the previous call still read it.
+struct StreamOrder {
+    cudaEvent_t done;
+    cudaStream_t s;
+    cudaError_t wait;
+    StreamOrder(cudaEvent_t done_, cudaStream_t s_) : done(done_), s(s_), wait(cudaStreamWaitEvent(s_, done_, 0)) {}
+    StreamOrder(const StreamOrder &) = delete;
+    StreamOrder &operator=(const StreamOrder &) = delete;
+    ~StreamOrder() { if (wait == cudaSuccess) cudaEventRecord(done, s); }
+};
+
 }  // namespace tbc
 
 struct tfhe_b200_ctx {
@@ -85,8 +100,11 @@ struct tfhe_b200_ctx {
     int tuned512_min = 0;    // 0 = default (SM count); smaller batches stay on the generic kernel
     int narrow_cluster = 1;  // classic levels of at most SM count / 2 ciphertexts: one ciphertext per two-SM cluster (pbs_classic_kernel_v8x2)
     int narrow_max = 0;      // widest level the narrow kernel takes (0 = 2 * SM count); env TFHE_B200_NARROW_MAX
-    // staging for the host-pointer entry points
+    // staging for the host-pointer entry points; d_small is also the keyswitch -> PBS hand-off of the device entries and programs
     tbc::DevBuf d_in, d_small, d_out, d_idx;
+    // recorded after the last launch of a call that uses ks_digits or d_small, on the call's stream: every such call, on any stream,
+    // waits for it first (tbc::StreamOrder)
+    cudaEvent_t scratch_done = nullptr;
     // two copy/compute lanes for the host-buffer KS-PBS entry point: H2D of chunk k+1 and D2H of chunk k-1 overlap the
     // kernels of chunk k, and the tail wave of one chunk overlaps the head of the next
     struct Lane { cudaStream_t s = nullptr; tbc::DevBuf in, small, out, idx, digits; };

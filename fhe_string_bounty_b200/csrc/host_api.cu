@@ -8,6 +8,7 @@
 #include "../../include/tfhe_b200_sharded.h"
 
 #include <cstring>
+#include <deque>
 #include <memory>
 
 using tbc::DevBuf;
@@ -27,6 +28,9 @@ struct tfhe_b200_program {
     std::vector<uint32_t> lin_off, pbs_off;   // per level offsets
     float last_ms = 0.f;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    // recorded after the last launch of a run that reads d_arena (the output gather): a run on any stream waits for it before it writes
+    // its inputs there (tbc::StreamOrder)
+    cudaEvent_t arena_done = nullptr;
 };
 
 namespace {
@@ -466,7 +470,8 @@ void release_device_state(tfhe_b200_program &h) {
     for (DevBuf *b : {&h.d_luts, &h.d_lin, &h.d_terms, &h.d_pbs_in, &h.d_pbs_out, &h.d_pbs_lut, &h.d_arena, &h.d_out_slots, &h.d_out_rows}) b->release();
     if (h.ev0) cudaEventDestroy(h.ev0);
     if (h.ev1) cudaEventDestroy(h.ev1);
-    h.ev0 = h.ev1 = nullptr;
+    if (h.arena_done) cudaEventDestroy(h.arena_done);
+    h.ev0 = h.ev1 = h.arena_done = nullptr;
     h.owner_id = 0;
     h.device = -1;
 }
@@ -488,6 +493,7 @@ int bind_program(tfhe_b200_ctx *c, tfhe_b200_program *h) {
     h->device = c->device;            // from here on release_device_state() knows where the partial uploads live
     TB_CUDA(cudaEventCreate(&h->ev0));
     TB_CUDA(cudaEventCreate(&h->ev1));
+    TB_CUDA(cudaEventCreateWithFlags(&h->arena_done, cudaEventDisableTiming));
     std::vector<uint64_t> accs(std::max<size_t>(h->luts->size(), 1) * h->p.lut_len());
     for (size_t u = 0; u < h->luts->size(); ++u) h->luts->fill_accumulator(uint32_t(u), accs.data() + u * h->p.lut_len());
     TB_CUDA(h->d_luts.reserve(accs.size() * 8));
@@ -554,7 +560,10 @@ int enqueue_levels(const Member *m, uint32_t n, uint64_t min_shard_width, cudaSt
     const uint32_t world = m[0].ex ? m[0].ex->world : 1;
     size_t max_w = 0;
     for (auto &l : pg.levels()) max_w = std::max(max_w, l.pbs.size());
+    std::deque<tbc::StreamOrder> scratch;     // every member context's d_small and keyswitch digits, released when the levels are enqueued
     for (uint32_t i = 0; i < n; ++i) {
+        scratch.emplace_back(m[i].c->scratch_done, s);
+        TB_CUDA(scratch.back().wait);
         TB_CUDA(cudaEventRecord(m[i].h->ev0, s));
         TB_CUDA(m[i].c->d_small.reserve_on(std::max<size_t>(max_w, 1) * m[i].c->small_len() * 8, s));
     }
@@ -727,6 +736,8 @@ int tfhe_b200_program_run(tfhe_b200_ctx *c, tfhe_b200_program *h, const uint64_t
     cudaStream_t s = c->stream;
     const size_t L = c->big_len();
     if (bind_program(c, h)) return 1;
+    tbc::StreamOrder arena(h->arena_done, s);     // a run_device of this program may be pending on another stream
+    TB_CUDA(arena.wait);
     if (pg.n_inputs()) TB_CUDA(cudaMemcpyAsync(h->d_arena.p, inputs, (size_t)pg.n_inputs() * L * 8, cudaMemcpyHostToDevice, s));
     const Member m{c, h, nullptr, (uint64_t *)h->d_out_rows.p};
     if (enqueue_levels(&m, 1, 0, s)) return 1;
@@ -740,7 +751,7 @@ int tfhe_b200_program_run(tfhe_b200_ctx *c, tfhe_b200_program *h, const uint64_t
 /* The same on DEVICE buffers of the context's GPU, enqueued on `cuda_stream` (NULL = the context's own stream) WITHOUT synchronising:
  * d_inputs n_inputs x (k*N+1) words, d_outputs n_outputs x (k*N+1) words.  This is what chains a rank's share of a sharded string
  * operation, the exchange of the narrow-end blocks and the finishing program without a host round trip (multi_gpu.py).
- * One stream at a time per context: the keyswitch scratch and the program's arena are per context / per program. */
+ * Calls on other streams may overlap it: the context's keyswitch scratch and the program's arena are taken in enqueue order (StreamOrder). */
 int tfhe_b200_program_run_device(tfhe_b200_ctx *c, tfhe_b200_program *h, const uint64_t *d_inputs, uint64_t *d_outputs, void *cuda_stream) {
     if (!c || !h) return fail("null argument");
     const tbh::Program &pg = *h->prog;
@@ -751,6 +762,8 @@ int tfhe_b200_program_run_device(tfhe_b200_ctx *c, tfhe_b200_program *h, const u
     cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
     const size_t L = c->big_len();
     if (bind_program(c, h)) return 1;
+    tbc::StreamOrder arena(h->arena_done, s);
+    TB_CUDA(arena.wait);
     if (pg.n_inputs()) TB_CUDA(cudaMemcpyAsync(h->d_arena.p, d_inputs, (size_t)pg.n_inputs() * L * 8, cudaMemcpyDeviceToDevice, s));
     h->last_ms = -1.f;    // not synchronised: tfhe_b200_program_last_ms reads the events on demand
     const Member m{c, h, nullptr, d_outputs};
@@ -792,6 +805,8 @@ int tfhe_b200_program_run_sharded(tfhe_b200_ctx *c, tfhe_b200_program *h, tfhe_b
     DeviceGuard g(c->device);
     cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
     if (bind_program(c, h)) return 1;
+    tbc::StreamOrder arena(h->arena_done, s);
+    TB_CUDA(arena.wait);
     if (pg.n_inputs()) TB_CUDA(cudaMemcpyAsync(h->d_arena.p, d_inputs, (size_t)pg.n_inputs() * c->big_len() * 8, cudaMemcpyDeviceToDevice, s));
     h->last_ms = -1.f;
     const Member m{c, h, ex, d_outputs};
@@ -833,7 +848,10 @@ int tfhe_b200_program_run_sharded_group(tfhe_b200_ctx *const *ctxs, tfhe_b200_pr
         if (bind_program(ctxs[r], progs[r])) return 1;
         m[r] = Member{ctxs[r], progs[r], exs[r], d_outputs[r]};
     }
+    std::deque<tbc::StreamOrder> arena;
     for (uint32_t r = 0; r < world; ++r) {
+        arena.emplace_back(progs[r]->arena_done, s);
+        TB_CUDA(arena.back().wait);
         if (pg.n_inputs())
             TB_CUDA(cudaMemcpyAsync(progs[r]->d_arena.p, d_inputs[r], (size_t)pg.n_inputs() * ctxs[r]->big_len() * 8, cudaMemcpyDeviceToDevice, s));
         progs[r]->last_ms = -1.f;

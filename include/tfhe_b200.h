@@ -119,7 +119,10 @@ int tfhe_b200_pbs_ks_batch(tfhe_b200_ctx *ctx, const uint64_t *lwe_small_in, con
 
 /* Same operations on DEVICE buffers of the context's GPU, enqueued on `cuda_stream` (a cudaStream_t;
  * NULL = the context's own stream) without synchronising: used to chain tree levels and by the
- * multi-GPU driver. */
+ * multi-GPU driver.  Calls on any streams of one context may overlap.  Where they share the context's
+ * scratch (the keyswitch digits, the keyswitch -> PBS hand-off rows), the context orders them in the
+ * order they were enqueued, and the host entries above too; runs of one program are ordered the same
+ * way around its arena.  Your own buffers are yours to order. */
 int tfhe_b200_keyswitch_batch_device(tfhe_b200_ctx *ctx, const uint64_t *d_lwe_big, uint64_t *d_lwe_small, size_t batch,
                                      void *cuda_stream);
 int tfhe_b200_pbs_batch_device(tfhe_b200_ctx *ctx, const uint64_t *d_lwe_small, const uint32_t *d_lut_idx,
@@ -216,7 +219,8 @@ int tfhe_b200_program_copy(const tfhe_b200_program *prog, uint32_t *level_lin_of
 int tfhe_b200_program_accumulators(const tfhe_b200_program *prog, uint64_t *accs);
 int tfhe_b200_program_run(tfhe_b200_ctx *ctx, tfhe_b200_program *prog, const uint64_t *inputs, uint64_t *outputs);
 /* Same on DEVICE buffers of the context's GPU, enqueued on `cuda_stream` (NULL = the context's stream) without synchronising; chains a
- * rank's share of a sharded operation, the exchange below and the finishing program with no host round trip in between. */
+ * rank's share of a sharded operation, the exchange below and the finishing program with no host round trip in between.  Runs of one
+ * program, on any streams and through either entry, are ordered around its arena in the order they were enqueued. */
 int tfhe_b200_program_run_device(tfhe_b200_ctx *ctx, tfhe_b200_program *prog, const uint64_t *d_inputs, uint64_t *d_outputs,
                                  void *cuda_stream);
 int tfhe_b200_program_last_ms(const tfhe_b200_program *prog, float *ms);
