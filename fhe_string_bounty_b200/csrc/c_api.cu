@@ -371,7 +371,9 @@ static int finish_ksk(tfhe_b200_ctx *c, const tbc::DevBuf &raw) {
     TB_CUDA(tbk::launch_ksk_pack((const uint64_t *)raw.p, (uint64_t *)c->ksk_packed.p, (uint64_t *)c->ksk_colsum.p, (int)rows,
                                  (int)c->p.lwe_dim, c->stream));
     c->launches += 2;
-    if (c->ks_kernel >= 1) {
+    // the byte planes are rebuilt whenever a copy exists, even with ks_kernel = 0 selected for now: set_tuning lets a tensor-core
+    // kernel back in as soon as planes exist, and they must be this key's
+    if (c->ks_kernel >= 1 || c->ksk_planes.p) {
         TB_CUDA(c->ksk_planes.reserve(rows * (size_t)ldk * 8));
         TB_CUDA(tbk::launch_ksk_planes((const uint64_t *)c->ksk_packed.p, (uint8_t *)c->ksk_planes.p, (int)rows, ldk, c->stream));
         c->launches += 1;
@@ -392,7 +394,10 @@ static int finish_bsk(tfhe_b200_ctx *c, const tbc::DevBuf &raw) {
     TB_CUDA(c->bskf.reserve(n_polys * (c->p.poly_size / 2) * sizeof(double) * 2));
     if (c->generic) {
         TB_CUDA(tbk::launch_bsk_convert_generic((const uint64_t *)raw.p, c->bskf.p, c->tw_generic.p, n_polys, (int)c->p.poly_size, c->stream));
-        if (c->tuned8192) {    // second copy of the key, per output polynomial, in pbs_n8192.cu's ring order
+        // second copy of the key, per output polynomial, in pbs_n8192.cu's ring order; rebuilt whenever a copy exists, even with
+        // tuned8192 = 0 selected for now (set_tuning turns pbs_n8192.cu back on as soon as bskf8 exists)
+        if (c->tuned8192 || (c->bskf8.p && tbk::pbs_n8192_supported((int)c->p.poly_size, (int)c->p.glwe_dim, (int)c->p.pbs_level,
+                                                                     (int)c->p.pbs_base_log, (int)c->p.grouping_factor))) {
             TB_CUDA(c->bskf8.reserve(n_polys * (c->p.poly_size / 2) * sizeof(double) * 2));
             TB_CUDA(tbk::launch_bsk_convert_n8192((const uint64_t *)raw.p, c->bskf8.p, c->tbl16.p, (int)c->p.lwe_dim, c->stream));
             c->launches += 1;
